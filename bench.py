@@ -14,6 +14,10 @@ memory (H2D inside the timed region) and the flag grids (bit-packed) + event tab
   python bench.py --workload decade-track --hours H ...     (detection of H consecutive hours sharded over the
                                                             ranks + track_events(by_overlap) across the shard
                                                             boundaries; BASELINE.json configs[4])
+  python bench.py ... --dump-outputs DIR                    (also write what the last timed batch returned as
+                                                            DIR/<name>.npy, see dump_outputs)
+
+The benchmark writes nothing into the source tree (no bytecode caches either), so it runs from a read-only checkout.
 """
 
 import argparse
@@ -30,6 +34,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the package modules imported below leave no __pycache__ in the tree
 
 METRIC = "time steps/sec, 0.25deg hourly PV 2-PVU detection (streamers+overturnings+cutoffs+to_xarray)"
 UNIT = "time steps/s"
@@ -62,7 +67,13 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip the stress line, the e2e variants and the link test")
     ap.add_argument("--workload", default="c25", choices=["c25", "decade-track"])
     ap.add_argument("--hours", type=int, default=None, help="decade-track: consecutive hours (default 8760 per GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (rank 0)")
     a = ap.parse_args()
+    if a.dump_outputs is not None and (a.impl != "b200" or a.workload != "c25"):
+        ap.error("--dump-outputs applies to the default workload of the CUDA path (--impl b200 --workload c25)")
+    if a.steps is not None and a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.steps is None:
         a.steps = 100 if a.impl == "b200" else 2
     if a.warmup is None:
@@ -257,6 +268,83 @@ def cpu_baseline(a, raw_host, hours):
                       "({:.1f} s)".format(n, dt)}
 
 
+# ------------------------------------------------------------------------------------------------ output dump
+DUMP_SEED = 20260101
+# row caps of the dumped arrays: larger outputs are replaced by a fixed, seeded sample of their rows (sorted, so that
+# the order of the rows is kept).  Worst case in all: 12.6 + 2.6 + 16.8 + 3 x 4.5 + 2 x 4.5 + 0.2 MB < 64 MB
+DUMP_CAPS = {"flags_sample": 3 << 20, "contours": 1 << 16, "contour_points": 1 << 21, "events": 1 << 15,
+             "ring_points": 1 << 19, "ring_sizes": 1 << 15, "near": 1 << 12}
+DUMP_MAX_BYTES = 64 * 10**6
+
+
+def _sample_rows(n, cap):
+    """Row indices kept of an array of n rows: all of them, or `cap` drawn with DUMP_SEED (same n -> same rows)."""
+    if n <= cap:
+        return None
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, cap, replace=False))
+
+
+def dump_outputs(res, out_dir):
+    """Write what the detection path returned for one batch (a pipeline.BatchResult) as out_dir/<name>.npy, float32
+    where the values are exact in it and float64 otherwise, at most DUMP_MAX_BYTES in all:
+
+      flags_sample        float32 [<= 3 Mi]   int8 flag grids [3, T, nlat, nlon] (streamers, overturnings, cutoffs) at
+                                              sorted flat cell indices drawn with DUMP_SEED (all cells if there are few)
+      contours            float64 [C, 5]      job (time step * levels + level), closed, nx (exp_lon in columns), sum_y,
+                                              number of vertices
+      contour_points      float32 [P, 2]      x, y of every contour vertex (index coordinates of the extended grid)
+      <kind>_events       float64 [n, 17]     job, contour, ind1, ind2, box x0 y0 x1 y1, orientation, split, near,
+                                              sums (area, area x data, area x intensity, area x x, area x y, members)
+      <kind>_ring_sizes   float64 [n]         vertices of each event ring (streamers, cutoffs)
+      <kind>_ring_points  float32 [m, 2]      x, y of the ring vertices
+      near                float64 [k, 6]      streamer pairs decided within 1e-9 of a threshold (BatchResult.near)
+      counts              float64 [8]         time steps, contours, contour vertices, streamers, overturnings, cutoffs,
+                                              events that straddle the last meridian, near pairs (BatchResult.near_total)
+
+    Arrays longer than their DUMP_CAPS entry keep a seeded sample of their rows.  An array without rows (no near pairs,
+    no events of a kind) is not written: `counts` holds its length.  Returns the bytes written."""
+    import torch
+
+    from wavebreaking_b200 import detect
+
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+
+    def put(name, arr, cap_key, dtype):
+        arr = np.asarray(arr)
+        keep = _sample_rows(len(arr), DUMP_CAPS[cap_key])
+        arrays[name] = np.ascontiguousarray((arr if keep is None else arr[keep]).astype(dtype))
+
+    flat = res.flags.reshape(-1)
+    keep = _sample_rows(flat.numel(), DUMP_CAPS["flags_sample"])
+    if keep is not None:  # gathered where the grids are: those of a benchmark batch take about 1 GB
+        flat = flat[torch.from_numpy(keep).to(flat.device)]
+    put("flags_sample", flat.cpu().numpy(), "flags_sample", np.float32)
+
+    h = res.contours.host()
+    put("contours", np.c_[h["job"], h["closed"], h["nx"], h["sum_y"], np.diff(h["pt_off"])], "contours", np.float64)
+    put("contour_points", np.c_[h["x"], h["y"]], "contour_points", np.float32)
+    for kind in detect.KINDS:
+        t = res.tables[kind]
+        cols = np.c_[t.job, t.contour, t.ind1, t.ind2, t.box, t.orientation, t.split, t.near].astype(np.float64)
+        put(kind + "_events", np.c_[cols, t.sums].reshape(len(t), 17), "events", np.float64)
+        if t.rings is not None:
+            put(kind + "_ring_sizes", np.diff(t.rings.off), "ring_sizes", np.float64)
+            p = t.rings.packed
+            put(kind + "_ring_points", np.c_[p & 0xFFFF, p >> 16], "ring_points", np.float32)
+    put("near", res.near.reshape(-1, 6), "near", np.float64)
+    arrays = {k: v for k, v in arrays.items() if v.size}
+    arrays["counts"] = np.array([res.ntime, res.contours.ncontours, res.contours.npoints, *res.counts, res.n_split,
+                                 res.near_total], dtype=np.float64)
+
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError("output dump of {} bytes exceeds {} (DUMP_CAPS)".format(total, DUMP_MAX_BYTES))
+    for name, arr in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+    return total
+
+
 # ------------------------------------------------------------------------------------------------ GPU arm
 def _setup_ranks():
     import torch
@@ -341,7 +429,8 @@ def run_b200(a):
     depth = n_resident = a.depth
 
     def timed_region(detector, inputs, k_steps, shared_stream, profile, depth=depth):
-        """k_steps batches, `depth` in flight; returns (ms, per-kernel profile, kernel launches, per-batch counts)."""
+        """k_steps batches, `depth` in flight; returns (ms, per-kernel profile, kernel launches, per-batch counts,
+        result of the last batch: valid until the detector runs again)."""
         n_in = len(inputs)
         # warm-up: every slot allocates its arenas on first use, and every (slot, buffer) combination is captured
         # into its CUDA graph on its second submission
@@ -368,14 +457,18 @@ def run_b200(a):
         lib.cdll.wbk_prof_enable(0)
         launches = lib.cdll.wbk_launch_count() - launches0 + detector.graph_kernel_launches - g0
         # batches run on side streams: the host clock bounds the region
-        return max(e0.elapsed_time(e1), wall_ms), (_lib.prof_read(lib) if profile else {}), launches, cnts
+        return max(e0.elapsed_time(e1), wall_ms), (_lib.prof_read(lib) if profile else {}), launches, cnts, res
 
     # ---- headline region (value): every slot on its own stream, one CUDA graph per batch, so the latency-bound
     #      kernels of one batch overlap the FP64-bound smoothing of another
     log("inputs ready; device-resident leg")
-    ms, _, launches, counts = timed_region(det, slabs, K, shared_stream=a.serial, profile=False)
+    ms, _, launches, counts, last = timed_region(det, slabs, K, shared_stream=a.serial, profile=False)
     clocks = sampler.stop()
     log("device-resident leg done: {:.1f} ms for {} batches".format(ms, K))
+    if a.dump_outputs is not None and rank == 0:
+        nbytes = dump_outputs(last, a.dump_outputs)
+        log("outputs of the last timed batch: {:.1f} MB in {}".format(nbytes / 1e6, a.dump_outputs))
+    del last
     ms_max = _max_over_ranks(ms, world)
     value = world * K * T / (ms_max / 1000.0)
     # ---- the same batches on ONE stream with eager launches and CUDA events around every kernel: clean per-kernel
@@ -383,7 +476,7 @@ def run_b200(a):
     det_prof = pipeline.Detector(lat, lon, levels=[2.0], passes=a.passes, graphs=False)
     k_prof = min(K, 20)
     sampler = ClockSampler(local)
-    ms_ser, prof, _, counts_ser = timed_region(det_prof, slabs, k_prof, shared_stream=True, profile=True, depth=min(depth, 3))
+    ms_ser, prof, _, counts_ser, _ = timed_region(det_prof, slabs, k_prof, shared_stream=True, profile=True, depth=min(depth, 3))
     value_serial = world * k_prof * T / (_max_over_ranks(ms_ser, world) / 1000.0)
 
     # per-time-step work statistics (device counters of the batches) for the algorithmic byte counts
@@ -541,7 +634,7 @@ def run_b200(a):
         # (arenas grow to ~25 GB per slot on this field: three batches in flight)
         det.close()
         det = pipeline.Detector(lat, lon, levels=[2.0], passes=a.passes, graphs=graphs)
-        ms_st, _, _, cnt_st = timed_region(det, noisy, k_st, shared_stream=a.serial, profile=False, depth=min(n_resident, 3))
+        ms_st, _, _, cnt_st, _ = timed_region(det, noisy, k_st, shared_stream=a.serial, profile=False, depth=min(n_resident, 3))
         det.close()
         log("stress line done")
         extras["stress"] = {"value": world * k_st * T / (_max_over_ranks(ms_st, world) / 1000.0), "unit": UNIT,
