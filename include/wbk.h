@@ -222,7 +222,13 @@ int wbk_index_run(wbk_ctx* ctx, int njobs, int nlevels, const int* d_job_off, co
  * the events of the last wbk_index_run.  d_data / d_intensity: [ntime, nlat, nlon] (intensity may be NULL).
  * d_flags: NULL or int8 [3][ntime][nlat][nlon] (kind-major), zeroed here and set to 1 where an event of that
  * kind is present; events that straddle the last meridian (split = 1 in their record) are clipped on the
- * device (utils/index_utils.py:148-173) and their pieces rasterised too. */
+ * device (utils/index_utils.py:148-173) and their pieces rasterised too.
+ * The flags use the buffer of events.py:75-79, r = (dlon + dlat) / 4 degrees, measured in degrees: on a grid with
+ * dlon != dlat a lattice point is flagged when it is inside, on the boundary or closer than r (in degrees) to an
+ * edge.  Flag grids need params->dlon / params->dlat to be an exact ratio p / q of integers <= 64 with
+ * max(dlon, dlat) / min(dlon, dlat) < 3 (spacings within 1e-9 of each other count as equal); other spacings give
+ * WBK_ERR_INVALID with a message.  The property sums use the radius (dlon + dlat) / 4 in index units on any grid
+ * (index_utils.py:47-50). */
 int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* d_pt_off, const uint32_t* d_pts,
                       const double* d_coords, const void* d_data, int dtype, const void* d_intensity, int ntime,
                       int8_t* d_flags, const wbk_index_params* params, void* stream);
@@ -254,6 +260,15 @@ int wbk_events_fetch(wbk_ctx* ctx, int kind, int n, int* h_ints, double* h_f64, 
 int wbk_rasterize_rings(const int* d_xy, const int* d_ring_off, const int* d_ring_t, const double* d_ring_val,
                         int nrings, int nlat, int nlon, int ntime, double r2, int8_t* d_out_i8, double* d_out_f64,
                         int* d_owner, void* stream);
+
+/* processing/events.py:66-106 to_xarray on a regular grid with spacings dlon, dlat (degrees): like
+ * wbk_rasterize_rings (same rings, outputs and last-writer rule), with the buffer r = (dlon + dlat) / 4 degrees
+ * (events.py:75-79) measured in degrees, so that on a grid with dlon != dlat the buffer is an ellipse in index units.
+ * dlon / dlat must be an exact ratio p / q of integers <= 64 with max(dlon, dlat) / min(dlon, dlat) < 3 (spacings
+ * within 1e-9 of each other count as equal: r = 1/2 cell); other spacings give WBK_ERR_INVALID with a message. */
+int wbk_rasterize_rings_grid(const int* d_xy, const int* d_ring_off, const int* d_ring_t, const double* d_ring_val,
+                             int nrings, int nlat, int nlon, int ntime, double dlon, double dlat, int8_t* d_out_i8,
+                             double* d_out_f64, int* d_owner, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Sync-free batch plumbing (what wavebreaking_b200/pipeline.py uses): nothing below waits for the device.

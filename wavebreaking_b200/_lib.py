@@ -84,6 +84,8 @@ _SIGNATURES = {
     "wbk_events_fetch": (c_int, [c_void_p, c_int, c_int, POINTER(c_int), POINTER(c_double), POINTER(c_int), c_void_p]),
     "wbk_rasterize_rings": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_double,
                                     c_void_p, c_void_p, c_void_p, c_void_p]),
+    "wbk_rasterize_rings_grid": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_double,
+                                         c_double, c_void_p, c_void_p, c_void_p, c_void_p]),
     "wbk_workspace_bytes": (c_size_t, [POINTER(Caps), c_int, c_int, c_int]),
     "wbk_create": (c_int, [POINTER(c_void_p), POINTER(Caps), c_int, c_int, c_int, c_void_p, c_size_t]),
     "wbk_destroy": (c_int, [c_void_p]),

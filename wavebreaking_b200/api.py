@@ -631,8 +631,9 @@ def calculate_cutoffs(data, contour_level, contours=None, min_exp=5, intensity=N
 def to_xarray(data, events, flag="ones", name="flag", *args, **kwargs):
     """Flag the grid cells covered by events (processing/events.py:37-110)."""
     c = _Canon(data, kwargs, need_values=False)
-    if abs(c.dlon - c.dlat) > 1e-9 * abs(c.dlon):
-        raise ValueError("to_xarray needs dlon == dlat (the buffer radius of events.py:75-78 is isotropic in degrees)")
+    # the buffer of events.py:75-78 is measured in degrees: ValueError before any device work for spacings the
+    # rasteriser cannot measure it in exactly
+    detect.grid_ratio(c.dlon, c.dlat)
     if flag != "ones":
         try:
             set_val = np.asarray(events[flag].values, dtype=np.float64)
@@ -664,11 +665,12 @@ def to_xarray(data, events, flag="ones", name="flag", *args, **kwargs):
         ring_v = (np.ones(len(flat)) if flag == "ones" else set_val[ev_of_ring]).tolist()
     lib = _lib.get()
     if flag == "ones":
-        dev = detect.rasterize_rings(rings, ring_t, c.nlat, c.nlon, c.ntime, 0.5)
+        dev = detect.rasterize_rings(rings, ring_t, c.nlat, c.nlon, c.ntime, spacing=(c.dlon, c.dlat))
         out_dtype = np.dtype(np.int8)
     else:
         grid = torch.zeros((c.ntime, c.nlat, c.nlon), dtype=torch.float64, device=lib.device)
-        dev = detect.rasterize_rings(rings, ring_t, c.nlat, c.nlon, c.ntime, 0.5, values=(grid, ring_v))
+        dev = detect.rasterize_rings(rings, ring_t, c.nlat, c.nlon, c.ntime, spacing=(c.dlon, c.dlat),
+                                     values=(grid, ring_v))
         out_dtype = np.dtype(data.dtype)
     shape = tuple(len(data[d]) for d in data.dims)
     # the grid stays on the device until its values are read (a DataArray result is downloaded at once)

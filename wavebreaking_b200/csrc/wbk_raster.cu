@@ -2,6 +2,8 @@
 // Reference: wavebreaking/utils/index_utils.py:35-126 (calculate_properties) and
 // wavebreaking/processing/events.py:66-106 (to_xarray); buffer(r)+sjoin(contains) restated as
 // "inside (non-zero winding) or on the boundary or closer than r to an edge" (SURVEY.md A.5).
+#include <cmath>
+
 #include "wbk_ctx.cuh"
 
 struct RingView {
@@ -101,12 +103,38 @@ __device__ __forceinline__ int fold_x(int px, int nlon) {
   return px;
 }
 
+// The to_xarray buffer (events.py:75-79) on a grid with dlon : dlat = p : q (reduced): r = (dlon + dlat) / 4
+// degrees.  In index units a lattice point at (ex, ey) from an edge (dx, dy) is closer than r (in degrees) to the
+// edge's interior iff 16 p^2 q^2 C^2 < (p + q)^2 L, with C = dx ey - dy ex, L = p^2 dx^2 + q^2 dy^2 and the foot of
+// the perpendicular inside the edge (0 < D < L, D = p^2 ex dx + q^2 ey dy); closer than r to a vertex iff
+// 16 (p^2 ex^2 + q^2 ey^2) < (p + q)^2.  Below aspect 3 the vertex discs hold no lattice point but the vertex itself
+// (the host refuses other grids: grid_ratio), so GEOS's polygonal arcs cannot matter (SURVEY.md A.5).
+struct FlagMetric {
+  long long p2, q2;  // p^2, q^2 (p, q <= 64)
+  long long kc, kl;  // 16 p^2 q^2, (p + q)^2
+  int unit_ok;       // no lattice point off a diagonal unit step lies in the band: kc >= kl (p^2 + q^2)
+};
+
+__device__ __forceinline__ bool metric_near(const FlagMetric& m, long long ex, long long ey, long long dx, long long dy) {
+  const long long D = m.p2 * ex * dx + m.q2 * ey * dy, L = m.p2 * dx * dx + m.q2 * dy * dy;
+  if (D <= 0) return 16 * (m.p2 * ex * ex + m.q2 * ey * ey) < m.kl;
+  if (D >= L) {
+    const long long fx = ex - dx, fy = ey - dy;
+    return 16 * (m.p2 * fx * fx + m.q2 * fy * fy) < m.kl;
+  }
+  const long long C = dx * ey - dy * ex;
+  // kc C^2 reaches 2^94 for |C| < 2^33: exact in 128 bits
+  return C == 0 || (__int128)m.kc * C * C < (__int128)m.kl * L;
+}
+
 // Warp-cooperative scan of lattice row y over columns [bx0, bx0 + bw): on return acc[i] is the winding number
 // of (bx0 + i, y) (for points not on the boundary) and flg[i] has bit 0 / bit 1 set if the point is on the
-// boundary or closer than sqrt(r2a) / sqrt(r2b) to an edge.  R = floor(max radius).
+// boundary or closer than sqrt(r2a) / sqrt(r2b) to an edge.  ANISO: bit 1 is the to_xarray rule of `fm` instead
+// of sqrt(r2b).  rmax >= every radius in index units (for ANISO: >= r / min(dlon, dlat)), R = floor(rmax).
+template <bool ANISO>
 __device__ inline void raster_scan_row(const RingView& rv, int y, int bx0, int bw, int* acc, u32* flg, double r2a,
-                                       double r2b, double rmax, int R, const unsigned short* elist = nullptr,
-                                       int ecount = 0) {
+                                       double r2b, double rmax, int R, const FlagMetric& fm,
+                                       const unsigned short* elist = nullptr, int ecount = 0) {
   const int lane = wbk_lane();
   for (int i = lane; i < bw; i += 32) {
     acc[i] = 0;
@@ -141,10 +169,11 @@ __device__ inline void raster_scan_row(const RingView& rv, int y, int bx0, int b
         // boundary / near-edge candidates of this row
         if (y >= lo - R && y <= hi + R) {
           const long long len2 = (long long)dx * dx + (long long)dy * dy;
-          if (len2 <= 2 && rmax * rmax <= 0.5) {
+          if (len2 <= 2 && (ANISO ? r2a <= 0.5 && fm.unit_ok : rmax * rmax <= 0.5)) {
             // unit step of a contour ring with radii <= sqrt(1/2): every lattice point off the edge is at least
             // 1/sqrt(2) away, so only the end points qualify; the start vertex is marked here, the end vertex is the
-            // start of the next edge
+            // start of the next edge.  (ANISO: a diagonal step's off-edge neighbours stay out of the band while
+            // 16 p^2 q^2 >= (p + q)^2 (p^2 + q^2), i.e. up to aspect ~2.76.)
             const int idx = xa - bx0;
             if (ya == y && idx >= 0 && idx < bw) atomicOr(&flg[idx], 3u);
             continue;
@@ -186,6 +215,7 @@ __device__ inline void raster_scan_row(const RingView& rv, int y, int bx0, int b
                 bits = (c2 < r2a * l2 ? 1u : 0u) | (c2 < r2b * l2 ? 2u : 0u);
               }
             }
+            if (ANISO) bits = (bits & 1u) | (metric_near(fm, ex, ey, dx, dy) ? 2u : 0u);
             if (bits) atomicOr(&flg[px - bx0], bits);
           }
         }
@@ -228,12 +258,14 @@ __global__ void __launch_bounds__(1024) event_list_kernel(WbkIdx x, int J, int n
 #define RS_EDGE_CAP 8192     // edge incidences in the row buckets
 #define RS_PRE 4             // 32-column groups of a row whose field values are prefetched before the scan
 
-template <typename T>
+// r2_flag: the squared flag radius in cells (dlon == dlat), or with ANISO the squared extent r / min(dlon, dlat) of
+// fm's band, which is below one cell: R and the margins below are those of r2_prop wherever that is >= 1 cell
+template <typename T, bool ANISO>
 __global__ void __launch_bounds__(RS_THREADS, 3)
 events_raster_kernel(WbkDev d, WbkIdx x, const int* __restrict__ job_off, const int* __restrict__ pt_off,
                      const u32* __restrict__ pts, const double* __restrict__ area, const T* __restrict__ data,
                      const T* __restrict__ intensity, int8_t* __restrict__ flags, int ntime, int nlevels, int J,
-                     int njobs, double r2_prop, double r2_flag, int rowcap) {
+                     int njobs, double r2_prop, double r2_flag, FlagMetric fm, int rowcap) {
   WBK_DYN_SMEM(int, sm);
   __shared__ int s_box[5];
   __shared__ int s_scan[40];
@@ -353,7 +385,7 @@ events_raster_kernel(WbkDev d, WbkIdx x, const int* __restrict__ job_off, const 
         }
       }
       int8_t* frow = flags ? flags + (((size_t)kind * ntime + t) * nlat + y) * nlon : nullptr;
-      if (!boxfast) raster_scan_row(rv, y, cx0, cw, acc, flg, r2_prop, r2_flag, rmax, R, elist, ecount);
+      if (!boxfast) raster_scan_row<ANISO>(rv, y, cx0, cw, acc, flg, r2_prop, r2_flag, rmax, R, fm, elist, ecount);
       const double a = area[y];
       int row_members = 0;
       auto visit = [&](int i, double dv) {
@@ -688,9 +720,12 @@ split_events_kernel(WbkDev d, WbkIdx x, const int* __restrict__ pt_off, const u3
   }
 }
 
-// rasterise the split pieces (real grid, r = 1/2 cell: processing/events.py:75-79) into the flag grids
+// rasterise the split pieces (real grid, r = 1/2 cell or with ANISO the rule of fm: processing/events.py:75-79) into
+// the flag grids; rf: r / min(dlon, dlat) in cells (< 1)
+template <bool ANISO>
 __global__ void __launch_bounds__(RS_THREADS)
-split_raster_kernel(WbkIdx x, int nlat, int nlon, int ntime, int8_t* __restrict__ flags, int rowcap, int* status) {
+split_raster_kernel(WbkIdx x, int nlat, int nlon, int ntime, int8_t* __restrict__ flags, int rowcap, int* status,
+                    FlagMetric fm, double rf) {
   WBK_DYN_SMEM(int, sm);
   __shared__ int s_box[4];
   const int tid = threadIdx.x, lane = wbk_lane(), warp = wbk_warp(), nwarps = blockDim.x >> 5;
@@ -733,9 +768,10 @@ split_raster_kernel(WbkIdx x, int nlat, int nlon, int ntime, int8_t* __restrict_
     const int bw = bx1 - bx0 + 1;
     if (rv.n > 0 && bw > 0) {
       for (int y = by0 + warp; y <= by1; y += nwarps) {
-        raster_scan_row(rv, y, bx0, bw, acc, flg, 0.25, 0.25, 0.5, 0);
+        if (ANISO) raster_scan_row<true>(rv, y, bx0, bw, acc, flg, rf * rf, rf * rf, rf, 0, fm);
+        else raster_scan_row<false>(rv, y, bx0, bw, acc, flg, 0.25, 0.25, 0.5, 0, fm);
         for (int i = lane; i < bw; i += 32)
-          if (acc[i] != 0 || (flg[i] & 1u)) flags[(((size_t)kind * ntime + t) * nlat + y) * nlon + (bx0 + i)] = 1;
+          if (acc[i] != 0 || (flg[i] & (ANISO ? 2u : 1u))) flags[(((size_t)kind * ntime + t) * nlat + y) * nlon + (bx0 + i)] = 1;
         __syncwarp();
       }
     }
@@ -745,6 +781,48 @@ split_raster_kernel(WbkIdx x, int nlat, int nlon, int ntime, int8_t* __restrict_
 
 static int raster_rowcap(int W) { return (W + 2 + 31) & ~31; }
 
+// dlon : dlat as the reduced ratio p : q of the to_xarray metric (FlagMetric).  Spacings within 1e-9 (relative) of
+// each other are the isotropic grid p = q = 1 (fm->p2 == 0: the radius-in-cells path).  Otherwise the ratio of the two
+// doubles must be exactly p / q with p, q <= 64 (so the products of metric_near stay exact) and max / min < 3 (vertex
+// discs without lattice points); anything else sets the error (prefixed with `who`) and returns WBK_ERR_INVALID.
+static int grid_ratio(const char* who, double dlon, double dlat, FlagMetric* fm) {
+  *fm = FlagMetric{0, 0, 0, 0, 0};
+  if (!(dlon > 0) || !(dlat > 0) || !std::isfinite(dlon) || !std::isfinite(dlat)) {
+    wbk_set_error("%s: grid spacings dlon=%.17g, dlat=%.17g must be positive and finite", who, dlon, dlat);
+    return WBK_ERR_INVALID;
+  }
+  if (fabs(dlon - dlat) <= 1e-9 * fabs(dlon)) return WBK_OK;
+  // dlon / dlat = (a / b) * 2^k with a, b odd integers (53-bit significands)
+  int ea, eb;
+  unsigned long long a = (unsigned long long)ldexp(frexp(dlon, &ea), 53);
+  unsigned long long b = (unsigned long long)ldexp(frexp(dlat, &eb), 53);
+  int k = ea - eb;
+  while (!(a & 1)) { a >>= 1; ++k; }
+  while (!(b & 1)) { b >>= 1; --k; }
+  unsigned long long g = a, h = b;
+  while (h) { const unsigned long long t = g % h; g = h; h = t; }
+  a /= g;
+  b /= g;
+  while (k > 0 && a <= 64) { a <<= 1; --k; }
+  while (k < 0 && b <= 64) { b <<= 1; ++k; }
+  if (k != 0 || a > 64 || b > 64) {
+    wbk_set_error("%s: dlon=%.17g / dlat=%.17g is not a ratio p/q of integers <= 64", who, dlon, dlat);
+    return WBK_ERR_INVALID;
+  }
+  const long long p = (long long)a, q = (long long)b;
+  if (p >= 3 * q || q >= 3 * p) {
+    wbk_set_error("%s: dlon=%.17g, dlat=%.17g: flag grids need an aspect ratio max(dlon, dlat) / min(dlon, dlat) < 3",
+                  who, dlon, dlat);
+    return WBK_ERR_INVALID;
+  }
+  fm->p2 = p * p;
+  fm->q2 = q * q;
+  fm->kc = 16 * p * p * q * q;
+  fm->kl = (p + q) * (p + q);
+  fm->unit_ok = fm->kc >= fm->kl * (fm->p2 + fm->q2);
+  return WBK_OK;
+}
+
 
 extern "C" int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* d_pt_off, const uint32_t* d_pts,
                                  const double* d_coords, const void* d_data, int dtype, const void* d_intensity,
@@ -753,21 +831,26 @@ extern "C" int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* 
     wbk_set_error("wbk_events_raster: invalid argument");
     return WBK_ERR_INVALID;
   }
+  FlagMetric fm;
+  if (d_flags) {
+    const int rc = grid_ratio("wbk_events_raster", prm->dlon, prm->dlat, &fm);
+    if (rc != WBK_OK) return rc;
+  } else {
+    fm = FlagMetric{0, 0, 0, 0, 0};
+  }
+  const bool aniso = fm.p2 != 0;
   cudaStream_t st = (cudaStream_t)stream;
   WbkDev& d = ctx->d;
   const int njobs = ctx->njobs, J = ctx->caps.max_jobs;
   if (d_flags && ntime > 0)
     WBK_CUDA_CHECK(cudaMemsetAsync(d_flags, 0, (size_t)3 * ntime * d.nlat * d.nlon, st));
   if (njobs == 0) return WBK_OK;
-  if (d_flags && fabs(prm->dlon - prm->dlat) > 1e-9 * fabs(prm->dlon)) {
-    wbk_set_error("wbk_events_raster: to_xarray flags need dlon == dlat (buffer radius is isotropic in degrees)");
-    return WBK_ERR_INVALID;
-  }
   WBK_CUDA_CHECK(cudaMemsetAsync(ctx->x.split_count, 0, 16, st));  // cursors of the meridian split (filled by the rasteriser)
   WBK_LAUNCH(KID_EVENT_LIST, event_list_kernel, dim3(1), dim3(1024), 0, st, ctx->x, J, njobs);
   WBK_LAUNCH_CHECK();
   const double r_prop = (prm->dlon + prm->dlat) / 2.0 / 2.0;  // index units (index_utils.py:47-50)
-  const double r_flag = d_flags ? ((prm->dlon + prm->dlat) / 2.0 / 2.0) / prm->dlon : r_prop;  // degrees -> cells
+  // degrees -> cells (anisotropic: the larger of the band's two extents, r / dlon and r / dlat)
+  const double r_flag = !d_flags ? r_prop : r_prop / (aniso ? fmin(prm->dlon, prm->dlat) : prm->dlon);
   const int rowcap = raster_rowcap(d.W) < RS_EVENT_ROWCAP ? raster_rowcap(d.W) : RS_EVENT_ROWCAP;
   int nwarps = RS_THREADS / 32;
   const size_t smem = (size_t)nwarps * 2 * rowcap * sizeof(int) + (size_t)RS_RING_CAP * sizeof(u32) +
@@ -775,15 +858,17 @@ extern "C" int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* 
   const double* area = d_coords + 3 * (size_t)d.nlat;
   const int grid = 148 * 9;
   if (dtype == WBK_F32) {
-    WBK_CUDA_CHECK(cudaFuncSetAttribute(events_raster_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    WBK_LAUNCH(KID_EVENTS_RASTER, events_raster_kernel<float>, dim3(grid), dim3(RS_THREADS), smem, st, d, ctx->x, d_job_off, d_pt_off,
+    auto kern = aniso ? events_raster_kernel<float, true> : events_raster_kernel<float, false>;
+    WBK_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    WBK_LAUNCH(KID_EVENTS_RASTER, kern, dim3(grid), dim3(RS_THREADS), smem, st, d, ctx->x, d_job_off, d_pt_off,
                (const u32*)d_pts, area, (const float*)d_data, (const float*)d_intensity, d_flags, ntime, ctx->nlevels, J,
-               njobs, r_prop * r_prop, r_flag * r_flag, rowcap);
+               njobs, r_prop * r_prop, r_flag * r_flag, fm, rowcap);
   } else if (dtype == WBK_F64) {
-    WBK_CUDA_CHECK(cudaFuncSetAttribute(events_raster_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    WBK_LAUNCH(KID_EVENTS_RASTER, events_raster_kernel<double>, dim3(grid), dim3(RS_THREADS), smem, st, d, ctx->x, d_job_off, d_pt_off,
+    auto kern = aniso ? events_raster_kernel<double, true> : events_raster_kernel<double, false>;
+    WBK_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    WBK_LAUNCH(KID_EVENTS_RASTER, kern, dim3(grid), dim3(RS_THREADS), smem, st, d, ctx->x, d_job_off, d_pt_off,
                (const u32*)d_pts, area, (const double*)d_data, (const double*)d_intensity, d_flags, ntime, ctx->nlevels,
-               J, njobs, r_prop * r_prop, r_flag * r_flag, rowcap);
+               J, njobs, r_prop * r_prop, r_flag * r_flag, fm, rowcap);
   } else {
     wbk_set_error("wbk_events_raster: unsupported dtype");
     return WBK_ERR_INVALID;
@@ -797,9 +882,10 @@ extern "C" int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* 
     WBK_LAUNCH_CHECK();
     const int rc2 = raster_rowcap(d.nlon);
     const size_t smem2 = (size_t)(RS_THREADS / 32) * 2 * rc2 * sizeof(int);
-    WBK_CUDA_CHECK(cudaFuncSetAttribute(split_raster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
-    WBK_LAUNCH(KID_SPLIT_RASTER, split_raster_kernel, dim3(148 * 2), dim3(RS_THREADS), smem2, st, ctx->x, d.nlat, d.nlon,
-               ntime, d_flags, rc2, d.status);
+    auto split_raster = aniso ? split_raster_kernel<true> : split_raster_kernel<false>;
+    WBK_CUDA_CHECK(cudaFuncSetAttribute(split_raster, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
+    WBK_LAUNCH(KID_SPLIT_RASTER, split_raster, dim3(148 * 2), dim3(RS_THREADS), smem2, st, ctx->x, d.nlat, d.nlon,
+               ntime, d_flags, rc2, d.status, fm, r_flag);
     WBK_LAUNCH_CHECK();
   }
   return WBK_OK;
@@ -821,9 +907,12 @@ extern "C" int wbk_split_clip(wbk_ctx* ctx, const int* d_pt_off, const uint32_t*
 }
 
 // ------------------------------------------------------------------------------------------ generic rings
+// r2: squared radius in cells, or with ANISO the squared extent of fm's band (r / min(dlon, dlat))^2
+template <bool ANISO>
 __global__ void __launch_bounds__(RS_THREADS)
 rings_raster_kernel(const int* __restrict__ xy, const int* __restrict__ ring_off, const int* __restrict__ ring_t,
-                    int nrings, int nlat, int nlon, int ntime, double r2, int8_t* out_i8, int* owner, int rowcap) {
+                    int nrings, int nlat, int nlon, int ntime, double r2, int8_t* out_i8, int* owner, int rowcap,
+                    FlagMetric fm) {
   WBK_DYN_SMEM(int, sm);
   __shared__ int s_box[4];
   const int tid = threadIdx.x, lane = wbk_lane(), warp = wbk_warp(), nwarps = blockDim.x >> 5;
@@ -860,9 +949,9 @@ rings_raster_kernel(const int* __restrict__ xy, const int* __restrict__ ring_off
     const int bw = bx1 - bx0 + 1;
     if (rv.n > 0 && bw > 0 && t >= 0 && t < ntime) {
       for (int y = by0 + warp; y <= by1; y += nwarps) {
-        raster_scan_row(rv, y, bx0, bw, acc, flg, r2, r2, rmax, R);
+        raster_scan_row<ANISO>(rv, y, bx0, bw, acc, flg, r2, r2, rmax, R, fm);
         for (int i = lane; i < bw; i += 32) {
-          if (acc[i] != 0 || (flg[i] & 1u)) {
+          if (acc[i] != 0 || (flg[i] & (ANISO ? 2u : 1u))) {
             const size_t o = ((size_t)t * nlat + y) * nlon + (bx0 + i);
             if (out_i8) out_i8[o] = 1;
             if (owner) atomicMax(&owner[o], r);
@@ -885,12 +974,13 @@ __global__ void owner_apply_kernel(const int* __restrict__ owner, const double* 
   }
 }
 
-extern "C" int wbk_rasterize_rings(const int* d_xy, const int* d_ring_off, const int* d_ring_t,
-                                   const double* d_ring_val, int nrings, int nlat, int nlon, int ntime, double r2,
-                                   int8_t* d_out_i8, double* d_out_f64, int* d_owner, void* stream) {
+// r2: squared radius in cells (fm.p2 == 0), or the squared extent of fm's band
+static int rasterize_rings(const char* who, const int* d_xy, const int* d_ring_off, const int* d_ring_t,
+                           const double* d_ring_val, int nrings, int nlat, int nlon, int ntime, double r2,
+                           const FlagMetric& fm, int8_t* d_out_i8, double* d_out_f64, int* d_owner, void* stream) {
   if (nrings < 0 || nlat < 1 || nlon < 1 || ntime < 0 || !(r2 >= 0) || (!d_out_i8 && !d_out_f64) ||
       (d_out_f64 && (!d_owner || !d_ring_val)) || (nrings > 0 && (!d_xy || !d_ring_off || !d_ring_t))) {
-    wbk_set_error("wbk_rasterize_rings: invalid argument");
+    wbk_set_error("%s: invalid argument", who);
     return WBK_ERR_INVALID;
   }
   if (nrings == 0 || ntime == 0) return WBK_OK;
@@ -898,7 +988,7 @@ extern "C" int wbk_rasterize_rings(const int* d_xy, const int* d_ring_off, const
   const int rowcap = raster_rowcap(nlon);
   const size_t smem = (size_t)(RS_THREADS / 32) * 2 * rowcap * sizeof(int);
   if (smem > 200 * 1024) {
-    wbk_set_error("wbk_rasterize_rings: grid width %d too large for the row buffers", nlon);
+    wbk_set_error("%s: grid width %d too large for the row buffers", who, nlon);
     return WBK_ERR_CAPACITY;
   }
   const size_t ncell = (size_t)ntime * nlat * nlon;
@@ -906,14 +996,35 @@ extern "C" int wbk_rasterize_rings(const int* d_xy, const int* d_ring_off, const
     WBK_LAUNCH(KID_OWNER, owner_fill_kernel, dim3(592), dim3(256), 0, st, d_owner, ncell, -1);
     WBK_LAUNCH_CHECK();
   }
-  WBK_CUDA_CHECK(cudaFuncSetAttribute(rings_raster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  auto kern = fm.p2 != 0 ? rings_raster_kernel<true> : rings_raster_kernel<false>;
+  WBK_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int grid = nrings < 148 * 4 ? nrings : 148 * 4;
-  WBK_LAUNCH(KID_RINGS_RASTER, rings_raster_kernel, dim3(grid), dim3(RS_THREADS), smem, st, d_xy, d_ring_off, d_ring_t, nrings, nlat, nlon,
-             ntime, r2, d_out_i8, d_out_f64 ? d_owner : (int*)nullptr, rowcap);
+  WBK_LAUNCH(KID_RINGS_RASTER, kern, dim3(grid), dim3(RS_THREADS), smem, st, d_xy, d_ring_off, d_ring_t, nrings, nlat,
+             nlon, ntime, r2, d_out_i8, d_out_f64 ? d_owner : (int*)nullptr, rowcap, fm);
   WBK_LAUNCH_CHECK();
   if (d_out_f64) {
     WBK_LAUNCH(KID_OWNER, owner_apply_kernel, dim3(592), dim3(256), 0, st, (const int*)d_owner, d_ring_val, d_out_f64, ncell);
     WBK_LAUNCH_CHECK();
   }
   return WBK_OK;
+}
+
+extern "C" int wbk_rasterize_rings(const int* d_xy, const int* d_ring_off, const int* d_ring_t,
+                                   const double* d_ring_val, int nrings, int nlat, int nlon, int ntime, double r2,
+                                   int8_t* d_out_i8, double* d_out_f64, int* d_owner, void* stream) {
+  return rasterize_rings("wbk_rasterize_rings", d_xy, d_ring_off, d_ring_t, d_ring_val, nrings, nlat, nlon, ntime, r2,
+                         FlagMetric{0, 0, 0, 0, 0}, d_out_i8, d_out_f64, d_owner, stream);
+}
+
+extern "C" int wbk_rasterize_rings_grid(const int* d_xy, const int* d_ring_off, const int* d_ring_t,
+                                        const double* d_ring_val, int nrings, int nlat, int nlon, int ntime,
+                                        double dlon, double dlat, int8_t* d_out_i8, double* d_out_f64, int* d_owner,
+                                        void* stream) {
+  FlagMetric fm;
+  const int rc = grid_ratio("wbk_rasterize_rings_grid", dlon, dlat, &fm);
+  if (rc != WBK_OK) return rc;
+  // isotropic: r = (dlon + dlat) / 4 degrees is half a cell; otherwise the band reaches r / min(dlon, dlat) cells
+  const double rcell = fm.p2 == 0 ? 0.5 : (dlon + dlat) / 4.0 / fmin(dlon, dlat);
+  return rasterize_rings("wbk_rasterize_rings_grid", d_xy, d_ring_off, d_ring_t, d_ring_val, nrings, nlat, nlon, ntime,
+                         rcell * rcell, fm, d_out_i8, d_out_f64, d_owner, stream);
 }

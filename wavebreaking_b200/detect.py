@@ -7,6 +7,7 @@ Columnar layer under the drop-in API (``wavebreaking_b200.api``).  A *job* is on
 
 import ctypes
 from dataclasses import dataclass
+from fractions import Fraction
 
 import numpy as np
 import torch
@@ -363,8 +364,41 @@ def event_rings(cs, table):
     return rings
 
 
-def rasterize_rings(rings, ring_t, nlat, nlon, ntime, r_cells, out_i8=None, values=None):
-    """OR lattice rings into an int8 grid (or write ``values`` into a float64 grid, last ring wins)."""
+def grid_ratio(dlon, dlat):
+    """``dlon : dlat`` as the reduced ratio ``(p, q)`` that the to_xarray buffer of an anisotropic grid is measured
+    in (the rule of ``wbk_events_raster`` / ``wbk_rasterize_rings_grid``; raises ``ValueError`` on grids they refuse).
+
+    Spacings within 1e-9 (relative) of each other are the isotropic grid ``(1, 1)``.  Otherwise ``dlon / dlat`` must
+    be exactly ``p / q`` with ``p, q <= 64`` (the integer products of the membership test stay exact) and
+    ``max(dlon, dlat) / min(dlon, dlat) < 3`` (the buffer discs around vertices hold no other grid point)."""
+    dlon, dlat = float(dlon), float(dlat)
+    if not (np.isfinite(dlon) and np.isfinite(dlat) and dlon > 0 and dlat > 0):
+        raise ValueError("grid spacings dlon={!r}, dlat={!r} must be positive and finite".format(dlon, dlat))
+    if abs(dlon - dlat) <= 1e-9 * abs(dlon):
+        return 1, 1
+    ratio = Fraction(dlon) / Fraction(dlat)
+    p, q = ratio.numerator, ratio.denominator
+    if p > 64 or q > 64:
+        raise ValueError("flag grids need dlon / dlat to be an exact ratio p/q of integers <= 64; "
+                         "dlon={!r}, dlat={!r}".format(dlon, dlat))
+    if max(p, q) >= 3 * min(p, q):
+        raise ValueError("flag grids need an aspect ratio max(dlon, dlat) / min(dlon, dlat) < 3; "
+                         "dlon={!r}, dlat={!r}".format(dlon, dlat))
+    return p, q
+
+
+def rasterize_rings(rings, ring_t, nlat, nlon, ntime, r_cells=None, out_i8=None, values=None, spacing=None):
+    """OR lattice rings into an int8 grid (or write ``values`` into a float64 grid, last ring wins).
+
+    The buffer is ``r_cells`` grid cells, or with ``spacing=(dlon, dlat)`` the to_xarray buffer
+    ``(dlon + dlat) / 4`` measured in degrees (``wbk_rasterize_rings_grid``; see :func:`grid_ratio`)."""
+    if (r_cells is None) == (spacing is None):
+        raise ValueError("rasterize_rings: give exactly one of r_cells and spacing")
+    if spacing is not None:
+        grid_ratio(*spacing)
+        fn, radius = "wbk_rasterize_rings_grid", [float(spacing[0]), float(spacing[1])]
+    else:
+        fn, radius = "wbk_rasterize_rings", [float(r_cells) ** 2]
     lib = _lib.get()
     dev = lib.device
     n = len(rings)
@@ -380,14 +414,14 @@ def rasterize_rings(rings, ring_t, nlat, nlon, ntime, r_cells, out_i8=None, valu
     d_off = torch.from_numpy(off).to(dev)
     d_t = torch.from_numpy(np.ascontiguousarray(ring_t, dtype=np.int32)).to(dev)
     if values is None:
-        lib.call("wbk_rasterize_rings", _lib.ptr(d_xy), _lib.ptr(d_off), _lib.ptr(d_t), None, n, nlat, nlon, ntime,
-                 float(r_cells) ** 2, _lib.ptr(out_i8), None, None, lib.stream())
+        lib.call(fn, _lib.ptr(d_xy), _lib.ptr(d_off), _lib.ptr(d_t), None, n, nlat, nlon, ntime, *radius,
+                 _lib.ptr(out_i8), None, None, lib.stream())
         return out_i8
     out, vals = values
     d_val = torch.from_numpy(np.ascontiguousarray(vals, dtype=np.float64)).to(dev)
     owner = torch.empty((ntime, nlat, nlon), dtype=torch.int32, device=dev)
-    lib.call("wbk_rasterize_rings", _lib.ptr(d_xy), _lib.ptr(d_off), _lib.ptr(d_t), _lib.ptr(d_val), n, nlat, nlon,
-             ntime, float(r_cells) ** 2, None, _lib.ptr(out), _lib.ptr(owner), lib.stream())
+    lib.call(fn, _lib.ptr(d_xy), _lib.ptr(d_off), _lib.ptr(d_t), _lib.ptr(d_val), n, nlat, nlon, ntime, *radius,
+             None, _lib.ptr(out), _lib.ptr(owner), lib.stream())
     return out
 
 

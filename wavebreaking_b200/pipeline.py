@@ -168,6 +168,8 @@ class Detector:
         self.params = dict(geo_dis=geo_dis, cont_dis=cont_dis, range_group=range_group, ot_min_exp=ot_min_exp,
                            co_min_exp=co_min_exp)
         self.want_flags = want_flags
+        if want_flags:
+            detect.grid_ratio(self.dlon, self.dlat)  # flag grids need spacings wbk_events_raster can measure in
         # smoothing that also leaves the marching-squares bit planes (wbk_smooth_contours): the contour stage then
         # does not re-read the smoothed field.  fuse=False runs wbk_smooth + wbk_contours (same results).
         self.fuse = bool(fuse)
