@@ -307,6 +307,18 @@ int wbk_split_fetch(wbk_ctx* ctx, int* d_ring_ev, int* d_ring_off, int* d_xy, in
  * 4 * ceil(ncells / 32) bytes; d_flags 16-byte aligned, d_packed 4-byte aligned. */
 int wbk_pack_flags(const int8_t* d_flags, uint8_t* d_packed, long long ncells, void* stream);
 
+/* Occurrence counts behind a flag-frequency climatology.
+ * d_flags : int8 [nkinds][ntime][ncells], the layout wbk_events_raster writes (nkinds = 3, kind stride ntime * ncells,
+ *           where ntime is the batch length, not the capacity of the buffer).
+ * d_group : int32 [ntime] (device): the group of each time step in [0, ngroups), or -1 = step not counted.  Any value
+ *           outside [0, ngroups) is ignored like -1.
+ * d_counts: uint32 [ngroups][nkinds][ncells]; counts[g][k][c] += #{t : group[t] == g && flags[k][t][c] != 0}.
+ * Several streams may add into the same d_counts at once (atomic adds).  Nothing is zeroed.  16-byte loads are used
+ * when ncells % 16 == 0 and d_flags is 16-byte aligned, byte loads otherwise.  ntime == 0 or ncells == 0 is a no-op.
+ * Asynchronous. */
+int wbk_flag_counts(const int8_t* d_flags, int nkinds, int ntime, long long ncells, const int* d_group, int ngroups,
+                    uint32_t* d_counts, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * Per-kernel device timing (CUDA events on the launching stream around every kernel launch of the
  * library).  wbk_prof_enable(1) starts collecting, wbk_prof_read synchronises the device and returns, for

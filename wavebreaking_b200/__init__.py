@@ -7,7 +7,7 @@ Same public names as ``wavebreaking/__init__.py:19-34`` (plotting is out of scop
 __version__ = "0.1.0"
 
 _API = ("calculate_momentum_flux", "calculate_smoothed_field", "to_xarray", "track_events", "event_tracking",
-        "calculate_contours", "calculate_streamers", "calculate_overturnings", "calculate_cutoffs", "combine_shared")
+        "calculate_contours", "calculate_streamers", "calculate_overturnings", "calculate_cutoffs", "combine_shared", "flag_frequency")
 
 
 def __getattr__(name):  # lazy: importing the package must not need torch / a GPU

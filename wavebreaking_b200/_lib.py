@@ -79,6 +79,7 @@ _SIGNATURES = {
     "wbk_split_clip": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "wbk_split_fetch": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "wbk_pack_flags": (c_int, [c_void_p, c_void_p, ctypes.c_longlong, c_void_p]),
+    "wbk_flag_counts": (c_int, [c_void_p, c_int, c_int, ctypes.c_longlong, c_void_p, c_int, c_void_p, c_void_p]),
     "wbk_near_list": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "wbk_events_counts": (c_int, [c_void_p, POINTER(c_int), POINTER(c_int), c_void_p]),
     "wbk_events_fetch": (c_int, [c_void_p, c_int, c_int, POINTER(c_int), POINTER(c_double), POINTER(c_int), c_void_p]),

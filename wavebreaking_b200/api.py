@@ -24,7 +24,7 @@ logger = logging.getLogger(__name__)
 __all__ = [
     "calculate_smoothed_field", "calculate_momentum_flux", "calculate_contours", "calculate_streamers",
     "calculate_overturnings", "calculate_cutoffs", "to_xarray", "track_events", "event_tracking", "combine_shared",
-    "check_argument_types", "get_dimension_attributes", "check_empty_dataframes",
+    "check_argument_types", "get_dimension_attributes", "check_empty_dataframes", "flag_frequency",
 ]
 
 _FIELD = "field"
@@ -673,12 +673,62 @@ def to_xarray(data, events, flag="ones", name="flag", *args, **kwargs):
                                      values=(grid, ring_v))
         out_dtype = np.dtype(data.dtype)
     shape = tuple(len(data[d]) for d in data.dims)
-    # the grid stays on the device until its values are read (a DataArray result is downloaded at once)
+    # the grid stays on the device until its values are read (a DataArray result is downloaded at once).  The int8
+    # grid is also offered as `device` (flag_frequency counts it there); without device_meta no index function takes it
     lazy = compat.LazyValues(shape, out_dtype,
-                             lambda: np.ascontiguousarray(c.to_input_layout(_to_host(dev)).astype(out_dtype, copy=False)))
+                             lambda: np.ascontiguousarray(c.to_input_layout(_to_host(dev)).astype(out_dtype, copy=False)),
+                             device=dev if flag == "ones" else None)
     res = compat.like(data, lazy, data.dims, name=name, attrs=dict(getattr(data, "attrs", {}) or {}))
     res.attrs["long_name"] = "flag wave breaking"
     return res
+
+
+@check_argument_types(["flag_data"], [_FIELD])
+@get_dimension_attributes("flag_data")
+def flag_frequency(flag_data, months=None, *args, **kwargs):
+    """Flag frequency: the percentage of time steps in which each grid cell is flagged.
+
+    ``flag_data``: the int8 output of ``to_xarray(..., flag="ones")`` (any other dtype raises TypeError); a result of
+    ``to_xarray`` that still lives on the device is counted there, without a download.  ``months``: count only the
+    time steps whose month (1-12, from the time coordinate, which then has to be datetime64) is in this list.
+    Returns a (lat, lon) array in ``flag_data``'s dimension order and orientation, float64 percent (NaN when no time
+    step is selected).  No smoothing is applied (``calculate_smoothed_field`` can be called on the result).
+
+    This is the frequency the reference's ``plot_clim`` draws, as this project defines it: 100 * (number of selected
+    steps with a nonzero flag) / (number of selected steps).  The reference's own formula could not be compared here
+    (it is not installed), so small differences in its normalisation are possible.
+    """
+    if np.dtype(flag_data.dtype) != np.int8:
+        raise TypeError("flag_data has to be the int8 output of to_xarray(..., flag='ones'), got dtype {}".format(
+            np.dtype(flag_data.dtype)))
+    c = _Canon(flag_data, kwargs, need_values=False)
+    if months is None:
+        group = np.zeros(c.ntime, dtype=np.int32)
+    else:
+        if not np.issubdtype(c.time.dtype, np.datetime64):
+            raise ValueError("months needs a datetime64 time coordinate, got dtype {}".format(c.time.dtype))
+        month = c.time.astype("datetime64[M]").astype(np.int64) % 12 + 1
+        group = np.where(np.isin(month, np.asarray(months, dtype=np.int64).ravel()), 0, -1).astype(np.int32)
+    lib = _lib.get()
+    lazy = getattr(flag_data, "_lazy", None)
+    if lazy is not None and lazy.device is not None and getattr(flag_data, "_values", None) is None:
+        grid = lazy.device  # int8 [time, lat, lon], ascending coordinates: counted where it is
+    else:
+        host = np.transpose(np.asarray(flag_data.values), c.order)
+        host = host[:, ::-1 if c.flip_lat else 1, ::-1 if c.flip_lon else 1]
+        grid = torch.from_numpy(np.ascontiguousarray(host)).to(lib.device)
+    counts = torch.zeros((c.nlat, c.nlon), dtype=torch.int32, device=lib.device)
+    dev_group = torch.from_numpy(group).to(lib.device)
+    lib.call("wbk_flag_counts", _lib.ptr(grid), 1, c.ntime, c.nlat * c.nlon, _lib.ptr(dev_group), 1, _lib.ptr(counts),
+             lib.stream())
+    from . import pipeline
+
+    freq = pipeline._percent(_to_host(counts).view(np.uint32)[None], [int((group == 0).sum())])
+    freq = c.to_input_layout(freq)  # [1, lat, lon] -> the input's dimension order, with a time axis of length 1
+    dims = tuple(d for d in flag_data.dims if d != c.time_name)
+    values = np.ascontiguousarray(freq.reshape([freq.shape[i] for i, d in enumerate(flag_data.dims) if d != c.time_name]))
+    return compat.like(flag_data, values, dims, name="flag_frequency",
+                       attrs={"long_name": "flag frequency", "units": "%"})
 
 
 @check_argument_types(["events"], [_PANDAS])

@@ -55,7 +55,8 @@ class _Coord:
 class LazyValues:
     """Values that still live on the device: ``load()`` brings them to the host (once) as a numpy array in the
     Field's dimension order.  ``device`` is the canonical device tensor [time, lat, lon] (ascending lat / lon) that
-    the next API call can use without any upload."""
+    the next API call can use without any upload; the index functions take it only when ``device_meta`` matches
+    (``to_xarray``'s int8 grid has none and is read by ``flag_frequency`` alone)."""
 
     def __init__(self, shape, dtype, load, device=None, device_meta=None):
         self.shape, self.dtype, self._load = tuple(shape), np.dtype(dtype), load

@@ -248,6 +248,140 @@ extern "C" int wbk_pack_flags(const int8_t* d_flags, uint8_t* d_packed, long lon
 }
 
 // ------------------------------------------------------------------------------------------------------------
+// Occurrence counts behind a flag-frequency climatology: counts[g][k][c] += #{t : group[t] == g, flags[k][t][c] != 0}.
+// A thread owns consecutive cells of one kind and walks the time axis, keeping its counts in registers while the group
+// stays the same.  group[t] is the same for every thread at a given t, so the flushes (RED.ADD) do not diverge and
+// happen once per run of equal groups.  Steps whose group is outside [0, ngroups) are neither loaded nor counted.  The
+// flags are read exactly once; the loads of FC_STEPS steps are issued before any of them is counted.
+#define FC_STEPS 4
+
+__device__ __forceinline__ int fc_group(const int* __restrict__ group, int t, int ntime, int ngroups) {
+  const int g = t < ntime ? group[t] : -1;
+  return (g >= 0 && g < ngroups) ? g : -1;
+}
+
+// 16 cells per thread, one 16-byte load per step (ncells % 16 == 0, flags 16-byte aligned).  The counts are kept as
+// 16-bit lanes, two per register (lo: bytes 0 and 2 of a word, hi: bytes 1 and 3), and flushed at least every 65535
+// counted steps so that no lane overflows.
+__device__ __forceinline__ void fc_flush16(u32* __restrict__ dst, const u32 (&lo)[4], const u32 (&hi)[4]) {
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    const u32 c[4] = {lo[q] & 0xffffu, hi[q] & 0xffffu, lo[q] >> 16, hi[q] >> 16};
+#pragma unroll
+    for (int b = 0; b < 4; ++b)
+      if (c[b]) atomicAdd(dst + 4 * q + b, c[b]);
+  }
+}
+
+__global__ void __launch_bounds__(256, 4) flag_counts16_kernel(const int8_t* __restrict__ flags, int nkinds, int ntime,
+                                                            long long ncells, const int* __restrict__ group, int ngroups,
+                                                            u32* __restrict__ counts) {
+  const long long nrun = ncells >> 4;
+  const long long items = (long long)nkinds * nrun;
+  for (long long it = (long long)blockIdx.x * blockDim.x + threadIdx.x; it < items;
+       it += (long long)gridDim.x * blockDim.x) {
+    const int k = (int)(it / nrun);
+    const long long c0 = (it - (long long)k * nrun) << 4;
+    const int8_t* base = flags + (size_t)k * (size_t)ntime * (size_t)ncells + (size_t)c0;
+    u32 lo[4] = {0u, 0u, 0u, 0u}, hi[4] = {0u, 0u, 0u, 0u};
+    int cur = -1, run = 0;
+    for (int t0 = 0; t0 < ntime; t0 += FC_STEPS) {
+      int g[FC_STEPS];
+      uint4 v[FC_STEPS];
+#pragma unroll
+      for (int u = 0; u < FC_STEPS; ++u) {
+        g[u] = fc_group(group, t0 + u, ntime, ngroups);
+        v[u] = g[u] >= 0 ? *reinterpret_cast<const uint4*>(base + (size_t)(t0 + u) * (size_t)ncells)
+                         : make_uint4(0u, 0u, 0u, 0u);
+      }
+#pragma unroll
+      for (int u = 0; u < FC_STEPS; ++u) {
+        if (g[u] != cur || run == 0xffff) {
+          if (cur >= 0) fc_flush16(counts + ((size_t)cur * (size_t)nkinds + (size_t)k) * (size_t)ncells + (size_t)c0, lo, hi);
+#pragma unroll
+          for (int q = 0; q < 4; ++q) lo[q] = hi[q] = 0u;
+          cur = g[u];
+          run = 0;
+        }
+        if (g[u] < 0) continue;
+        const u32 w[4] = {v[u].x, v[u].y, v[u].z, v[u].w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          // bit 7 of every byte := byte != 0 (no carry crosses a byte: 0x7f + 0x7f < 0x100)
+          const u32 nz = ((((w[q] & 0x7f7f7f7fu) + 0x7f7f7f7fu) | w[q]) >> 7) & 0x01010101u;
+          lo[q] += nz & 0x00ff00ffu;
+          hi[q] += (nz >> 8) & 0x00ff00ffu;
+        }
+        ++run;
+      }
+    }
+    if (cur >= 0) fc_flush16(counts + ((size_t)cur * (size_t)nkinds + (size_t)k) * (size_t)ncells + (size_t)c0, lo, hi);
+  }
+}
+
+// any ncells or alignment: one cell (one byte per lane and step) per thread
+__global__ void __launch_bounds__(256) flag_counts1_kernel(const int8_t* __restrict__ flags, int nkinds, int ntime,
+                                                           long long ncells, const int* __restrict__ group, int ngroups,
+                                                           u32* __restrict__ counts) {
+  const long long items = (long long)nkinds * ncells;
+  for (long long it = (long long)blockIdx.x * blockDim.x + threadIdx.x; it < items;
+       it += (long long)gridDim.x * blockDim.x) {
+    const int k = (int)(it / ncells);
+    const long long c = it - (long long)k * ncells;
+    const int8_t* base = flags + (size_t)k * (size_t)ntime * (size_t)ncells + (size_t)c;
+    u32 cnt = 0;
+    int cur = -1;
+    for (int t0 = 0; t0 < ntime; t0 += FC_STEPS) {
+      int g[FC_STEPS];
+      int8_t v[FC_STEPS];
+#pragma unroll
+      for (int u = 0; u < FC_STEPS; ++u) {
+        g[u] = fc_group(group, t0 + u, ntime, ngroups);
+        v[u] = g[u] >= 0 ? base[(size_t)(t0 + u) * (size_t)ncells] : (int8_t)0;
+      }
+#pragma unroll
+      for (int u = 0; u < FC_STEPS; ++u) {
+        if (g[u] != cur) {
+          if (cur >= 0 && cnt) atomicAdd(counts + ((size_t)cur * (size_t)nkinds + (size_t)k) * (size_t)ncells + (size_t)c, cnt);
+          cnt = 0;
+          cur = g[u];
+        }
+        cnt += v[u] != 0 ? 1u : 0u;
+      }
+    }
+    if (cur >= 0 && cnt) atomicAdd(counts + ((size_t)cur * (size_t)nkinds + (size_t)k) * (size_t)ncells + (size_t)c, cnt);
+  }
+}
+
+extern "C" int wbk_flag_counts(const int8_t* d_flags, int nkinds, int ntime, long long ncells, const int* d_group,
+                               int ngroups, uint32_t* d_counts, void* stream) {
+  if (nkinds < 1 || ntime < 0 || ncells < 0 || ngroups < 1) {
+    wbk_set_error("wbk_flag_counts: invalid argument (nkinds %d, ntime %d, ncells %lld, ngroups %d)", nkinds, ntime,
+                  ncells, ngroups);
+    return WBK_ERR_INVALID;
+  }
+  if (ntime == 0 || ncells == 0) return WBK_OK;
+  if (!d_flags || !d_group || !d_counts) {
+    wbk_set_error("wbk_flag_counts: invalid argument (null pointer)");
+    return WBK_ERR_INVALID;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const bool vec = ncells % 16 == 0 && ((uintptr_t)d_flags & 15) == 0;
+  const long long items = (long long)nkinds * (vec ? ncells / 16 : ncells);
+  const long long blocks = (items + 255) / 256;
+  const int grid = (int)(blocks < 148 * 64 ? blocks : 148 * 64);
+  if (vec) {
+    WBK_LAUNCH(KID_FLAG_COUNTS, flag_counts16_kernel, dim3(grid), dim3(256), 0, st, d_flags, nkinds, ntime, ncells,
+               d_group, ngroups, (u32*)d_counts);
+  } else {
+    WBK_LAUNCH(KID_FLAG_COUNTS, flag_counts1_kernel, dim3(grid), dim3(256), 0, st, d_flags, nkinds, ntime, ncells,
+               d_group, ngroups, (u32*)d_counts);
+  }
+  WBK_LAUNCH_CHECK();
+  return WBK_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // Pieces of the events that straddle the last meridian (utils/index_utils.py:148-173), as the device clipper of
 // wbk_events_raster left them: compacted into ring r = vertices [ring_off[r], ring_off[r+1]) of d_xy (folded index
 // coordinates of the real grid), ring_ev[r] = the event (row of the wbk_batch_fetch tables) the piece belongs to.

@@ -133,6 +133,7 @@ class _Slot:
         self.pending = None   # (raw, ntime, flags_dev, flags_host, gmax)
         self.grow_seen = 0
         self.packed = None    # bit-packed flag grids (device), allocated on first use
+        self.clim_group = None  # int32 [T] (device): groups of the batch's steps for FlagClimatology, on first use
         self.graphs = {}      # buffers key -> (torch.cuda.CUDAGraph, pending record)
         self.graph_seen = set()
 
@@ -356,7 +357,7 @@ class Detector:
         use_stream = stream if stream is not None else slot.stream
         args = (slot, raw, flags_out, flags_host, gmax_nx, smoothed, intensity, packed_host)
         if use_stream is None:  # emulator
-            slot.pending = self._enqueue(*args)
+            slot.pending = dict(self._enqueue(*args), stream=None)
             return slot
         graphable = self.graphs and smoothed is None and intensity is None
         key = None
@@ -389,11 +390,15 @@ class Detector:
                 slot.pending = self._enqueue(*args)
                 if key is not None:
                     slot.graph_seen.add(key)
+            slot.pending = dict(slot.pending, stream=use_stream)  # (a replayed graph's record is shared: copy it)
             slot.done.record()
         return slot
 
-    def collect(self, slot):
-        """Wait for the slot's batch and return its BatchResult (re-runs it with larger arenas on overflow)."""
+    def collect(self, slot, climatology=None):
+        """Wait for the slot's batch and return its BatchResult (re-runs it with larger arenas on overflow).
+
+        ``climatology``: a :class:`FlagClimatology` that the batch's flag grids are added to.  That happens here, after
+        every check that can make the batch run again has passed, so each batch is counted exactly once."""
         pend = slot.pending
         if pend is None:
             raise RuntimeError("nothing was submitted on this slot")
@@ -408,7 +413,7 @@ class Detector:
             raise _lib.WbkError(_lib.ERR_INVALID, "an event crosses the last meridian too often for the device clipper; "
                                                   "its cells would be missing from the flag grids")
         if bad:
-            return self._regrow_and_rerun(slot, status)
+            return self._regrow_and_rerun(slot, status, climatology)
         slot.pending = None
         nt = pend["nt"]
         L = len(self.levels)
@@ -444,19 +449,22 @@ class Detector:
                 grow = dict(self._grow)
                 grow["cap_sr"], grow["cap_sv"] = max(2 * slot.cap_sr, 2 * npc), max(2 * slot.cap_sv, 2 * nvx)
                 self._grow = grow
-                return self._regrow_and_rerun(slot, 0)
+                slot.pending = pend  # the re-run submits the batch again from its pending record
+                return self._regrow_and_rerun(slot, 0, climatology)
             off = slot.h_sp_off.numpy()[:npc + 1].astype(np.int64)
             pieces = dict(ev=slot.h_sp_ev.numpy()[:npc].copy(), off=off, xy=slot.h_sp_xy.numpy()[:nvx].copy(),
                           overflow=bool(clip_over))
         n_near = int(slot.h_near_cnt[0]) if "streamers" in self.which else 0
         rec = slot.h_near.numpy()[:min(n_near, _lib.NEAR_CAP)]
         near = np.c_[rec[:, 0] // L, rec[:, 0] % L, rec[:, 1], rec[:, 2], rec[:, 3] & 0x0FFFFFFF, (rec[:, 3] >> 28) & 7]
+        if climatology is not None:
+            climatology._add(slot, pend)
         return BatchResult(ntime=nt, contours=cs, tables=tables, flags=flags,
                            gmax_nx=max_nx if pend["gmax"] is None else int(pend["gmax"]), n_split=n_sp,
                            near=near.astype(np.int32), near_total=n_near, flags_packed=packed, work=work, pieces=pieces,
                            counts=(ns, no, nc))
 
-    def _regrow_and_rerun(self, slot, status):
+    def _regrow_and_rerun(self, slot, status, climatology=None):
         pend = slot.pending
         caps = dict(slot.ctx.caps)
         grow = dict(self._grow)
@@ -491,7 +499,7 @@ class Detector:
         self._slots[key] = new
         self.submit(new, pend["raw"], flags_out=pend["flags"], flags_host=pend["flags_host"], gmax_nx=pend["gmax"],
                     smoothed=pend["smoothed"], intensity=pend["intensity"], packed_host=pend.get("packed_host"))
-        return self.collect(new)
+        return self.collect(new, climatology)
 
     # ------------------------------------------------------------------ convenience
     def run_batch(self, raw, gmax_nx=None, smoothed=None, intensity=None):
@@ -517,7 +525,8 @@ class Detector:
         self.submit(slot, raw_host, flags_host=flags_host)
         return self.collect(slot)
 
-    def stream(self, batches, depth=3, flags_host=None, shared_stream=False, gmax_nx="full", packed_host=None):
+    def stream(self, batches, depth=3, flags_host=None, shared_stream=False, gmax_nx="full", packed_host=None,
+               climatology=None):
         """Pipelined execution: yields one BatchResult per input batch, in order.
 
         ``batches``: iterable of device or pinned-host tensors of (at most) equal length.  ``depth`` batches are
@@ -535,7 +544,11 @@ class Detector:
         width a warning is logged with the maximum that was seen -- re-run with ``gmax_nx=<that value>`` to get the
         reference's result for such a record.  ``None`` = every batch uses its own maximum; an int = that value.
         The flag grids / contour set of a result are only valid until its slot is reused (``depth`` batches later).
+        ``climatology``: a :class:`FlagClimatology`; the flag grids of every batch are added to its counters on the
+        device (the batches take consecutive time steps of its group array, from its cursor on).
         """
+        if climatology is not None:
+            climatology._check_detector(self)
         common = None
         if shared_stream and self.lib.is_cuda:
             if getattr(self, "_shared", None) is None:
@@ -551,7 +564,7 @@ class Detector:
         for raw in batches:
             idx = i % depth
             if len(inflight) == depth:
-                res = self.collect(inflight.pop(0))
+                res = self.collect(inflight.pop(0), climatology)
                 seen_max = max(seen_max, res.contours.max_nx)
                 yield res
             slot = self._slot(int(raw.shape[0]), idx)
@@ -560,13 +573,128 @@ class Detector:
             inflight.append(self.submit(slot, raw, flags_host=fh, stream=common, gmax_nx=gmax_nx, packed_host=ph))
             i += 1
         while inflight:
-            res = self.collect(inflight.pop(0))
+            res = self.collect(inflight.pop(0), climatology)
             seen_max = max(seen_max, res.contours.max_nx)
             yield res
         if assumed and i > 0 and seen_max < full:
             logger.warning("no contour of the %d batches spans the extended grid (%d columns; widest: %d): the "
                            "reference's exp_lon.max() would be %d columns, re-run with gmax_nx=%d", i, full, seen_max,
                            seen_max, seen_max)
+
+
+GROUPINGS = ("all", "month", "season")
+
+
+def groups_from_dates(dates, by):
+    """int32 group of every date for :class:`FlagClimatology`: ``by="all"`` puts every step in group 0, ``"month"``
+    gives January = 0 .. December = 11, ``"season"`` gives DJF = 0, MAM = 1, JJA = 2, SON = 3 (December counts with
+    the following January and February).  Missing dates (NaT) get -1, i.e. are not counted."""
+    if by not in GROUPINGS:
+        raise ValueError("by has to be one of {}, got {!r}".format(GROUPINGS, by))
+    d = np.asarray(dates)
+    if not np.issubdtype(d.dtype, np.datetime64):
+        raise ValueError("dates have to be datetime64 values, got dtype {}".format(d.dtype))
+    month = d.astype("datetime64[M]").astype(np.int64) % 12
+    if by == "all":
+        g = np.zeros(d.shape, dtype=np.int32)
+    elif by == "month":
+        g = month.astype(np.int32)
+    else:
+        g = ((month + 1) // 3 % 4).astype(np.int32)
+    g[np.isnat(d)] = -1
+    return g
+
+
+def _percent(counts, steps):
+    """100 * counts / steps (float64) over the leading group axis; NaN for groups without steps."""
+    c = np.asarray(counts, dtype=np.float64)
+    s = np.asarray(steps, dtype=np.float64).reshape((-1,) + (1,) * (c.ndim - 1))
+    with np.errstate(invalid="ignore", divide="ignore"):
+        out = 100.0 * c / s
+    out[np.broadcast_to(s == 0, out.shape)] = np.nan
+    return out
+
+
+class FlagClimatology:
+    """Flag-frequency climatology accumulated on the device while ``Detector.stream`` runs.
+
+    ``groups``: int array over the global time axis of the record: the group of every time step in [0, ngroups), or
+    -1 for a step that is not counted (``groups_from_dates`` makes monthly / seasonal ones).  ``ngroups`` defaults to
+    ``max(groups) + 1``.  ``t0``: the time step of the record the first batch starts at (the start of a rank's shard
+    in a sharded run, ``sharding.shard_range``).  The counters, uint32 ``[ngroups, 3, nlat, nlon]`` (streamers,
+    overturnings, cutoffs), live on the device and are zeroed once; every batch adds the number of its steps in which a
+    cell is flagged, in the group of that step, without any flag grid leaving the device.
+    """
+
+    def __init__(self, det, groups, ngroups=None, t0=0):
+        if not det.want_flags:
+            raise ValueError("a flag climatology needs the flag grids: the Detector has want_flags=False")
+        g = np.asarray(groups)
+        if g.ndim != 1 or not (np.issubdtype(g.dtype, np.integer) or g.size == 0):
+            raise ValueError("groups has to be a 1-D integer array over the time axis")
+        g = np.ascontiguousarray(g, dtype=np.int64)
+        if ngroups is None:
+            ngroups = int(g.max()) + 1 if g.size and g.max() >= 0 else 1
+        ngroups = int(ngroups)
+        if ngroups < 1:
+            raise ValueError("ngroups has to be positive, got {}".format(ngroups))
+        if g.size and (g.min() < -1 or g.max() >= ngroups):
+            raise ValueError("groups has values outside [-1, {}): {}..{}".format(ngroups, int(g.min()), int(g.max())))
+        if not 0 <= int(t0) <= len(g):
+            raise ValueError("t0 = {} is outside the group array (length {})".format(t0, len(g)))
+        self.lib = det.lib
+        self.nlat, self.nlon = det.nlat, det.nlon
+        self.groups = g.astype(np.int32)
+        self.ngroups = ngroups
+        self.cursor = int(t0)
+        self._steps = np.zeros(ngroups, dtype=np.int64)
+        # uint32 counters, held in an int32 tensor (the bits are read back as uint32)
+        self._counts = torch.zeros((ngroups, 3, self.nlat, self.nlon), dtype=torch.int32, device=self.lib.device)
+
+    def _check_detector(self, det):
+        if not det.want_flags:
+            raise ValueError("a flag climatology needs the flag grids: the Detector has want_flags=False")
+        if (det.nlat, det.nlon) != (self.nlat, self.nlon):
+            raise ValueError("the climatology is for a {} x {} grid, the Detector's is {} x {}".format(
+                self.nlat, self.nlon, det.nlat, det.nlon))
+
+    def _add(self, slot, pend):
+        """Add the flag grids of one collected batch, on the stream the batch ran on."""
+        nt, flags = int(pend["nt"]), pend["flags"]
+        if self.cursor + nt > len(self.groups):
+            raise ValueError("the batch covers time steps {}..{} of the record, the group array has {}".format(
+                self.cursor, self.cursor + nt - 1, len(self.groups)))
+        g = self.groups[self.cursor:self.cursor + nt]
+        add = np.bincount(g[g >= 0], minlength=self.ngroups)
+        if (self._steps + add > 0xFFFFFFFF).any():
+            raise ValueError("a group would count more than 2**32 - 1 time steps")
+        lib = self.lib
+        st = pend.get("stream")
+        with torch.cuda.stream(st) if st is not None else _null():
+            if slot.clim_group is None:
+                slot.clim_group = torch.empty(slot.T, dtype=torch.int32, device=lib.device)
+            slot.clim_group[:nt].copy_(torch.from_numpy(g), non_blocking=True)
+            # the grids as the rasteriser wrote them: kind stride nt * nlat * nlon (also for a partial last batch)
+            lib.call("wbk_flag_counts", _lib.ptr(flags), 3, nt, self.nlat * self.nlon, _lib.ptr(slot.clim_group),
+                     self.ngroups, _lib.ptr(self._counts), lib.stream())
+        self._steps += add
+        self.cursor += nt
+
+    def counts(self):
+        """uint32 ``[ngroups, 3, nlat, nlon]`` on the host (ascending coordinates, like the Detector's flag grids)."""
+        if self.lib.is_cuda:
+            torch.cuda.synchronize(self.lib.device)
+        return self._counts.cpu().numpy().view(np.uint32)
+
+    @property
+    def steps(self):
+        """int64 ``[ngroups]``: time steps counted in every group."""
+        return self._steps.copy()
+
+    def frequency(self):
+        """float64 ``[ngroups, 3, nlat, nlon]``: percent of the group's time steps in which a cell is flagged (NaN for
+        groups without steps)."""
+        return _percent(self.counts(), self._steps)
 
 
 class _null:

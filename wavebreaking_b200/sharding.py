@@ -7,7 +7,8 @@ collective is needed.  Three small host-side merges remain (SURVEY.md 8e):
 1. ``exp_lon.max()`` is global over all dates (streamer_index.py:106) -> scalar MAX all-reduce;
 2. event ids / row indices are global (streamer_index.py:281-283) -> exclusive prefix sum of the per-rank counts;
 3. the event tables are gathered to rank 0 in rank (= time) order;
-4. ``track_events`` across shard boundaries: a halo of the event table (:func:`track_sharded`).
+4. ``track_events`` across shard boundaries: a halo of the event table (:func:`track_sharded`);
+5. flag-frequency climatologies: a SUM all-reduce of the per-rank counters (:func:`reduce_climatology`).
 """
 
 import numpy as np
@@ -54,6 +55,25 @@ def exclusive_offset(count):
     dist.all_reduce(t, op=dist.ReduceOp.SUM)
     counts = t.cpu().numpy()
     return int(counts[:rank].sum()), int(counts.sum())
+
+
+def reduce_climatology(clim):
+    """Totals of a ``pipeline.FlagClimatology`` over all ranks, on every rank: ``(counts, steps)``, int64
+    ``[ngroups, 3, nlat, nlon]`` and int64 ``[ngroups]``.  Every rank builds its climatology from the same group array
+    with ``t0`` = the start of its shard (``shard_range``), so each time step is counted on exactly one rank."""
+    rank, ws = world()
+    if ws == 1:
+        return clim.counts().astype(np.int64), clim.steps
+    dev = _device_for_collectives()
+    if dev.type == "cuda":
+        torch.cuda.synchronize(dev)
+        counts = clim._counts.to(device=dev, dtype=torch.int64) & 0xFFFFFFFF  # the int32 storage holds uint32 bits
+    else:
+        counts = torch.from_numpy(clim.counts().astype(np.int64))
+    steps = torch.from_numpy(clim.steps).to(dev)
+    dist.all_reduce(counts, op=dist.ReduceOp.SUM)
+    dist.all_reduce(steps, op=dist.ReduceOp.SUM)
+    return counts.cpu().numpy(), steps.cpu().numpy()
 
 
 def gather_frames(frame, dst=0):
