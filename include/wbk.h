@@ -364,6 +364,26 @@ int wbk_track_overlap(const double* d_xy, const int* d_ring_off, const int* d_po
  * re-decides pairs within 1e-9 of its threshold on the host. */
 int wbk_track_distance(const double* d_rad, const int* d_pairs, int npairs, double* d_out, void* stream);
 
+/* Tracking polygons of one kind of a batch, read from the device buffers of wbk_batch_fetch / wbk_split_fetch and
+ * appended to a caller-owned window in the layout wbk_track_candidates and wbk_track_overlap_exact read
+ * (utils/index_utils.py:129-184 transform_polygons, vertex for vertex as pipeline.events_soup builds them).
+ * Input: the rows [first, first + n) of d_ev_int [rows][WBK_EV_INTS] (the kind-major gather), their rings
+ * d_ring_off [rows + 1] / d_ring_pts (packed x | y << 16), and the npieces device-clipper pieces d_sp_ev / d_sp_off /
+ * d_sp_xy.  A row with split == 1 becomes its pieces (in piece order), an overturning (is_box) the box
+ * (x1, y0), (x1, y1), (x0, y1), (x0, y0), any other row its ring; x is folded with x % nlon.
+ * Output, starting at vertex v0, ring r0 and polygon p0 of the window: d_edges [V][4] (x0, y0, x1, y1 of the edge
+ * to the next vertex of the ring), d_vsign [V] (sign of the ring's doubled area), d_win_ring_off (ring r0 + k =
+ * vertices [ring_off[r0 + k], ring_off[r0 + k + 1]), absolute), d_win_poly_off (absolute, like the ring offsets) and
+ * d_bbox [P][4] (x0, y0, x1, y1; (1, 1, 0, 0) for a polygon without vertices).  nrings / nverts: what this batch adds
+ * (the caller knows them from the host copies of the ring and piece offsets).  cap_v / cap_r / cap_p: the sizes of
+ * d_edges (and d_vsign), d_win_ring_off and d_win_poly_off in elements; WBK_ERR_INVALID when the batch does not fit
+ * or the window would pass 2^31 - 1 vertices, rings or polygons (the offsets are int32).  Asynchronous. */
+int wbk_track_append(const int* d_ev_int, const int* d_ring_off, const uint32_t* d_ring_pts, const int* d_sp_ev,
+                     const int* d_sp_off, const int* d_sp_xy, int npieces, int first, int n, int is_box, int nlon,
+                     long long nrings, long long nverts, int* d_edges, int* d_vsign, int* d_win_ring_off,
+                     int* d_win_poly_off, int* d_bbox, long long v0, long long r0, long long p0, long long cap_v,
+                     long long cap_r, long long cap_p, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -105,6 +105,9 @@ _SIGNATURES = {
     "wbk_track_candidates": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "wbk_track_overlap_exact": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
     "wbk_track_distance": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p]),
+    "wbk_track_append": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
+                                 c_int, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64,
+                                 c_int64, c_int64, c_int64, c_int64, c_int64, c_void_p]),
     "wbk_prof_enable": (c_int, [c_int]),
     "wbk_prof_reset": (c_int, []),
     "wbk_prof_read": (c_int, [POINTER(c_int), POINTER(c_double)]),

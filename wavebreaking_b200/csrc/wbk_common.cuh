@@ -20,7 +20,7 @@ enum WbkKernelId {
   KID_SMOOTH = 0, KID_CONVOLVE, KID_NAN_BORDER, KID_MFLUX, KID_FLIP, KID_SYNTH, KID_MS_SEGMENTS, KID_CONTOUR_LINK,
   KID_CONTOUR_PACK, KID_SELECT, KID_OVERTURNING, KID_STREAMER_PREP, KID_TILE_SCAN, KID_PAIR_SCAN, KID_CASCADE,
   KID_EVENT_LIST, KID_EVENTS_RASTER, KID_RINGS_RASTER, KID_OWNER, KID_EVENTS_GATHER, KID_TRACK_OVERLAP, KID_MISC, KID_SPLIT, KID_SPLIT_RASTER, KID_TOUCH, KID_FINISH, KID_SMOOTH_MS, KID_TRACK_PAIRS, KID_TRACK_EXACT, KID_TRACK_DIST,
-  KID_FLAG_COUNTS
+  KID_FLAG_COUNTS, KID_TRACK_APPEND
 };
 void wbk_prof_begin(int kid, void* stream);
 void wbk_prof_end(int kid, void* stream);

@@ -39,7 +39,7 @@ static const char* kKernelNames[WBK_PROF_NKERNELS] = {
     "contours_pack", "select", "overturning", "streamer_prep", "tile_scan", "pair_scan", "streamer_dedupe",
     "event_list", "events_raster", "rings_raster", "owner", "events_gather", "track_overlap", "misc", "split_events",
     "split_raster", "streamer_touch", "streamer_finish", "smooth_ms_fused", "track_pairs", "track_exact", "track_distance",
-    "flag_counts", ""};
+    "flag_counts", "track_append"};
 
 static std::atomic<long long> g_launches{0};
 static std::atomic<int> g_prof_on{0};

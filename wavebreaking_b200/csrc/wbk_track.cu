@@ -417,3 +417,186 @@ extern "C" int wbk_track_distance(const double* d_rad, const int* d_pairs, int n
   WBK_LAUNCH_CHECK();
   return WBK_OK;
 }
+
+// ------------------------------------------------------------------------------------------------------------
+// Tracking polygons of one kind of one collected batch, appended to a device window in the layout that
+// wbk_track_candidates / wbk_track_overlap_exact read (utils/index_utils.py:129-184 transform_polygons, as
+// pipeline.events_soup builds it on the host): x folded with x % nlon, an event with split == 1 replaced by its
+// device-clipper pieces (in piece order), an overturning = its box (x1, y0), (x1, y1), (x0, y1), (x0, y0).
+// count -> exclusive scan (one CTA) -> fill (one warp per event).
+#define TAP_THREADS 1024
+#define TAP_SPLIT_COL 8
+#define TAP_BOX_COL 3
+
+struct TapIn {
+  const int* ev_int;       // [rows][WBK_EV_INTS] of the batch (kind-major gather)
+  const int* ring_off;     // [rows + 1] ring vertices of every row in ring_pts
+  const u32* ring_pts;     // packed lattice points (x low 16 bits, y high 16 bits)
+  const int* sp_ev;        // [npieces] row of every piece
+  const int* sp_off;       // [npieces + 1]
+  const int* sp_xy;        // [..][2] folded piece vertices
+  int npieces, first, n, is_box, nlon;
+};
+
+struct TapOut {
+  int4* edges;
+  int* vsign;
+  int* ring_off;
+  int* poly_off;
+  int4* bbox;
+  int v0, r0, p0;          // where this batch starts in the window
+  int cap_v, cap_r, cap_p;  // window capacities (writes beyond them are dropped)
+};
+
+__device__ __forceinline__ int2 tap_i2(int x, int y) {
+  int2 r;
+  r.x = x; r.y = y;
+  return r;
+}
+__device__ __forceinline__ int4 tap_i4(int x, int y, int z, int w) {
+  int4 r;
+  r.x = x; r.y = y; r.z = z; r.w = w;
+  return r;
+}
+
+__device__ __forceinline__ bool tap_split(const TapIn& in, int e) {
+  return in.ev_int[(size_t)(in.first + e) * WBK_EV_INTS + TAP_SPLIT_COL] == 1;
+}
+
+// one warp: the k-th piece (in piece order) of row `row`, for k = 0, 1, ...: f(k, piece)
+template <typename F>
+__device__ __forceinline__ void tap_pieces(const TapIn& in, int row, F f) {
+  const int lane = wbk_lane();
+  int k = 0;
+  for (int b = 0; b < in.npieces; b += 32) {
+    const int r = b + lane;
+    u32 m = __ballot_sync(WBK_FULL, r < in.npieces && in.sp_ev[r] == row);
+    while (m) {
+      const int bit = __ffs(m) - 1;
+      m &= m - 1;
+      f(k++, b + bit);
+    }
+  }
+}
+
+__global__ void __launch_bounds__(TAP_THREADS) track_append_scan_kernel(TapIn in, TapOut out) {
+  __shared__ int sscan[40];
+  const int lane = wbk_lane(), nw = blockDim.x >> 5;
+  int* nr = out.poly_off + out.p0;  // rings per event, scanned in place into the polygon offsets
+  for (int e = wbk_warp(); e < in.n; e += nw) {
+    int cnt = 1;
+    if (tap_split(in, e)) {
+      cnt = 0;
+      tap_pieces(in, in.first + e, [&](int, int) { ++cnt; });
+    }
+    if (lane == 0) nr[e] = cnt;
+  }
+  __syncthreads();
+  const int nrings = wbk_block_excl_scan(nr, in.n, sscan);
+  if ((long long)out.r0 + nrings + 1 > out.cap_r) return;  // (the caller sized the window from the same tables)
+  for (int e = threadIdx.x; e < in.n; e += blockDim.x) nr[e] += out.r0;
+  if (threadIdx.x == 0) nr[in.n] = out.r0 + nrings;
+  __syncthreads();
+  int* nv = out.ring_off + out.r0;  // vertices per ring, scanned in place into the ring offsets
+  for (int e = wbk_warp(); e < in.n; e += nw) {
+    const int R = nr[e] - out.r0;
+    if (tap_split(in, e)) {
+      tap_pieces(in, in.first + e, [&](int k, int r) {
+        if (lane == 0) nv[R + k] = in.sp_off[r + 1] - in.sp_off[r];
+      });
+    } else if (lane == 0) {
+      nv[R] = in.is_box ? 4 : in.ring_off[in.first + e + 1] - in.ring_off[in.first + e];
+    }
+  }
+  __syncthreads();
+  const int nverts = wbk_block_excl_scan(nv, nrings, sscan);
+  for (int r = threadIdx.x; r < nrings; r += blockDim.x) nv[r] += out.v0;
+  if (threadIdx.x == 0) nv[nrings] = out.v0 + nverts;
+}
+
+// one warp writes the edges of ring [s, s + len) of the window and its orientation sign; vertex k = xy(k)
+template <typename XY>
+__device__ __forceinline__ void tap_ring(const TapOut& out, int s, int len, XY xy, int4& box) {
+  const int lane = wbk_lane();
+  long long a2 = 0;
+  for (int k = lane; k < len; k += 32) {
+    const int2 p = xy(k), q = xy(k + 1 == len ? 0 : k + 1);
+    if (s + k < out.cap_v) out.edges[s + k] = tap_i4(p.x, p.y, q.x, q.y);
+    a2 += (long long)p.x * q.y - (long long)q.x * p.y;
+    box.x = min(box.x, p.x); box.y = min(box.y, p.y); box.z = max(box.z, p.x); box.w = max(box.w, p.y);
+  }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) a2 += __shfl_xor_sync(WBK_FULL, a2, d);
+  const int sg = a2 > 0 ? 1 : (a2 < 0 ? -1 : 0);
+  for (int k = lane; k < len && s + k < out.cap_v; k += 32) out.vsign[s + k] = sg;
+}
+
+__global__ void __launch_bounds__(256) track_append_fill_kernel(TapIn in, TapOut out) {
+  const int lane = wbk_lane(), wpb = blockDim.x >> 5;
+  for (int e = blockIdx.x * wpb + wbk_warp(); e < in.n; e += gridDim.x * wpb) {
+    const int row = in.first + e, nlon = in.nlon;
+    int4 box = tap_i4(0x7fffffff, 0x7fffffff, -0x7fffffff - 1, -0x7fffffff - 1);
+    const int R = out.poly_off[out.p0 + e];
+    if (tap_split(in, e)) {
+      tap_pieces(in, row, [&](int k, int r) {
+        const int a = in.sp_off[r];
+        const int2* pxy = reinterpret_cast<const int2*>(in.sp_xy);
+        tap_ring(out, out.ring_off[R + k], in.sp_off[r + 1] - a, [&](int i) { return pxy[a + i]; }, box);
+      });
+    } else if (in.is_box) {
+      const int* b = in.ev_int + (size_t)row * WBK_EV_INTS + TAP_BOX_COL;
+      const int x0 = ((b[0] % nlon) + nlon) % nlon, y0 = b[1], x1 = ((b[2] % nlon) + nlon) % nlon, y1 = b[3];
+      tap_ring(out, out.ring_off[R], 4, [&](int i) {
+        return i == 0 ? tap_i2(x1, y0) : i == 1 ? tap_i2(x1, y1) : i == 2 ? tap_i2(x0, y1) : tap_i2(x0, y0);
+      }, box);
+    } else {
+      const int a = in.ring_off[row];
+      tap_ring(out, out.ring_off[R], in.ring_off[row + 1] - a, [&](int i) {
+        const u32 p = in.ring_pts[a + i];
+        return tap_i2((int)(p & 0xffffu) % nlon, (int)(p >> 16));
+      }, box);
+    }
+    box.x = wbk_warp_min(box.x); box.y = wbk_warp_min(box.y);
+    box.z = wbk_warp_max(box.z); box.w = wbk_warp_max(box.w);
+    if (box.x > box.z) box = tap_i4(1, 1, 0, 0);  // no vertex: an empty box (PolygonSoup.bounds)
+    if (lane == 0 && out.p0 + e < out.cap_p) out.bbox[out.p0 + e] = box;
+  }
+}
+
+extern "C" int wbk_track_append(const int* d_ev_int, const int* d_ring_off, const uint32_t* d_ring_pts, const int* d_sp_ev,
+                                const int* d_sp_off, const int* d_sp_xy, int npieces, int first, int n, int is_box,
+                                int nlon, long long nrings, long long nverts, int* d_edges, int* d_vsign,
+                                int* d_win_ring_off, int* d_win_poly_off, int* d_bbox, long long v0, long long r0,
+                                long long p0, long long cap_v, long long cap_r, long long cap_p, void* stream) {
+  const long long lim = 2147483647LL;
+  if (n < 0 || first < 0 || npieces < 0 || nlon < 1 || nrings < 0 || nverts < 0 || v0 < 0 || r0 < 0 || p0 < 0) {
+    wbk_set_error("wbk_track_append: invalid argument (n %d, first %d, npieces %d, nlon %d)", n, first, npieces, nlon);
+    return WBK_ERR_INVALID;
+  }
+  if (v0 + nverts > lim || r0 + nrings + 1 > lim || p0 + n + 1 > lim) {
+    wbk_set_error("wbk_track_append: the window would hold %lld vertices, %lld rings and %lld polygons; its 32-bit "
+                  "offsets allow at most 2^31 - 1", v0 + nverts, r0 + nrings, p0 + n);
+    return WBK_ERR_INVALID;
+  }
+  if (v0 + nverts > cap_v || r0 + nrings + 1 > cap_r || p0 + n + 1 > cap_p) {
+    wbk_set_error("wbk_track_append: the window is too small (%lld / %lld vertices, %lld / %lld ring offsets, "
+                  "%lld / %lld polygon offsets)", v0 + nverts, cap_v, r0 + nrings + 1, cap_r, p0 + n + 1, cap_p);
+    return WBK_ERR_INVALID;
+  }
+  if (n == 0) return WBK_OK;
+  if (!d_ev_int || (!is_box && (!d_ring_off || !d_ring_pts)) || (npieces > 0 && (!d_sp_ev || !d_sp_off || !d_sp_xy)) ||
+      !d_edges || !d_vsign || !d_win_ring_off || !d_win_poly_off || !d_bbox) {
+    wbk_set_error("wbk_track_append: invalid argument (null pointer)");
+    return WBK_ERR_INVALID;
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const TapIn in{d_ev_int, d_ring_off, d_ring_pts, d_sp_ev, d_sp_off, d_sp_xy, npieces, first, n, is_box, nlon};
+  const TapOut out{(int4*)d_edges, d_vsign, d_win_ring_off, d_win_poly_off, (int4*)d_bbox, (int)v0, (int)r0, (int)p0,
+                   (int)(cap_v < lim ? cap_v : lim), (int)(cap_r < lim ? cap_r : lim), (int)(cap_p < lim ? cap_p : lim)};
+  WBK_LAUNCH(KID_TRACK_APPEND, track_append_scan_kernel, dim3(1), dim3(TAP_THREADS), 0, st, in, out);
+  WBK_LAUNCH_CHECK();
+  const int blocks = (n + 7) / 8 < 148 * 8 ? (n + 7) / 8 : 148 * 8;
+  WBK_LAUNCH(KID_TRACK_APPEND, track_append_fill_kernel, dim3(blocks), dim3(256), 0, st, in, out);
+  WBK_LAUNCH_CHECK();
+  return WBK_OK;
+}

@@ -79,17 +79,18 @@ def iter_batches(field, batch, depth=3, start=0, stop=None):
 
 
 def detect_file(path, lat, lon, batch=296, depth=3, shape=None, dtype=np.float32, gmax_nx="full", climatology=None,
-                **detector_kwargs):
+                trackers=None, **detector_kwargs):
     """Run the whole detection path over a field file; yields ``(t0, BatchResult)`` per batch in time order.
 
     ``gmax_nx``: see ``Detector.stream`` (the reference's global ``exp_lon.max()``).  ``climatology``: a
-    ``pipeline.FlagClimatology`` for the same grid; the flag grids of every batch are added to it on the device."""
+    ``pipeline.FlagClimatology`` for the same grid; the flag grids of every batch are added to it on the device.
+    ``trackers``: a list of ``pipeline.EventTracker`` for the same grid, which track the events of every batch."""
     from . import pipeline
 
     field = open_field(path, shape=shape, dtype=dtype)
     det = pipeline.Detector(lat, lon, **detector_kwargs)
     t0 = 0
     for res in det.stream(iter_batches(field, batch, depth=depth), depth=depth, gmax_nx=gmax_nx,
-                          climatology=climatology):
+                          climatology=climatology, trackers=trackers):
         yield t0, res
         t0 += res.ntime

@@ -394,11 +394,12 @@ class Detector:
             slot.done.record()
         return slot
 
-    def collect(self, slot, climatology=None):
+    def collect(self, slot, climatology=None, trackers=()):
         """Wait for the slot's batch and return its BatchResult (re-runs it with larger arenas on overflow).
 
-        ``climatology``: a :class:`FlagClimatology` that the batch's flag grids are added to.  That happens here, after
-        every check that can make the batch run again has passed, so each batch is counted exactly once."""
+        ``climatology``: a :class:`FlagClimatology` that the batch's flag grids are added to; ``trackers``: a list of
+        :class:`EventTracker` that link the batch's events.  Both happen here, after every check that can make the batch
+        run again has passed, so each batch is counted exactly once."""
         pend = slot.pending
         if pend is None:
             raise RuntimeError("nothing was submitted on this slot")
@@ -413,7 +414,7 @@ class Detector:
             raise _lib.WbkError(_lib.ERR_INVALID, "an event crosses the last meridian too often for the device clipper; "
                                                   "its cells would be missing from the flag grids")
         if bad:
-            return self._regrow_and_rerun(slot, status, climatology)
+            return self._regrow_and_rerun(slot, status, climatology, trackers)
         slot.pending = None
         nt = pend["nt"]
         L = len(self.levels)
@@ -450,7 +451,7 @@ class Detector:
                 grow["cap_sr"], grow["cap_sv"] = max(2 * slot.cap_sr, 2 * npc), max(2 * slot.cap_sv, 2 * nvx)
                 self._grow = grow
                 slot.pending = pend  # the re-run submits the batch again from its pending record
-                return self._regrow_and_rerun(slot, 0, climatology)
+                return self._regrow_and_rerun(slot, 0, climatology, trackers)
             off = slot.h_sp_off.numpy()[:npc + 1].astype(np.int64)
             pieces = dict(ev=slot.h_sp_ev.numpy()[:npc].copy(), off=off, xy=slot.h_sp_xy.numpy()[:nvx].copy(),
                           overflow=bool(clip_over))
@@ -459,12 +460,14 @@ class Detector:
         near = np.c_[rec[:, 0] // L, rec[:, 0] % L, rec[:, 1], rec[:, 2], rec[:, 3] & 0x0FFFFFFF, (rec[:, 3] >> 28) & 7]
         if climatology is not None:
             climatology._add(slot, pend)
+        for tr in trackers or ():
+            tr._add(slot, pend, tables, counts)
         return BatchResult(ntime=nt, contours=cs, tables=tables, flags=flags,
                            gmax_nx=max_nx if pend["gmax"] is None else int(pend["gmax"]), n_split=n_sp,
                            near=near.astype(np.int32), near_total=n_near, flags_packed=packed, work=work, pieces=pieces,
                            counts=(ns, no, nc))
 
-    def _regrow_and_rerun(self, slot, status, climatology=None):
+    def _regrow_and_rerun(self, slot, status, climatology=None, trackers=()):
         pend = slot.pending
         caps = dict(slot.ctx.caps)
         grow = dict(self._grow)
@@ -499,7 +502,7 @@ class Detector:
         self._slots[key] = new
         self.submit(new, pend["raw"], flags_out=pend["flags"], flags_host=pend["flags_host"], gmax_nx=pend["gmax"],
                     smoothed=pend["smoothed"], intensity=pend["intensity"], packed_host=pend.get("packed_host"))
-        return self.collect(new, climatology)
+        return self.collect(new, climatology, trackers)
 
     # ------------------------------------------------------------------ convenience
     def run_batch(self, raw, gmax_nx=None, smoothed=None, intensity=None):
@@ -526,7 +529,7 @@ class Detector:
         return self.collect(slot)
 
     def stream(self, batches, depth=3, flags_host=None, shared_stream=False, gmax_nx="full", packed_host=None,
-               climatology=None):
+               climatology=None, trackers=None):
         """Pipelined execution: yields one BatchResult per input batch, in order.
 
         ``batches``: iterable of device or pinned-host tensors of (at most) equal length.  ``depth`` batches are
@@ -546,9 +549,14 @@ class Detector:
         The flag grids / contour set of a result are only valid until its slot is reused (``depth`` batches later).
         ``climatology``: a :class:`FlagClimatology`; the flag grids of every batch are added to its counters on the
         device (the batches take consecutive time steps of its group array, from its cursor on).
+        ``trackers``: a list of :class:`EventTracker` (for example one per kind); every batch's events are linked to the
+        events of the last ``time_range`` hours, whose polygons stay on the device.
         """
         if climatology is not None:
             climatology._check_detector(self)
+        trackers = list(trackers or ())
+        for tr in trackers:
+            tr._check_detector(self)
         common = None
         if shared_stream and self.lib.is_cuda:
             if getattr(self, "_shared", None) is None:
@@ -561,19 +569,23 @@ class Detector:
         seen_max = 0
         inflight = []
         i = 0
+        starts, submitted = [tr.cursor for tr in trackers], 0
         for raw in batches:
             idx = i % depth
             if len(inflight) == depth:
-                res = self.collect(inflight.pop(0), climatology)
+                res = self.collect(inflight.pop(0), climatology, trackers)
                 seen_max = max(seen_max, res.contours.max_nx)
                 yield res
+            for tr, start in zip(trackers, starts):  # before any device work on a batch the dates do not cover
+                tr._check_steps(start + submitted, int(raw.shape[0]))
+            submitted += int(raw.shape[0])
             slot = self._slot(int(raw.shape[0]), idx)
             fh = flags_host[idx] if flags_host is not None else None
             ph = packed_host[idx] if packed_host is not None else None
             inflight.append(self.submit(slot, raw, flags_host=fh, stream=common, gmax_nx=gmax_nx, packed_host=ph))
             i += 1
         while inflight:
-            res = self.collect(inflight.pop(0), climatology)
+            res = self.collect(inflight.pop(0), climatology, trackers)
             seen_max = max(seen_max, res.contours.max_nx)
             yield res
         if assumed and i > 0 and seen_max < full:
@@ -695,6 +707,328 @@ class FlagClimatology:
         """float64 ``[ngroups, 3, nlat, nlon]``: percent of the group's time steps in which a cell is flagged (NaN for
         groups without steps)."""
         return _percent(self.counts(), self._steps)
+
+
+TRACK_METHODS = ("by_overlap", "by_distance")
+
+
+class EventTracker:
+    """``track_events`` (events.py:151-241, ``buffer=0``) of one kind of event while ``Detector.stream`` runs.
+
+    ``dates``: the date of every time step of the record (datetime64 or numbers, increasing); an event of a batch that
+    starts at step ``cursor`` has the date ``dates[cursor + job // nlevels]``.  ``t0``: the step the first batch
+    starts at (the start of a rank's shard in a sharded run, ``sharding.shard_range``).  ``time_range`` (hours) is
+    required: the reference's default, the smallest positive gap between event dates, is only known at the end.
+
+    Only the polygons of the last ``time_range`` hours are kept, on the device, in the layout of
+    ``wbk_track_overlap_exact`` (``wbk_track_append`` builds them from the batch's device buffers, exactly as
+    :func:`events_soup` does on the host).  Every batch is linked against that window with the kernels and the
+    decision of :func:`tracking.link_events`; the links are kept as event ids on the host.  After the last batch
+    :meth:`labels` gives the labels of all events of the kind in the order of the concatenated batch tables, equal to
+    ``tracking.track_columnar`` on the whole record; :func:`sharding.finish_tracks` does the same for a sharded run.
+    """
+
+    def __init__(self, det, dates, kind, time_range, method="by_overlap", overlap=0, distance=1000, t0=0):
+        from . import tracking
+
+        if kind not in detect.KINDS:
+            raise ValueError("kind has to be one of {}, got {!r}".format(detect.KINDS, kind))
+        if method not in TRACK_METHODS:
+            raise ValueError("'{}' not supported as method! Supported methods are 'by_overlap' and 'by_distance'"
+                             .format(method))
+        if time_range is None:
+            raise ValueError("time_range (hours) is required for tracking in a stream")
+        self.kind, self.method = kind, method
+        self.overlap, self.distance, self.time_range = float(overlap), float(distance), time_range
+        self.lib = det.lib
+        self.nlat, self.nlon, self.nlevels = det.nlat, det.nlon, len(det.levels)
+        self.lat, self.lon = det.lat.copy(), det.lon.copy()
+        self._check_detector(det)
+        d = np.asarray(dates)
+        if d.ndim != 1:
+            raise ValueError("dates has to be a 1-D array over the time axis")
+        self.keys, window = tracking.time_keys(d)
+        if len(d) > 1 and not np.all(self.keys[1:] - self.keys[:-1] > 0):
+            raise ValueError("dates have to increase from one time step to the next")
+        if not 0 <= int(t0) <= len(d):
+            raise ValueError("t0 = {} is outside the dates array (length {})".format(t0, len(d)))
+        self.win = window(time_range)
+        self.cursor = int(t0)
+        self.n_events = 0
+        self.stats = dict(pairs_in_range=0, candidates=0, links=0, near=0)
+        self.host_ms = []  # host time of every batch's tracking step
+        self._links, self._near = [], []
+        # the head: events within time_range of the previous shard's last step (linked by the earlier ranks)
+        self._prev = self.keys[self.cursor - 1] if self.cursor > 0 else None
+        self._head = None if self._prev is not None else {}
+        # the window: device polygons + host keys / event ids / per-polygon ring and vertex counts
+        self._wkeys = self.keys[:0].copy()
+        self._wgid = np.zeros(0, dtype=np.int64)
+        self._wrad = np.zeros((0, 2))
+        self._wnr = np.zeros(0, dtype=np.int64)
+        self._wnv = np.zeros(0, dtype=np.int64)
+        self._nv = self._nr = 0
+        self._buf = None  # edges, vsign, ring_off, poly_off, bbox
+        # the tracker's own stream: its read-backs wait for its own work only, not for the batches queued behind the
+        # collected one (with shared_stream=True they would wait for the whole pipeline)
+        self._stream = torch.cuda.Stream(device=self.lib.device) if self.lib.is_cuda else None
+        self._done = torch.cuda.Event() if self.lib.is_cuda else None
+
+    def _on_stream(self):
+        return torch.cuda.stream(self._stream) if self._stream is not None else _null()
+
+    def _check_steps(self, first, nt):
+        """Refuse a batch of nt steps starting at step ``first`` that runs past the dates array."""
+        if first + nt > len(self.keys):
+            raise ValueError("the batch covers time steps {}..{} of the record, the dates array has {}".format(
+                first, first + nt - 1, len(self.keys)))
+
+    def _check_detector(self, det):
+        if self.method == "by_overlap" and not (det.want_flags and det.want_pieces):
+            raise ValueError("a by_overlap tracker needs the device clipper's pieces: build the Detector with "
+                             "want_flags=True and want_pieces=True")
+        if ((det.nlat, det.nlon) != (self.nlat, self.nlon) or len(det.levels) != self.nlevels
+                or not np.array_equal(det.lat, self.lat) or not np.array_equal(det.lon, self.lon)):
+            raise ValueError("the tracker is for a {} x {} grid with {} level(s), the Detector has a different grid "
+                             "({} x {}, {} level(s))".format(self.nlat, self.nlon, self.nlevels, det.nlat, det.nlon,
+                                                            len(det.levels)))
+
+    # ------------------------------------------------------------------ device window
+    def _reserve(self, nv, nr, npoly):
+        """Room for nv more vertices, nr more rings and npoly more polygons (grown by doubling)."""
+        need = (self._nv + nv, self._nr + nr + 1, len(self._wkeys) + npoly + 1)
+        b = self._buf
+        if b is not None and need[0] <= len(b[0]) and need[1] <= len(b[2]) and need[2] <= len(b[3]):
+            return
+        dev = self.lib.device
+        cap = [max(2 * c, 1024) for c in need]
+        if b is not None:
+            cap = [max(c, len(x)) for c, x in zip(cap, (b[0], b[2], b[3]))]
+        i32 = torch.int32
+        new = (torch.empty((cap[0], 4), dtype=i32, device=dev), torch.empty(cap[0], dtype=i32, device=dev),
+               torch.zeros(cap[1], dtype=i32, device=dev), torch.zeros(cap[2], dtype=i32, device=dev),
+               torch.empty((cap[2], 4), dtype=i32, device=dev))
+        if b is not None:
+            np_ = len(self._wkeys)
+            new[0][:self._nv].copy_(b[0][:self._nv])
+            new[1][:self._nv].copy_(b[1][:self._nv])
+            new[2][:self._nr + 1].copy_(b[2][:self._nr + 1])
+            new[3][:np_ + 1].copy_(b[3][:np_ + 1])
+            new[4][:np_].copy_(b[4][:np_])
+            if self.lib.is_cuda:
+                torch.cuda.current_stream(dev).synchronize()  # nothing reads the old window any more
+        self._buf = new
+
+    def _push(self, keys, gid, rad, nr, nv):
+        self._wkeys = np.concatenate([self._wkeys, keys])
+        self._wgid = np.concatenate([self._wgid, gid])
+        self._wrad = np.concatenate([self._wrad, rad])
+        self._wnr = np.concatenate([self._wnr, nr])
+        self._wnv = np.concatenate([self._wnv, nv])
+        self._nr += int(nr.sum())
+        self._nv += int(nv.sum())
+
+    def _evict(self, m):
+        """Drop the first m window events (their dates can no longer link to a later date)."""
+        if m == 0:
+            return
+        dr, dv = int(self._wnr[:m].sum()), int(self._wnv[:m].sum())
+        np_ = len(self._wkeys)
+        if self.method == "by_overlap" and self._buf is not None:
+            e, vs, ro, po, bb = self._buf
+            kv, kr, kp = self._nv - dv, self._nr - dr, np_ - m
+            e[:kv].copy_(e[dv:self._nv].clone())
+            vs[:kv].copy_(vs[dv:self._nv].clone())
+            ro[:kr + 1].copy_(ro[dr:self._nr + 1] - dv)
+            po[:kp + 1].copy_(po[m:np_ + 1] - dr)
+            bb[:kp].copy_(bb[m:np_].clone())
+        self._wkeys, self._wgid, self._wrad = self._wkeys[m:], self._wgid[m:], self._wrad[m:]
+        self._wnr, self._wnv = self._wnr[m:], self._wnv[m:]
+        self._nr -= dr
+        self._nv -= dv
+
+    def _snapshot(self, m):
+        """Host copy of the first m window events (the head of a shard)."""
+        dr, dv = int(self._wnr[:m].sum()), int(self._wnv[:m].sum())
+        h = dict(keys=self._wkeys[:m].copy(), gid=self._wgid[:m].copy(), rad=self._wrad[:m].copy(),
+                 nr=self._wnr[:m].copy(), nv=self._wnv[:m].copy())
+        if self.method == "by_overlap" and m:
+            e, vs, ro, po, bb = self._buf
+            h.update(edges=e[:dv].cpu().numpy(), vsign=vs[:dv].cpu().numpy(), ring_off=ro[:dr + 1].cpu().numpy(),
+                     poly_off=po[:m + 1].cpu().numpy(), bbox=bb[:m].cpu().numpy())
+        return h
+
+    def _append_host(self, h, gid):
+        """Append polygons given on the host (a published head) to the window."""
+        m = len(h["keys"])
+        if self.method == "by_overlap" and m:
+            self._reserve(int(h["nv"].sum()), int(h["nr"].sum()), m)
+            e, vs, ro, po, bb = self._buf
+            np_, dv = len(self._wkeys), len(h["edges"])
+            dev = self.lib.device
+            e[self._nv:self._nv + dv].copy_(torch.from_numpy(h["edges"]).to(dev))
+            vs[self._nv:self._nv + dv].copy_(torch.from_numpy(h["vsign"]).to(dev))
+            ro[self._nr:self._nr + len(h["ring_off"])].copy_(torch.from_numpy(h["ring_off"] + self._nv).to(dev))
+            po[np_:np_ + m + 1].copy_(torch.from_numpy(h["poly_off"] + self._nr).to(dev))
+            bb[np_:np_ + m].copy_(torch.from_numpy(h["bbox"]).to(dev))
+        self._push(h["keys"], gid, h["rad"], h["nr"], h["nv"])
+
+    # ------------------------------------------------------------------ linking
+    def _link(self, W, owned):
+        """Link the window events [0, owned) to the events [W, len) appended last.  Returns (pairs in range, links as
+        window positions)."""
+        from . import tracking
+
+        lib = self.lib
+        n = len(self._wkeys)
+        lo, hi = tracking.windows(self._wkeys, self.win)
+        lo[:W] = np.maximum(lo[:W], W)
+        lo[owned:] = hi[owned:]
+        hi = np.maximum(hi, lo)
+        n_in = int((hi - lo).sum())
+        empty = np.zeros((0, 2), dtype=np.int32)
+        if n_in == 0:
+            return 0, empty, empty
+        dev = lib.device
+        st = lib.stream()
+        d_lo, d_hi = torch.from_numpy(lo).to(dev), torch.from_numpy(hi).to(dev)
+        d_pairs = torch.empty((n_in, 2), dtype=torch.int32, device=dev)
+        d_count = torch.zeros(1, dtype=torch.int32, device=dev)
+        box = self._buf[4] if self.method == "by_overlap" and self.overlap >= 0 else None
+        lib.call("wbk_track_candidates", _lib.ptr(d_lo), _lib.ptr(d_hi), _lib.ptr(box), n, _lib.ptr(d_pairs), n_in,
+                 _lib.ptr(d_count), st)
+        m = int(d_count.cpu()[0])
+        pairs = d_pairs[:m].cpu().numpy()
+        if self.method == "by_distance":
+            links, near = tracking.decide_pairs(pairs, "by_distance", distance=self.distance, rad=self._wrad,
+                                                dist=lambda p: tracking.pair_distances(self._wrad, p))
+        else:
+            e, vs, ro, po, _ = self._buf
+
+            def exact(p):
+                d_p = torch.from_numpy(np.ascontiguousarray(p, dtype=np.int32)).to(dev)
+                out = torch.empty(len(p), dtype=torch.int32, device=dev)
+                lib.call("wbk_track_overlap_exact", _lib.ptr(e), _lib.ptr(vs), _lib.ptr(ro), _lib.ptr(po),
+                         _lib.ptr(d_p), len(p), _lib.ptr(out), lib.stream())
+                return out.cpu().numpy()
+
+            def areas(p):
+                if len(p) == 0:
+                    return np.zeros((0, 3))
+                xy = e[:self._nv, :2].to(torch.float64).contiguous()
+                d_p = torch.from_numpy(np.ascontiguousarray(p, dtype=np.int32)).to(dev)
+                out = torch.empty((len(p), 3), dtype=torch.float64, device=dev)
+                lib.call("wbk_track_overlap", _lib.ptr(xy), _lib.ptr(ro), _lib.ptr(po), _lib.ptr(d_p), len(p),
+                         _lib.ptr(out), lib.stream())
+                return out.cpu().numpy()
+
+            links, near = tracking.decide_pairs(pairs, "by_overlap", self.overlap, exact=exact, areas=areas)
+        self.stats["pairs_in_range"] += n_in
+        self.stats["candidates"] += len(pairs)
+        self.stats["links"] += len(links)
+        self.stats["near"] += len(near)
+        return n_in, links, near
+
+    def _add(self, slot, pend, tables, counts):
+        """Append and link the events of one collected batch, on the stream the batch ran on."""
+        import time
+
+        tick = time.perf_counter()
+        nt = int(pend["nt"])
+        self._check_steps(self.cursor, nt)
+        st = pend.get("stream")
+        with self._on_stream():
+            if st is not None:
+                self._stream.wait_event(slot.done)  # the batch's buffers (final: collect has waited for this event)
+            self._add_batch(slot, tables, counts, nt)
+            if st is not None:
+                # the slot's next batch overwrites the buffers wbk_track_append reads
+                self._done.record(self._stream)
+                st.wait_event(self._done)
+        self.cursor += nt
+        self.host_ms.append(1e3 * (time.perf_counter() - tick))
+
+    def _add_batch(self, slot, tables, counts, nt):
+        from . import tracking
+
+        k = detect.KINDS.index(self.kind)
+        tab = tables[self.kind]
+        n, first = len(tab), int(sum(counts[:k]))
+        keys = self.keys[self.cursor + tab.job.astype(np.int64) // self.nlevels]
+        gid = self.n_events + np.arange(n, dtype=np.int64)
+        rad = np.zeros((n, 2))
+        nr = np.zeros(n, dtype=np.int64)
+        nv = np.zeros(n, dtype=np.int64)
+        W = len(self._wkeys)
+        if n and self.method == "by_distance":
+            # the reference feeds (lon, lat) where haversine expects (lat, lon) (events.py:189-195); kept
+            props = detect.finish_properties(tab, self.lon, self.lat, self.nlon)
+            rad = np.radians(np.asarray(props["com"], dtype=np.float64).reshape(-1, 2))
+        elif n:
+            npc, _, clip_over = (int(v) for v in slot.h_sp_cnt.numpy()[:3])
+            if clip_over:
+                raise _lib.WbkError(_lib.ERR_CAPACITY, "the device clipper's arenas overflowed: the pieces of the events "
+                                                       "that straddle the last meridian are incomplete")
+            split = tab.split == 1
+            is_box = self.kind == "overturnings"
+            ro = slot.h_ring_off.numpy()
+            nv[:] = 4 if is_box else np.diff(ro[first:first + n + 1])
+            nr[:] = 1
+            pev = slot.h_sp_ev.numpy()[:npc].astype(np.int64) - first
+            plen = np.diff(slot.h_sp_off.numpy()[:npc + 1]).astype(np.int64)
+            mine = (pev >= 0) & (pev < n)
+            mine[mine] = split[pev[mine]]
+            nr[split] = np.bincount(pev[mine], minlength=n)[split]
+            nv[split] = np.bincount(pev[mine], weights=plen[mine], minlength=n).astype(np.int64)[split]
+            self._reserve(int(nv.sum()), int(nr.sum()), n)
+            e, vs, wro, wpo, bb = self._buf
+            lib = self.lib
+            lib.call("wbk_track_append", _lib.ptr(slot.ev_int), _lib.ptr(slot.ring_off), _lib.ptr(slot.ring_pts),
+                     _lib.ptr(slot.sp_ev), _lib.ptr(slot.sp_off), _lib.ptr(slot.sp_xy), npc, first, n, int(is_box),
+                     self.nlon, int(nr.sum()), int(nv.sum()), _lib.ptr(e), _lib.ptr(vs), _lib.ptr(wro), _lib.ptr(wpo),
+                     _lib.ptr(bb), self._nv, self._nr, W, len(e), len(wro), len(wpo), lib.stream())
+        self._push(keys, gid, rad, nr, nv)
+        self.n_events += n
+        if n:
+            _, links, near = self._link(W, len(self._wkeys))
+            self._links.append(self._wgid[links.astype(np.int64)].reshape(-1, 2))
+            self._near.append(self._wgid[near.astype(np.int64)].reshape(-1, 2))
+        # the head of a shard is complete once the next date lies beyond time_range of the previous shard's last step
+        end = self.cursor + nt
+        nxt = self.keys[end] if end < len(self.keys) else None
+        if self._head is None and (nxt is None or not nxt - self._prev <= self.win):
+            self._head = self._snapshot(self._head_size())
+        if nxt is None:
+            self._evict(len(self._wkeys))
+        else:
+            self._evict(int(np.count_nonzero(~(nxt - self._wkeys <= self.win))))
+
+    def _head_size(self):
+        return int(np.count_nonzero(self._wkeys - self._prev <= self.win))
+
+    # ------------------------------------------------------------------ results
+    def _pairs(self, parts):
+        out = np.concatenate(parts) if parts else np.zeros((0, 2), dtype=np.int64)
+        return out[np.lexsort((out[:, 1], out[:, 0]))] if len(out) else out
+
+    @property
+    def links(self):
+        """int64 [m, 2]: the linked event pairs (event ids in the order of the concatenated batch tables)."""
+        return self._pairs(self._links)
+
+    @property
+    def near(self):
+        """int64 [m, 2]: the pairs decided within ``tracking.NEAR_REL`` of a threshold (event ids, sorted)."""
+        return self._pairs(self._near)
+
+    def labels(self):
+        """int64 labels of all events tracked so far (``track_events``' ``label`` column in the order of the
+        concatenated batch tables).  Raises ValueError when no pair of events was in range, like the reference."""
+        from . import tracking
+
+        if self.stats["pairs_in_range"] == 0:
+            raise ValueError("No events detected in the time range: {}".format(self.time_range))
+        return tracking.labels_from_links(self.n_events, self.links)
 
 
 class _null:

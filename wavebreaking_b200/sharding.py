@@ -7,7 +7,8 @@ collective is needed.  Three small host-side merges remain (SURVEY.md 8e):
 1. ``exp_lon.max()`` is global over all dates (streamer_index.py:106) -> scalar MAX all-reduce;
 2. event ids / row indices are global (streamer_index.py:281-283) -> exclusive prefix sum of the per-rank counts;
 3. the event tables are gathered to rank 0 in rank (= time) order;
-4. ``track_events`` across shard boundaries: a halo of the event table (:func:`track_sharded`);
+4. ``track_events`` across shard boundaries: a halo of the event table (:func:`track_sharded`), or, for events
+   tracked while streaming, the heads of the later shards (:func:`finish_tracks`);
 5. flag-frequency climatologies: a SUM all-reduce of the per-rank counters (:func:`reduce_climatology`).
 """
 
@@ -74,6 +75,43 @@ def reduce_climatology(clim):
     dist.all_reduce(counts, op=dist.ReduceOp.SUM)
     dist.all_reduce(steps, op=dist.ReduceOp.SUM)
     return counts.cpu().numpy(), steps.cpu().numpy()
+
+
+def finish_tracks(tracker):
+    """Collective: the labels of the events a ``pipeline.EventTracker`` tracked on this rank, equal to the labels of
+    the single-process run over the whole record.  Every rank streams its shard with ``t0 = shard_range(...)[0]``.
+
+    Every rank publishes its head (its events dated within ``time_range`` of the previous shard's last step), links
+    the events still in its window (the tail of its shard) to the heads of all later ranks (several of them when
+    shards are shorter than ``time_range``), and the cross-shard links are merged by :func:`boundary_labels`.  Raises
+    ValueError on every rank when no pair of events was in range.  The near-threshold pairs of the cross-shard links
+    are not collected: after a sharded run ``tracker.near`` holds the pairs among the rank's own events only."""
+    rank, ws = world()
+    tr = tracker
+    n = tr.n_events
+    off, _ = exclusive_offset(n)
+    if tr._head is None:  # the shard ended before its head was complete: all of it is still in the window
+        with tr._on_stream():
+            tr._head = tr._snapshot(tr._head_size())
+    head = dict(tr._head, gid=tr._head["gid"] + off) if tr._head and len(tr._head["keys"]) else None
+    heads = _allgather(head)
+    W = len(tr._wkeys)
+    cross_local, cross_gid = np.zeros(0, dtype=np.int64), np.zeros(0, dtype=np.int64)
+    later = [h for h in heads[rank + 1:] if h is not None]
+    if W and later:
+        local_gid = tr._wgid.copy()
+        with tr._on_stream():  # ordered after the last batch's tracking step
+            for h in later:
+                tr._append_host(h, h["gid"])
+            _, links, _ = tr._link(W, W)
+        links = links.astype(np.int64).reshape(-1, 2)
+        cross_local, cross_gid = local_gid[links[:, 0]], tr._wgid[links[:, 1]]
+        with tr._on_stream():
+            tr._evict(len(tr._wkeys))
+    if sum(_allgather(int(tr.stats["pairs_in_range"]))) == 0:
+        raise ValueError("No events detected in the time range: {}".format(tr.time_range))
+    links = np.concatenate(tr._links) if tr._links else np.zeros((0, 2), dtype=np.int64)
+    return boundary_labels(n, off, links, cross_local, cross_gid)
 
 
 def gather_frames(frame, dst=0):
@@ -202,10 +240,22 @@ def track_sharded(dates, method="by_overlap", soup=None, com=None, time_range=No
     if tot_in_range == 0:
         raise ValueError("No events detected in the time range: {}".format(time_range))
     links = np.asarray(links, dtype=np.int64).reshape(-1, 2)
-    inner = links[links[:, 1] < n]
-    cmin = off + tracking.component_min(n, inner)  # global id of the smallest member of the local component
     cross = links[links[:, 1] >= n]
-    cross_edges = np.c_[cmin[cross[:, 0]], g_all[cross[:, 1]]] if len(cross) else np.zeros((0, 2), dtype=np.int64)
+    return boundary_labels(n, off, links[links[:, 1] < n], cross[:, 0], g_all[cross[:, 1]])
+
+
+def boundary_labels(n, off, inner, cross_local, cross_gid):
+    """Collective: dense labels of this rank's ``n`` events (global ids ``off`` .. ``off + n - 1``) from the links among
+    them (``inner``, local index pairs) and the links from local event ``cross_local[k]`` to the event with global id
+    ``cross_gid[k]`` of a later rank.  Equal to ``tracking.labels_from_links`` on the whole record."""
+    from . import tracking
+
+    rank, ws = world()
+    inner = np.asarray(inner, dtype=np.int64).reshape(-1, 2)
+    cross_local = np.asarray(cross_local, dtype=np.int64)
+    cmin = off + tracking.component_min(n, inner)  # global id of the smallest member of the local component
+    cross_edges = (np.c_[cmin[cross_local], np.asarray(cross_gid, dtype=np.int64)] if len(cross_local)
+                   else np.zeros((0, 2), dtype=np.int64))
     # ---- merge: resolve the far end of every cross link to ITS local component, then union-find on the few
     #      boundary components (every rank holds the same tiny graph)
     all_cross = np.concatenate([c for c in _allgather(cross_edges) if len(c)] or [np.zeros((0, 2), dtype=np.int64)])

@@ -347,6 +347,37 @@ def pair_distances(rad, pairs):
 NEAR_REL = 1e-9
 
 
+def decide_pairs(pairs, method, overlap=0, distance=1000, exact=None, areas=None, dist=None, rad=None):
+    """The linking decision of events.py:187-217 for candidate pairs of lattice polygons (``by_overlap``) or of centres
+    of mass (``by_distance``).  ``exact(pairs)``: the ``overlap_exact`` flags, ``areas(pairs)``: ``overlap_areas``,
+    ``dist(pairs)``: ``pair_distances`` on the unit sphere, ``rad``: the radians rows for the libm re-decision.
+    Returns ``(links, near)``: the linked pairs and the pairs decided within NEAR_REL of a threshold."""
+    near = np.zeros((0, 2), dtype=np.int32)
+    if method == "by_distance":
+        d = dist(pairs) * 6371
+        check = d < distance
+        close = np.abs(d - distance) <= NEAR_REL * abs(distance)
+        for k in np.nonzero(close)[0]:  # CUDA libm vs glibc: re-decide in the reference's arithmetic
+            check[k] = _haversine_libm(rad[pairs[k, 0]], rad[pairs[k, 1]]) * 6371 < distance
+        return pairs[check], pairs[close]
+    flag = exact(pairs)
+    pos = (flag & 1) == 1
+    if overlap == 0:
+        return pairs[pos], near
+    ratio = np.zeros(len(pairs))
+    if pos.any():
+        ar = areas(pairs[pos])
+        inter = np.maximum(ar[:, 2], np.finfo(np.float64).tiny)  # exact test says positive
+        ratio[pos] = inter / (ar[:, 1] + ar[:, 0] - inter)
+    if overlap < 0:
+        ar = areas(pairs[~pos])
+        with np.errstate(divide="ignore", invalid="ignore"):
+            ratio[~pos] = 0.0 / (ar[:, 1] + ar[:, 0])
+    with np.errstate(invalid="ignore"):
+        check = ratio > overlap
+    return pairs[check], pairs[pos & (np.abs(ratio - overlap) <= NEAR_REL)]
+
+
 def link_events(keys_sorted, win, method="by_overlap", soup=None, com=None, overlap=0, distance=1000, first=0,
                 last=None, stats=None):
     """Linked pairs among events sorted by ``keys_sorted`` (events.py:160-217).
@@ -374,13 +405,7 @@ def link_events(keys_sorted, win, method="by_overlap", soup=None, com=None, over
         pairs = candidate_pairs(lo, hi, None, first, last)
         # the reference feeds (lon, lat) where haversine expects (lat, lon) (events.py:189-195); kept
         rad = np.radians(np.asarray(com, dtype=np.float64).reshape(-1, 2))
-        d = pair_distances(rad, pairs) * 6371
-        check = d < distance
-        close = np.abs(d - distance) <= NEAR_REL * abs(distance)
-        for k in np.nonzero(close)[0]:  # CUDA libm vs glibc: re-decide in the reference's arithmetic
-            check[k] = _haversine_libm(rad[pairs[k, 0]], rad[pairs[k, 1]]) * 6371 < distance
-        near = pairs[close]
-        links = pairs[check]
+        links, near = decide_pairs(pairs, method, distance=distance, dist=lambda p: pair_distances(rad, p), rad=rad)
     elif method == "by_overlap":
         if overlap < 0:
             pairs = candidate_pairs(lo, hi, None, first, last)  # 0 / union > overlap holds for disjoint pairs too
@@ -392,24 +417,9 @@ def link_events(keys_sorted, win, method="by_overlap", soup=None, com=None, over
             pairs = candidate_pairs(lo, hi, box.astype(np.int32), first, last)
         lap("candidates")
         if soup.lattice:
-            flag = overlap_exact(soup, pairs)
+            links, near = decide_pairs(pairs, method, overlap, exact=lambda p: overlap_exact(soup, p),
+                                       areas=lambda p: overlap_areas(soup, p))
             lap("overlap_exact")
-            pos = (flag & 1) == 1
-            if overlap == 0:
-                check = pos
-            else:
-                ratio = np.zeros(len(pairs))
-                if pos.any():
-                    ar = overlap_areas(soup, pairs[pos])
-                    inter = np.maximum(ar[:, 2], np.finfo(np.float64).tiny)  # exact test says positive
-                    ratio[pos] = inter / (ar[:, 1] + ar[:, 0] - inter)
-                if overlap < 0:
-                    ar = overlap_areas(soup, pairs[~pos])
-                    with np.errstate(divide="ignore", invalid="ignore"):
-                        ratio[~pos] = 0.0 / (ar[:, 1] + ar[:, 0])
-                with np.errstate(invalid="ignore"):
-                    check = ratio > overlap
-                near = pairs[pos & (np.abs(ratio - overlap) <= NEAR_REL)]
         else:
             # polygons off any common lattice: float64 areas; an intersection below 1e-12 of the summed areas is
             # rounding noise of the triangle-fan sum and counts as empty (such pairs are listed as near)
@@ -420,7 +430,7 @@ def link_events(keys_sorted, win, method="by_overlap", soup=None, com=None, over
                 ratio = inter / (ar[:, 1] + ar[:, 0] - inter)
                 check = ratio > overlap
             near = pairs[(np.abs(ar[:, 2]) <= 10 * noise) | (np.abs(ratio - overlap) <= NEAR_REL)]
-        links = pairs[check]
+            links = pairs[check]
     else:
         raise ValueError("'{}' not supported as method! Supported methods are 'by_overlap' and 'by_distance'".format(method))
     if stats is not None:
