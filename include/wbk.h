@@ -219,7 +219,12 @@ int wbk_index_run(wbk_ctx* ctx, int njobs, int nlevels, const int* d_job_off, co
                   const wbk_index_params* params, void* stream);
 
 /* utils/index_utils.py:35-126 calculate_properties sums and processing/events.py:66-106 to_xarray flags for
- * the events of the last wbk_index_run.  d_data / d_intensity: [ntime, nlat, nlon] (intensity may be NULL).
+ * the events of the last wbk_index_run.  d_data: [ntime, nlat, nlon], latitude and longitude ascending.
+ * d_intensity: NULL (its sums are 0) or [ntime, nlat, nlon] of intensity_dtype (WBK_F32 / WBK_F64, independent of
+ * dtype), stored with descending latitudes / longitudes where intensity_flip_lat / intensity_flip_lon are set (the
+ * meaning of wbk_smooth_opts / wbk_flip): member cell (t, y, x) of the ascending grid is read from the stored array
+ * and widened to double, so the sums equal those of a converted, re-oriented copy bit for bit.  Only member cells
+ * are read.
  * d_flags: NULL or int8 [3][ntime][nlat][nlon] (kind-major), zeroed here and set to 1 where an event of that
  * kind is present; events that straddle the last meridian (split = 1 in their record) are clipped on the
  * device (utils/index_utils.py:148-173) and their pieces rasterised too.
@@ -230,8 +235,9 @@ int wbk_index_run(wbk_ctx* ctx, int njobs, int nlevels, const int* d_job_off, co
  * WBK_ERR_INVALID with a message.  The property sums use the radius (dlon + dlat) / 4 in index units on any grid
  * (index_utils.py:47-50). */
 int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* d_pt_off, const uint32_t* d_pts,
-                      const double* d_coords, const void* d_data, int dtype, const void* d_intensity, int ntime,
-                      int8_t* d_flags, const wbk_index_params* params, void* stream);
+                      const double* d_coords, const void* d_data, int dtype, const void* d_intensity,
+                      int intensity_dtype, int intensity_flip_lat, int intensity_flip_lon, int ntime, int8_t* d_flags,
+                      const wbk_index_params* params, void* stream);
 
 /* Near-threshold decisions of the streamer pair scan of the last wbk_index_run (streamer_index.py:130-139): every
  * pair (i < j, |x_i - x_j| <= 120) for which `geo < geo_dis` or `cont > cont_dis` was decided within 1e-9 (relative)

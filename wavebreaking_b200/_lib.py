@@ -75,7 +75,7 @@ _SIGNATURES = {
     "wbk_index_run": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p,
                               c_void_p, POINTER(IndexParams), c_void_p]),
     "wbk_events_raster": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int,
-                                  c_void_p, POINTER(IndexParams), c_void_p]),
+                                  c_int, c_int, c_int, c_void_p, POINTER(IndexParams), c_void_p]),
     "wbk_split_clip": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "wbk_split_fetch": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "wbk_pack_flags": (c_int, [c_void_p, c_void_p, ctypes.c_longlong, c_void_p]),

@@ -257,15 +257,19 @@ __global__ void __launch_bounds__(1024) event_list_kernel(WbkIdx x, int J, int n
 #define RS_ROWS_CAP 1024     // lattice rows of an event's bounding box that get an edge bucket
 #define RS_EDGE_CAP 8192     // edge incidences in the row buckets
 #define RS_PRE 4             // 32-column groups of a row whose field values are prefetched before the scan
+#define RS_NO_INTENSITY (-1)  // events_raster_kernel without an intensity field
 
 // r2_flag: the squared flag radius in cells (dlon == dlat), or with ANISO the squared extent r / min(dlon, dlat) of
-// fm's band, which is below one cell: R and the margins below are those of r2_prop wherever that is >= 1 cell
-template <typename T, bool ANISO>
+// fm's band, which is below one cell: R and the margins below are those of r2_prop wherever that is >= 1 cell.
+// IT: the intensity's dtype (WBK_F32 / WBK_F64), or RS_NO_INTENSITY (its sum stays 0 and `intensity` is not read).
+// The intensity is read in its stored orientation (iflip: bit 0 latitudes, bit 1 longitudes descending) and widened
+// to double, so the sums equal those of a converted, re-oriented copy bit for bit.
+template <typename T, bool ANISO, int IT>
 __global__ void __launch_bounds__(RS_THREADS, 3)
 events_raster_kernel(WbkDev d, WbkIdx x, const int* __restrict__ job_off, const int* __restrict__ pt_off,
                      const u32* __restrict__ pts, const double* __restrict__ area, const T* __restrict__ data,
-                     const T* __restrict__ intensity, int8_t* __restrict__ flags, int ntime, int nlevels, int J,
-                     int njobs, double r2_prop, double r2_flag, FlagMetric fm, int rowcap) {
+                     const void* __restrict__ intensity, int iflip, int8_t* __restrict__ flags, int ntime, int nlevels,
+                     int J, int njobs, double r2_prop, double r2_flag, FlagMetric fm, int rowcap) {
   WBK_DYN_SMEM(int, sm);
   __shared__ int s_box[5];
   __shared__ int s_scan[40];
@@ -396,7 +400,13 @@ events_raster_kernel(WbkDev d, WbkIdx x, const int* __restrict__ job_off, const 
           const int xf = fold_x(px, nlon);
           // sum(a) and sum(y * a) have one value per row: counted here, added once per row below
           dd_add(s_v, __dmul_rn(a, dv));
-          if (intensity) dd_add(s_i, __dmul_rn(a, (double)intensity[rowbase + xf]));
+          if (IT != RS_NO_INTENSITY) {
+            const int ys = (iflip & 1) ? nlat - 1 - y : y, xs = (iflip & 2) ? nlon - 1 - xf : xf;
+            const size_t k = ((size_t)t * nlat + ys) * nlon + xs;
+            const double iv = IT == WBK_F32 ? (double)static_cast<const float*>(intensity)[k]
+                                            : static_cast<const double*>(intensity)[k];
+            dd_add(s_i, __dmul_rn(a, iv));
+          }
           dd_add(s_x, __dmul_rn((double)px, a));
           ++row_members;
         }
@@ -824,11 +834,42 @@ static int grid_ratio(const char* who, double dlon, double dlat, FlagMetric* fm)
 }
 
 
+// one instantiation per (anisotropic metric, intensity dtype or none) of the data type T
+template <typename T>
+static int launch_events_raster(bool aniso, int it, size_t smem, cudaStream_t st, int grid, const WbkDev& d,
+                                const WbkIdx& x, const int* d_job_off, const int* d_pt_off, const uint32_t* d_pts,
+                                const double* area, const T* data, const void* intensity, int iflip, int8_t* d_flags,
+                                int ntime, int nlevels, int J, int njobs, double r2_prop, double r2_flag,
+                                const FlagMetric& fm, int rowcap) {
+  decltype(&events_raster_kernel<T, false, RS_NO_INTENSITY>) kern;
+  if (it == WBK_F32)
+    kern = aniso ? events_raster_kernel<T, true, WBK_F32> : events_raster_kernel<T, false, WBK_F32>;
+  else if (it == WBK_F64)
+    kern = aniso ? events_raster_kernel<T, true, WBK_F64> : events_raster_kernel<T, false, WBK_F64>;
+  else
+    kern = aniso ? events_raster_kernel<T, true, RS_NO_INTENSITY> : events_raster_kernel<T, false, RS_NO_INTENSITY>;
+  WBK_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  WBK_LAUNCH(KID_EVENTS_RASTER, kern, dim3(grid), dim3(RS_THREADS), smem, st, d, x, d_job_off, d_pt_off,
+             (const u32*)d_pts, area, data, intensity, iflip, d_flags, ntime, nlevels, J, njobs, r2_prop, r2_flag, fm,
+             rowcap);
+  WBK_LAUNCH_CHECK();
+  return WBK_OK;
+}
+
 extern "C" int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* d_pt_off, const uint32_t* d_pts,
                                  const double* d_coords, const void* d_data, int dtype, const void* d_intensity,
-                                 int ntime, int8_t* d_flags, const wbk_index_params* prm, void* stream) {
+                                 int intensity_dtype, int intensity_flip_lat, int intensity_flip_lon, int ntime,
+                                 int8_t* d_flags, const wbk_index_params* prm, void* stream) {
   if (!ctx || !d_job_off || !d_pt_off || !d_coords || !d_data || !prm || ntime < 0) {
     wbk_set_error("wbk_events_raster: invalid argument");
+    return WBK_ERR_INVALID;
+  }
+  if (dtype != WBK_F32 && dtype != WBK_F64) {
+    wbk_set_error("wbk_events_raster: unsupported dtype");
+    return WBK_ERR_INVALID;
+  }
+  if (d_intensity && intensity_dtype != WBK_F32 && intensity_dtype != WBK_F64) {
+    wbk_set_error("wbk_events_raster: unsupported intensity dtype %d", intensity_dtype);
     return WBK_ERR_INVALID;
   }
   FlagMetric fm;
@@ -857,23 +898,18 @@ extern "C" int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* 
                       (size_t)(2 * RS_ROWS_CAP + 1) * sizeof(int) + (size_t)RS_EDGE_CAP * sizeof(unsigned short);
   const double* area = d_coords + 3 * (size_t)d.nlat;
   const int grid = 148 * 9;
-  if (dtype == WBK_F32) {
-    auto kern = aniso ? events_raster_kernel<float, true> : events_raster_kernel<float, false>;
-    WBK_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    WBK_LAUNCH(KID_EVENTS_RASTER, kern, dim3(grid), dim3(RS_THREADS), smem, st, d, ctx->x, d_job_off, d_pt_off,
-               (const u32*)d_pts, area, (const float*)d_data, (const float*)d_intensity, d_flags, ntime, ctx->nlevels, J,
-               njobs, r_prop * r_prop, r_flag * r_flag, fm, rowcap);
-  } else if (dtype == WBK_F64) {
-    auto kern = aniso ? events_raster_kernel<double, true> : events_raster_kernel<double, false>;
-    WBK_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    WBK_LAUNCH(KID_EVENTS_RASTER, kern, dim3(grid), dim3(RS_THREADS), smem, st, d, ctx->x, d_job_off, d_pt_off,
-               (const u32*)d_pts, area, (const double*)d_data, (const double*)d_intensity, d_flags, ntime, ctx->nlevels,
-               J, njobs, r_prop * r_prop, r_flag * r_flag, fm, rowcap);
-  } else {
-    wbk_set_error("wbk_events_raster: unsupported dtype");
-    return WBK_ERR_INVALID;
-  }
-  WBK_LAUNCH_CHECK();
+  const int it = d_intensity ? intensity_dtype : RS_NO_INTENSITY;
+  const int iflip = (intensity_flip_lat ? 1 : 0) | (intensity_flip_lon ? 2 : 0);
+  int rc;
+  if (dtype == WBK_F32)
+    rc = launch_events_raster<float>(aniso, it, smem, st, grid, d, ctx->x, d_job_off, d_pt_off, d_pts, area,
+                                     (const float*)d_data, d_intensity, iflip, d_flags, ntime, ctx->nlevels, J, njobs,
+                                     r_prop * r_prop, r_flag * r_flag, fm, rowcap);
+  else
+    rc = launch_events_raster<double>(aniso, it, smem, st, grid, d, ctx->x, d_job_off, d_pt_off, d_pts, area,
+                                      (const double*)d_data, d_intensity, iflip, d_flags, ntime, ctx->nlevels, J, njobs,
+                                      r_prop * r_prop, r_flag * r_flag, fm, rowcap);
+  if (rc != WBK_OK) return rc;
   ctx->split_clipped = d_flags != nullptr;
   if (d_flags) {
     // events straddling the last meridian: clip on the device, rasterise the pieces

@@ -60,6 +60,25 @@ def _pinned(shape, dtype, lib):
     return torch.empty(shape, dtype=dtype, pin_memory=lib.is_cuda)
 
 
+def _intensity_item(item, shape):
+    """One intensity item of ``Detector.stream`` as the tuple ``(field,)`` or ``(u, v)``; raises ValueError unless its
+    tensors are float32 / float64 and shaped like the batch (``shape``), and u and v agree in shape and dtype."""
+    fields = tuple(item) if isinstance(item, (tuple, list)) else (item,)
+    if len(fields) not in (1, 2) or not all(isinstance(f, torch.Tensor) for f in fields):
+        raise ValueError("an intensity item is a tensor or a pair (u, v) of tensors")
+    if len(fields) == 2 and (fields[0].shape != fields[1].shape or fields[0].dtype != fields[1].dtype):
+        raise ValueError("u and v differ: shapes {} and {}, dtypes {} and {}".format(
+            tuple(fields[0].shape), tuple(fields[1].shape), fields[0].dtype, fields[1].dtype))
+    for f in fields:
+        if f.dtype not in (torch.float32, torch.float64):
+            raise ValueError("intensity has to be float32 or float64, got {} (packed int16 u / v are not "
+                             "supported)".format(f.dtype))
+        if tuple(f.shape) != tuple(shape):
+            raise ValueError("an intensity item of shape {} for a batch of shape {}".format(tuple(f.shape),
+                                                                                          tuple(shape)))
+    return fields
+
+
 class _Slot:
     """Context + device / pinned buffers + stream for one batch in flight."""
 
@@ -91,6 +110,8 @@ class _Slot:
         self.sm_f32 = None
         self.sm_tmp = torch.empty(shape, dtype=f64, device=dev) if det.passes > _lib.SMOOTH_MAX_FUSED else None
         self.raw_dev = None  # allocated on first host submit
+        self.inten_dev = [None, None]  # uploads of host intensity items (the field, or u and v), on first use
+        self.mflux = None  # momentum flux of (u, v) intensity items, on first use
         self.flipped = None
         self.job_off = torch.empty(J + 1, dtype=i32, device=dev)
         self.pt_off = torch.empty(self.cap_c + 1, dtype=i32, device=dev)
@@ -234,7 +255,18 @@ class Detector:
             raw = slot.raw_dev[:nt]
         raw = raw.contiguous()
         raw_in = raw  # what the caller handed over (the regrow path re-submits exactly this)
-        if intensity is not None:
+        if isinstance(intensity, tuple):  # the field or (u, v) as stored: host items go to the slot's own buffers
+            fields = []
+            for k, f in enumerate(intensity):
+                if f.device != lib.device:
+                    if slot.inten_dev[k] is None or slot.inten_dev[k].dtype != f.dtype:
+                        slot.inten_dev[k] = torch.empty((slot.T, self.nlat, self.nlon), dtype=f.dtype,
+                                                        device=lib.device)
+                    slot.inten_dev[k][:nt].copy_(f, non_blocking=True)
+                    f = slot.inten_dev[k][:nt]
+                fields.append(f.contiguous())
+            intensity = tuple(fields)
+        elif intensity is not None:
             intensity = intensity.to(lib.device).contiguous()
         if nvtx:
             nvtx.range_pop()
@@ -281,7 +313,7 @@ class Detector:
         if nvtx:
             nvtx.range_pop()
             nvtx.range_push("wbk.indices")
-        if intensity is not None and intensity.dtype != sm.dtype:
+        if isinstance(intensity, torch.Tensor) and intensity.dtype != sm.dtype:
             intensity = intensity.to(sm.dtype)
         prm = self._prm(-1 if gmax_nx is None else gmax_nx)
         lib.call("wbk_index_run", h, nt * L, L, _lib.ptr(slot.job_off), _lib.ptr(slot.pt_off), _lib.ptr(slot.meta),
@@ -300,9 +332,23 @@ class Detector:
                     slot.flags = torch.empty((3, slot.T, self.nlat, self.nlon), dtype=torch.int8, device=lib.device)
                 flags = slot.flags if nt == slot.T else torch.empty((3, nt, self.nlat, self.nlon), dtype=torch.int8,
                                                                     device=lib.device)
+        # the rasteriser reads the intensity's member cells in their stored dtype and orientation
+        inten, iflip = intensity, (0, 0)
+        if isinstance(intensity, tuple):
+            inten, iflip = intensity[0], (int(self.flip_lat), int(self.flip_lon))
+            if len(intensity) == 2:
+                # zonal means summed in the stored memory order (what numpy does on the user's array); longitude is
+                # the contiguous axis of a batch
+                u, v = intensity
+                if slot.mflux is None or slot.mflux.dtype != u.dtype:
+                    slot.mflux = torch.empty((slot.T, self.nlat, self.nlon), dtype=u.dtype, device=lib.device)
+                inten = slot.mflux[:nt]
+                lib.call("wbk_mflux", _lib.ptr(u), _lib.ptr(v), _lib.ptr(inten), _lib.dtype_code(u.dtype), nt,
+                         self.nlat, self.nlon, 0, st)
         lib.call("wbk_events_raster", h, _lib.ptr(slot.job_off), _lib.ptr(slot.pt_off), _lib.ptr(slot.pts),
-                 _lib.ptr(self.coords), _lib.ptr(sm), _lib.dtype_code(sm.dtype),
-                 None if intensity is None else _lib.ptr(intensity), nt, _lib.ptr(flags), ctypes.byref(prm), st)
+                 _lib.ptr(self.coords), _lib.ptr(sm), _lib.dtype_code(sm.dtype), _lib.ptr(inten),
+                 _lib.dtype_code(sm.dtype if inten is None else inten.dtype), iflip[0], iflip[1], nt, _lib.ptr(flags),
+                 ctypes.byref(prm), st)
         lib.call("wbk_batch_fetch", h, _lib.ptr(slot.pt_off), _lib.ptr(slot.pts), _lib.ptr(slot.ev_int),
                  _lib.ptr(slot.ev_f64), _lib.ptr(slot.ev_job), _lib.ptr(slot.ring_off), _lib.ptr(slot.ring_pts),
                  slot.cap_e, slot.cap_r, _lib.ptr(slot.summary), st)
@@ -339,8 +385,9 @@ class Detector:
             packed_host[:nb].copy_(slot.packed[:nb], non_blocking=True)
         if nvtx:
             nvtx.range_pop()
+        # (inten keeps the buffer a captured graph writes the momentum flux to alive)
         return dict(raw=raw_in, nt=nt, flags=flags, flags_host=flags_host, gmax=gmax_nx, smoothed=smoothed, sm=sm,
-                    intensity=intensity, packed_host=packed_host)
+                    intensity=intensity, inten=inten, packed_host=packed_host)
 
     def submit(self, slot, raw, flags_out=None, flags_host=None, gmax_nx=None, smoothed=None, stream=None,
                intensity=None, packed_host=None):
@@ -349,22 +396,29 @@ class Detector:
 
         With ``Detector(graphs=True)`` the whole batch (uploads, ~25 kernels and memsets, downloads) is captured into
         ONE CUDA graph per (slot, buffers) the second time the same buffers are submitted and replayed afterwards: one
-        launch per batch instead of ~40 driver calls, which is what limits several ranks sharing one host."""
+        launch per batch instead of ~40 driver calls, which is what limits several ranks sharing one host.
+
+        ``intensity``: a device tensor [T', nlat, nlon] in the ascending orientation, converted to the smoothed
+        field's dtype (as in ``detect.run_indices``; not captured in a graph), or a tuple ``(field,)`` / ``(u, v)``
+        in the form of :meth:`stream`'s items (stored orientation, own dtype, captured with the batch)."""
         lib = self.lib
         nt = int(raw.shape[0])
         if nt > slot.T:
             raise ValueError("batch of {} time steps exceeds the slot size {}".format(nt, slot.T))
+        if isinstance(intensity, tuple):
+            intensity = _intensity_item(intensity, raw.shape)
         use_stream = stream if stream is not None else slot.stream
         args = (slot, raw, flags_out, flags_host, gmax_nx, smoothed, intensity, packed_host)
         if use_stream is None:  # emulator
             slot.pending = dict(self._enqueue(*args), stream=None)
             return slot
-        graphable = self.graphs and smoothed is None and intensity is None
+        graphable = self.graphs and smoothed is None and not isinstance(intensity, torch.Tensor)
         key = None
         if graphable:
             key = (raw.data_ptr(), raw.dtype, nt, None if flags_out is None else flags_out.data_ptr(),
                    None if flags_host is None else flags_host.data_ptr(),
-                   None if packed_host is None else packed_host.data_ptr(), gmax_nx, use_stream.cuda_stream)
+                   None if packed_host is None else packed_host.data_ptr(), gmax_nx, use_stream.cuda_stream,
+                   None if intensity is None else tuple((f.data_ptr(), f.dtype, f.device.type) for f in intensity))
         with torch.cuda.stream(use_stream):
             use_stream.wait_stream(torch.cuda.default_stream(lib.device))
             if key is not None and key in slot.graphs:
@@ -529,7 +583,7 @@ class Detector:
         return self.collect(slot)
 
     def stream(self, batches, depth=3, flags_host=None, shared_stream=False, gmax_nx="full", packed_host=None,
-               climatology=None, trackers=None):
+               climatology=None, trackers=None, intensity=None):
         """Pipelined execution: yields one BatchResult per input batch, in order.
 
         ``batches``: iterable of device or pinned-host tensors of (at most) equal length.  ``depth`` batches are
@@ -551,7 +605,16 @@ class Detector:
         device (the batches take consecutive time steps of its group array, from its cursor on).
         ``trackers``: a list of :class:`EventTracker` (for example one per kind); every batch's events are linked to the
         events of the last ``time_range`` hours, whose polygons stay on the device.
+        ``intensity``: an iterable consumed in step with ``batches``; its item for a batch is a device or pinned-host
+        tensor shaped like the batch, float32 or float64, in the batch's stored orientation, or a pair ``(u, v)`` of
+        such tensors whose momentum flux (``wbk_mflux``, the reference's ``calculate_momentum_flux``) is computed on
+        the device.  Every event gets the area-weighted mean of it over its cells (the ``intensity`` column), the same
+        field for every contour level; without it that column is 0.  Host items are uploaded into the slot's own
+        buffers, so the batch, the upload and the momentum flux included, is captured in its CUDA graph.  A batch is
+        (time, lat, lon) with longitude contiguous, so the zonal means of the momentum flux are summed pairwise, as
+        ``spatial.momentum_flux(u, v, lon_contiguous=True)`` does.
         """
+        inten_it = iter(intensity) if intensity is not None else None
         if climatology is not None:
             climatology._check_detector(self)
         trackers = list(trackers or ())
@@ -576,13 +639,20 @@ class Detector:
                 res = self.collect(inflight.pop(0), climatology, trackers)
                 seen_max = max(seen_max, res.contours.max_nx)
                 yield res
+            item = None
+            if inten_it is not None:  # checked before any device work on the batch
+                item = next(inten_it, None)
+                if item is None:
+                    raise ValueError("the intensity iterable ended before the batches (batch {})".format(i))
+                item = _intensity_item(item, raw.shape)
             for tr, start in zip(trackers, starts):  # before any device work on a batch the dates do not cover
                 tr._check_steps(start + submitted, int(raw.shape[0]))
             submitted += int(raw.shape[0])
             slot = self._slot(int(raw.shape[0]), idx)
             fh = flags_host[idx] if flags_host is not None else None
             ph = packed_host[idx] if packed_host is not None else None
-            inflight.append(self.submit(slot, raw, flags_host=fh, stream=common, gmax_nx=gmax_nx, packed_host=ph))
+            inflight.append(self.submit(slot, raw, flags_host=fh, stream=common, gmax_nx=gmax_nx, packed_host=ph,
+                                        intensity=item))
             i += 1
         while inflight:
             res = self.collect(inflight.pop(0), climatology, trackers)

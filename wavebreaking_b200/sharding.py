@@ -129,11 +129,13 @@ def gather_frames(frame, dst=0):
     return pd.concat(parts).reset_index(drop=True) if parts else frame.iloc[:0]
 
 
-def run_sharded(detector, raw_full_or_shard, ntime_total=None, is_shard=False):
+def run_sharded(detector, raw_full_or_shard, ntime_total=None, is_shard=False, intensity=None):
     """Run ``detector`` on this rank's block of time steps with the global exp_lon maximum.
 
     Returns ``(t0, t1, BatchResult)``.  If the maximum of another rank exceeds the local one, the index
     stage is re-run with the global value (rare: every step normally has a full-width contour).
+    ``intensity``: a tensor or a pair ``(u, v)`` shaped and stored like the field (an item of ``Detector.stream``'s
+    ``intensity``), sliced like it.
     """
     rank, ws = world()
     if is_shard:
@@ -142,10 +144,15 @@ def run_sharded(detector, raw_full_or_shard, ntime_total=None, is_shard=False):
     else:
         t0, t1 = shard_range(raw_full_or_shard.shape[0], rank, ws)
         shard = raw_full_or_shard[t0:t1]
-    res = detector.run_batch(shard)
+    item = None
+    if intensity is not None:
+        item = tuple(intensity) if isinstance(intensity, (tuple, list)) else (intensity,)
+        if not is_shard:
+            item = tuple(f[t0:t1] for f in item)
+    res = detector.run_batch(shard, intensity=item)
     g = global_max(res.gmax_nx)
     if g != res.gmax_nx:
-        res = detector.run_batch(shard, gmax_nx=g)
+        res = detector.run_batch(shard, gmax_nx=g, intensity=item)
     return t0, t1, res
 
 
