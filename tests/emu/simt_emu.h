@@ -240,7 +240,18 @@ struct float2 { float x, y; };
 struct int2 { int x, y; };
 struct int4 { int x, y, z, w; };
 struct uint4 { unsigned x, y, z, w; };
+#ifdef WBK_EMU_SINF_WORST
+// __sinf at the worst case the CUDA programming guide documents for it (maximum absolute error 2^-21.41 on
+// [-pi, pi]): the correctly rounded sine moved by that much, the sign alternating from call to call, so that the
+// fp32 prefilter of the pair scan is checked against the documented bound rather than against an exact sine
+inline float __sinf(float v) {
+  static thread_local unsigned calls = 0;
+  const double e = 3.6471e-7;  // 2^-21.41, rounded up
+  return (float)((double)std::sin(v) + ((calls++ & 1u) ? e : -e));
+}
+#else
 inline float __sinf(float v) { return std::sin(v); }
+#endif
 inline double2 make_double2(double x, double y) { double2 r; r.x = x; r.y = y; return r; }
 inline float4 make_float4(float x, float y, float z, float w) { float4 r; r.x = x; r.y = y; r.z = z; r.w = w; return r; }
 inline uint4 make_uint4(unsigned x, unsigned y, unsigned z, unsigned w) { uint4 r; r.x = x; r.y = y; r.z = z; r.w = w; return r; }

@@ -464,15 +464,29 @@ __global__ void __launch_bounds__(ST_THREADS) streamer_prep_kernel(WbkDev d, Wbk
         // cont(i, j) = pfx[j] - pfx[i] <= max pfx(bj) - min pfx(bi) (the rounded subtraction is monotone)
         if (!(__dsub_rn(bp[2 * bj + 1], bp[2 * bi]) > cont_dis * (1.0 - 2e-9))) continue;  // keeps the tolerance band
         // lower bound of the great-circle distance between the two blocks' bounding boxes: the latitude gap, and
-        // the longitude gap at the most poleward latitude (h >= cos^2(lat_max) sin^2(dlon/2)); tiles that cannot
-        // reach geo_dis are left out (1e-6 relative slack; x gaps <= 120 columns are never folded)
+        // the longitude gap at the most poleward latitude (h >= cos^2(lat_max) min sin^2(dlon/2) over the blocks'
+        // column gaps [xgap, xgap_max]); tiles that cannot reach geo_dis are left out (1e-6 relative slack).  The
+        // reference measures longitudes after x % nlon, so a column gap g is the longitude gap g * dlon folded
+        // into a circle: while g * dlon < 180 degrees sin(dlon/2) grows with g and the smallest gap bounds it;
+        // past 180 degrees (coarse grids, or the pole-ward ends of 2.5-degree grids) it shrinks again and is 0 at
+        // g = nlon (a point and its periodic copy), so the minimum over the whole range is taken.
         const int ygap = max(max(bx[4 * bj + 2] - bx[4 * bi + 3], bx[4 * bi + 2] - bx[4 * bj + 3]), 0);
         if (EARTH_R * (dlat_deg * ygap * d2r) > geo_dis * 1.000001) continue;
         if (xgap > 0) {
           const double lat_lo = ct.lat_deg[min(bx[4 * bi + 2], bx[4 * bj + 2])], lat_hi = ct.lat_deg[max(bx[4 * bi + 3], bx[4 * bj + 3])];
           const double amax = fmax(fabs(lat_lo), fabs(lat_hi));
+          const int xgap_max = max(bx[4 * bj + 1] - bx[4 * bi], bx[4 * bi + 1] - bx[4 * bj]);
           const double dlon = prm_dlon * xgap * d2r;
-          const double lb_lon = 2.0 * EARTH_R * asin(fmin(1.0, cos(fmin(amax, 90.0) * d2r) * sin(fmin(0.5 * dlon, 1.5707963267948966))));
+          double s_lon;
+          if (prm_dlon * xgap_max < 180.0) {
+            s_lon = sin(fmin(0.5 * dlon, 1.5707963267948966));
+          } else if (xgap_max / nlon > (xgap - 1) / nlon) {
+            s_lon = 0.0;  // some gap in the range is a whole number of turns
+          } else {
+            // |sin(g dlon / 2)| is concave between two of its zeros: its minimum over the range is at an end
+            s_lon = fmin(fabs(sin(0.5 * dlon)), fabs(sin(0.5 * (prm_dlon * xgap_max * d2r))));
+          }
+          const double lb_lon = 2.0 * EARTH_R * asin(fmin(1.0, cos(fmin(amax, 90.0) * d2r) * s_lon));
           if (lb_lon > geo_dis * 1.000001) continue;
         }
         const int pos = atomicAdd(&x.total[0], 1);
@@ -488,9 +502,12 @@ __global__ void __launch_bounds__(ST_THREADS) streamer_prep_kernel(WbkDev d, Wbk
 // without materialising the N x N matrices.  One WARP per 32 x 32 tile of the batch-wide active-tile list (lane = the
 // point i of block bi, the 32 points of block bj are broadcast from shared memory); warps stride over the list on
 // their own, no block barrier.  The haversine test is decided in fp32 on
-// h = sin^2(dlat/2) + cos cos sin^2(dlon/2) against sin^2(geo_dis / 2R) with a 1e-4 relative margin; only pairs
-// inside the margin evaluate the reference's fp64 expression (and carry the near-threshold flag).
+// h = sin^2(dlat/2) + cos cos sin^2(dlon/2) against sin^2(geo_dis / 2R) with a margin derived from the error bounds
+// of __sinf and of fp32 (below); only pairs inside the margin evaluate the reference's fp64 expression (and carry the
+// near-threshold flag).
 #define PS_WARPS (PS_THREADS / 32)
+#define PS_EPS_S 1.25e-6  // absolute error bound of sqrt(h) in fp32
+#define PS_EPS_H 1e-6     // relative error bound of h from the fp32 roundings
 #define PS_BUF 256
 #ifndef PS_MINCTA
 #define PS_MINCTA 3  // resident CTAs per SM the register budget is sized for (2 -> 3: 1.03 -> 0.83 us per step)
@@ -504,9 +521,19 @@ __global__ void __launch_bounds__(PS_THREADS, PS_MINCTA) pair_scan_kernel(WbkDev
   __shared__ u64 sbuf[PS_WARPS][PS_BUF];  // candidates of the current tile
   const int lane = wbk_lane(), warp = wbk_warp(), nlon = d.nlon;
   const int total = min(x.total[0], x.TLC);
+  // margin of the fp32 test, from an absolute error bound on s = sqrt(h) = sin(distance / 2R):
+  //   __sinf: 2^-21.41 absolute on [-pi, pi] (CUDA C programming guide), 3.65e-7 per sine;
+  //   latitude sine argument: two latitudes rounded to fp32 (|lat| <= pi/2, 2^-24 each), their difference
+  //     (|.| <= pi, 2^-23), halved: 1.2e-7;
+  //   longitude sine argument: two longitudes rounded to fp32 (|lon| < 2 pi, 2^-22 each), their difference
+  //     (2^-22), halved: 3.6e-7;
+  //   so |s0 - s0_f| <= 4.85e-7, |s1 - s1_f| <= 7.25e-7 and |s - s_f| <= |s0 - s0_f| + |s1 - s1_f| < PS_EPS_S;
+  //   relative: cos(lat) in fp32, the products and the sum of non-negative terms in fp32 and the rounding of the
+  //     bounds to fp32 are each 2^-24 of h, a dozen of them < PS_EPS_H.
+  // A fixed relative margin is too narrow at small geo_dis: the absolute sine error is then a large part of s.
   const double sthr = sin(prm.geo_dis / (2.0 * EARTH_R));
-  const float hthr = (float)(sthr * sthr);
-  const float h_lo = hthr * 0.9999f, h_hi = hthr * 1.0001f;
+  const double s_lo = fmax(sthr - PS_EPS_S, 0.0), s_hi = sthr + PS_EPS_S;
+  const float h_lo = (float)(s_lo * s_lo * (1.0 - PS_EPS_H)), h_hi = (float)(s_hi * s_hi * (1.0 + PS_EPS_H));
   const int nwarps_grid = gridDim.x * PS_WARPS;
   for (int w = blockIdx.x * PS_WARPS + warp; w < total; w += nwarps_grid) {
     const u64 tl = x.tile_list[w];
