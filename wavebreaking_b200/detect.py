@@ -27,6 +27,18 @@ def default_caps(nlat, nlon, add, njobs):
                 pair_cap=p2(48 * W), event_cap=256)
 
 
+def grow_caps(caps, status):
+    """The context capacities of ``caps`` that a run with ``status`` (the OR of its status bits) outgrew, each
+    multiplied by its growth factor; empty when no context arena overflowed."""
+    grow = {}
+    for bit, key, factor in ((_lib.ST_SEG_OVERFLOW, "seg_cap", 2), (_lib.ST_CONTOUR_OVERFLOW, "contour_cap", 2),
+                             (_lib.ST_PAIR_OVERFLOW, "pair_cap", 4), (_lib.ST_EVENT_OVERFLOW, "event_cap", 4),
+                             (_lib.ST_SEL_OVERFLOW, "sel_cap", 4)):
+        if status & bit:
+            grow[key] = caps[key] * factor
+    return grow
+
+
 class Context:
     """Owns a wbk_ctx and its torch-allocated device workspace."""
 
@@ -160,10 +172,7 @@ def contours(field, levels, add, caps=None):
                      lib.stream())
             break
         except _lib.CapacityError:
-            if status.max() & _lib.ST_SEG_OVERFLOW or np.any(status & _lib.ST_SEG_OVERFLOW):
-                grow["seg_cap"] = ctx.caps["seg_cap"] * 2
-            if np.any(status & _lib.ST_CONTOUR_OVERFLOW):
-                grow["contour_cap"] = ctx.caps["contour_cap"] * 2
+            grow.update(grow_caps(ctx.caps, int(np.bitwise_or.reduce(status))))
     else:
         raise _lib.WbkError(_lib.ERR_CAPACITY, "contour arenas still overflow after 8 regrowths")
     nc, npnt, status = nc[:njobs], npnt[:njobs], status[:njobs]
@@ -297,12 +306,7 @@ def run_indices(cs, data, coords, dlon, dlat, intensity=None, which=KINDS, gmax_
             lib.call("wbk_events_counts", ctx.handle, _iptr(counts), _iptr(status), lib.stream())
             break
         except _lib.CapacityError:
-            if np.any(status & _lib.ST_PAIR_OVERFLOW):
-                grow["pair_cap"] = ctx.caps["pair_cap"] * 4
-            if np.any(status & _lib.ST_EVENT_OVERFLOW):
-                grow["event_cap"] = ctx.caps["event_cap"] * 4
-            if np.any(status & _lib.ST_SEL_OVERFLOW):
-                grow["sel_cap"] = ctx.caps["sel_cap"] * 4
+            grow.update(grow_caps(ctx.caps, int(np.bitwise_or.reduce(status))))
     else:
         raise _lib.WbkError(_lib.ERR_CAPACITY, "index arenas still overflow after 8 regrowths")
     counts = counts.reshape(3, -1)[:, :cs.njobs] if cs.njobs else counts[:, :0]

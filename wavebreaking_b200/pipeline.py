@@ -15,7 +15,7 @@ host<->device copies overlap with kernels (``Detector.stream``).
 
 import ctypes
 import logging
-from dataclasses import dataclass
+from dataclasses import dataclass, replace
 
 import numpy as np
 import torch
@@ -79,84 +79,81 @@ def _intensity_item(item, shape):
     return fields
 
 
+@dataclass
+class _Pending:
+    """One submitted batch: what ``collect`` reads, and what a re-run with larger arenas submits again."""
+
+    raw: torch.Tensor
+    nt: int
+    flags: torch.Tensor
+    flags_host: torch.Tensor
+    packed_host: torch.Tensor
+    gmax: int
+    smoothed: torch.Tensor
+    intensity: object
+    stream: object = None
+    # the smoothed / oriented field and the momentum flux: a captured graph writes to them, and its record in
+    # slot.graphs keeps them alive after the slot has replaced such a buffer with one of another dtype
+    graph_bufs: tuple = ()
+
+
 class _Slot:
     """Context + device / pinned buffers + stream for one batch in flight."""
 
-    def __init__(self, det, T, caps=None):
+    def __init__(self, det, T, grown=None):
         lib = det.lib
         self.det, self.T = det, int(T)
         dev = lib.device
-        L = len(det.levels)
-        J = self.T * L
-        self.J = J
-        want = detect.default_caps(det.nlat, det.nlon, det.add, J)
-        if caps:
-            for k, v in caps.items():
-                if k in want:  # (cap_c / cap_p / cap_e / cap_r size the slot's own buffers, below)
-                    want[k] = max(want[k], int(v))
-        self.ctx = detect.Context(det.nlat, det.nlon, det.add, want)
-        self.cap_c = int(max(64 * J, 1024))
-        self.cap_p = int(max(min(want["seg_cap"], 16384) * J, 1 << 16))
-        self.cap_e = int(max(48 * J, 1024))
-        self.cap_r = int(max(8192 * J, 1 << 16))
-        if caps:
-            self.cap_c = max(self.cap_c, int(caps.get("cap_c", 0)))
-            self.cap_p = max(self.cap_p, int(caps.get("cap_p", 0)))
-            self.cap_e = max(self.cap_e, int(caps.get("cap_e", 0)))
-            self.cap_r = max(self.cap_r, int(caps.get("cap_r", 0)))
+        J = self.T * len(det.levels)
+        ctx_caps = detect.default_caps(det.nlat, det.nlon, det.add, J)
+        caps = dict(ctx_caps, cap_c=max(64 * J, 1024), cap_p=1 << 16, cap_e=max(48 * J, 1024),
+                    cap_r=max(8192 * J, 1 << 16), cap_sr=max(16 * J, 1024), cap_sv=max(4096 * J, 1 << 16))
+        caps = {k: max(v, int((grown or {}).get(k, 0))) for k, v in caps.items()}
+        caps["cap_p"] = max(caps["cap_p"], min(caps["seg_cap"], 16384) * J)  # packed points follow the segment arena
+        self.ctx = detect.Context(det.nlat, det.nlon, det.add, {k: caps[k] for k in ctx_caps})
+        self.cap_c, self.cap_p, self.cap_e, self.cap_r = caps["cap_c"], caps["cap_p"], caps["cap_e"], caps["cap_r"]
+        # pieces of the events that straddle the last meridian (device clipper output, wbk_split_fetch)
+        self.cap_sr, self.cap_sv = caps["cap_sr"], caps["cap_sv"]
         shape = (self.T, det.nlat, det.nlon)
         i32, f64 = torch.int32, torch.float64
         self.sm = torch.empty(shape, dtype=f64, device=dev) if det.passes > 0 else None
-        self.sm_f32 = None
         self.sm_tmp = torch.empty(shape, dtype=f64, device=dev) if det.passes > _lib.SMOOTH_MAX_FUSED else None
-        self.raw_dev = None  # allocated on first host submit
-        self.inten_dev = [None, None]  # uploads of host intensity items (the field, or u and v), on first use
-        self.mflux = None  # momentum flux of (u, v) intensity items, on first use
-        self.flipped = None
         self.job_off = torch.empty(J + 1, dtype=i32, device=dev)
         self.pt_off = torch.empty(self.cap_c + 1, dtype=i32, device=dev)
         self.meta = torch.empty((self.cap_c, 4), dtype=i32, device=dev)
         self.pts = torch.empty(self.cap_p, dtype=i32, device=dev)
         self.work = torch.empty(2 * self.cap_p, dtype=f64, device=dev)
-        self.flags = None
-        self.ev_int = torch.empty((self.cap_e, _lib.EV_INTS), dtype=i32, device=dev)
-        self.ev_f64 = torch.empty((self.cap_e, _lib.EV_F64), dtype=f64, device=dev)
-        self.ev_job = torch.empty(self.cap_e, dtype=i32, device=dev)
-        self.ring_off = torch.empty(self.cap_e + 1, dtype=i32, device=dev)
-        self.ring_pts = torch.empty(self.cap_r, dtype=i32, device=dev)
-        self.summary = torch.zeros(16, dtype=i32, device=dev)
-        self.h_summary = _pinned(16, i32, lib)
-        # pieces of the events that straddle the last meridian (device clipper output, wbk_split_fetch)
-        self.cap_sr = int(max(16 * J, 1024))
-        self.cap_sv = int(max(4096 * J, 1 << 16))
-        if caps:
-            self.cap_sr = max(self.cap_sr, int(caps.get("cap_sr", 0)))
-            self.cap_sv = max(self.cap_sv, int(caps.get("cap_sv", 0)))
-        self.sp_ev = torch.zeros(self.cap_sr, dtype=i32, device=dev)
-        self.sp_off = torch.zeros(self.cap_sr + 1, dtype=i32, device=dev)
-        self.sp_xy = torch.zeros((self.cap_sv, 2), dtype=i32, device=dev)
-        self.sp_cnt = torch.zeros(4, dtype=i32, device=dev)
-        self.h_sp_ev = _pinned(self.cap_sr, i32, lib)
-        self.h_sp_off = _pinned(self.cap_sr + 1, i32, lib)
-        self.h_sp_xy = _pinned((self.cap_sv, 2), i32, lib)
-        self.h_sp_cnt = _pinned(4, i32, lib)
-        self.near = torch.zeros((_lib.NEAR_CAP, 4), dtype=i32, device=dev)
-        self.near_cnt = torch.zeros(1, dtype=i32, device=dev)
-        self.h_near = _pinned((_lib.NEAR_CAP, 4), i32, lib)
-        self.h_near_cnt = _pinned(1, i32, lib)
-        self.h_ev_int = _pinned((self.cap_e, _lib.EV_INTS), i32, lib)
-        self.h_ev_f64 = _pinned((self.cap_e, _lib.EV_F64), f64, lib)
-        self.h_ev_job = _pinned(self.cap_e, i32, lib)
-        self.h_ring_off = _pinned(self.cap_e + 1, i32, lib)
-        self.h_ring_pts = _pinned(self.cap_r, i32, lib)
+        # the device buffers that come back to the host, as (name, shape, dtype); each gets a pinned twin h_<name>
+        self.readback = [self._twin(*b) for b in (
+            ("summary", 16, i32), ("near", (_lib.NEAR_CAP, 4), i32), ("near_cnt", 1, i32),
+            ("ev_int", (self.cap_e, _lib.EV_INTS), i32), ("ev_f64", (self.cap_e, _lib.EV_F64), f64),
+            ("ev_job", self.cap_e, i32), ("ring_off", self.cap_e + 1, i32), ("ring_pts", self.cap_r, i32))]
+        self.readback_pieces = [self._twin(*b) for b in (  # only with want_pieces
+            ("sp_ev", self.cap_sr, i32), ("sp_off", self.cap_sr + 1, i32), ("sp_xy", (self.cap_sv, 2), i32),
+            ("sp_cnt", 4, i32))]
         self.stream = torch.cuda.Stream(device=dev) if lib.is_cuda else None
         self.done = torch.cuda.Event() if lib.is_cuda else None
-        self.pending = None   # (raw, ntime, flags_dev, flags_host, gmax)
+        self.pending = None   # _Pending of the batch in flight
         self.grow_seen = 0
-        self.packed = None    # bit-packed flag grids (device), allocated on first use
-        self.clim_group = None  # int32 [T] (device): groups of the batch's steps for FlagClimatology, on first use
-        self.graphs = {}      # buffers key -> (torch.cuda.CUDAGraph, pending record)
+        self.lazy = {}        # buffers allocated on first use (buffer())
+        self.graphs = {}      # buffers key -> (torch.cuda.CUDAGraph, _Pending, kernels in the graph)
         self.graph_seen = set()
+
+    def _twin(self, name, shape, dtype):
+        dev = torch.zeros(shape, dtype=dtype, device=self.det.lib.device)
+        host = _pinned(shape, dtype, self.det.lib)
+        setattr(self, name, dev)
+        setattr(self, "h_" + name, host)
+        return dev, host
+
+    def buffer(self, name, dtype, shape=None):
+        """The slot's buffer ``name`` (default shape: a batch), allocated on first use and again when the dtype
+        changes: the steady state allocates nothing, so a batch can be captured into a CUDA graph."""
+        b = self.lazy.get(name)
+        if b is None or b.dtype != dtype:
+            shape = (self.T, self.det.nlat, self.det.nlon) if shape is None else shape
+            b = self.lazy[name] = torch.empty(shape, dtype=dtype, device=self.det.lib.device)
+        return b
 
     def close(self):
         self.graphs.clear()
@@ -249,21 +246,14 @@ class Detector:
         if nvtx:
             nvtx.range_push("wbk.upload")
         if raw.device != lib.device:  # host input: H2D on this slot's stream
-            if slot.raw_dev is None or slot.raw_dev.dtype != raw.dtype:
-                slot.raw_dev = torch.empty((slot.T, self.nlat, self.nlon), dtype=raw.dtype, device=lib.device)
-            slot.raw_dev[:nt].copy_(raw, non_blocking=True)
-            raw = slot.raw_dev[:nt]
+            raw = slot.buffer("raw", raw.dtype)[:nt].copy_(raw, non_blocking=True)
         raw = raw.contiguous()
         raw_in = raw  # what the caller handed over (the regrow path re-submits exactly this)
         if isinstance(intensity, tuple):  # the field or (u, v) as stored: host items go to the slot's own buffers
             fields = []
             for k, f in enumerate(intensity):
                 if f.device != lib.device:
-                    if slot.inten_dev[k] is None or slot.inten_dev[k].dtype != f.dtype:
-                        slot.inten_dev[k] = torch.empty((slot.T, self.nlat, self.nlon), dtype=f.dtype,
-                                                        device=lib.device)
-                    slot.inten_dev[k][:nt].copy_(f, non_blocking=True)
-                    f = slot.inten_dev[k][:nt]
+                    f = slot.buffer(("intensity", k), f.dtype)[:nt].copy_(f, non_blocking=True)
                 fields.append(f.contiguous())
             intensity = tuple(fields)
         elif intensity is not None:
@@ -284,9 +274,7 @@ class Detector:
         elif self.passes > 0:
             f32 = raw.dtype == torch.float32
             if f32 and not spatial._numpy2():
-                if slot.sm_f32 is None:
-                    slot.sm_f32 = torch.empty((slot.T, self.nlat, self.nlon), dtype=torch.float32, device=lib.device)
-                sm, rmode = slot.sm_f32[:nt], _lib.ROUND_ALL
+                sm, rmode = slot.buffer("sm_f32", torch.float32)[:nt], _lib.ROUND_ALL
             else:
                 sm, rmode = slot.sm[:nt], (_lib.ROUND_FIRST if f32 else _lib.ROUND_NONE)
             if self.fuse and sm.dtype == torch.float64 and self.passes <= _lib.SMOOTH_MAX_FUSED and self.nlat >= 4:
@@ -299,12 +287,10 @@ class Detector:
                          rmode, opts, st)
         else:
             if opts is not None:  # no smoothing: orientation / decode only
-                want = torch.float64 if raw.dtype == torch.int16 else raw.dtype
-                if slot.flipped is None or slot.flipped.dtype != want:
-                    slot.flipped = torch.empty((slot.T, self.nlat, self.nlon), dtype=want, device=lib.device)
-                lib.call("wbk_orient", _lib.ptr(raw), _lib.dtype_code(raw.dtype), _lib.ptr(slot.flipped), nt,
-                         self.nlat, self.nlon, opts, st)
-                raw = slot.flipped[:nt]
+                flipped = slot.buffer("flipped", torch.float64 if raw.dtype == torch.int16 else raw.dtype)[:nt]
+                lib.call("wbk_orient", _lib.ptr(raw), _lib.dtype_code(raw.dtype), _lib.ptr(flipped), nt, self.nlat,
+                         self.nlon, opts, st)
+                raw = flipped
             sm = raw
         if not fused:
             lib.call("wbk_contours", h, _lib.ptr(sm), _lib.dtype_code(sm.dtype), nt, lv, L, st)
@@ -327,11 +313,10 @@ class Detector:
         if self.want_flags:
             if flags_out is not None:
                 flags = flags_out
+            elif nt == slot.T:
+                flags = slot.buffer("flags", torch.int8, (3, slot.T, self.nlat, self.nlon))
             else:
-                if slot.flags is None:
-                    slot.flags = torch.empty((3, slot.T, self.nlat, self.nlon), dtype=torch.int8, device=lib.device)
-                flags = slot.flags if nt == slot.T else torch.empty((3, nt, self.nlat, self.nlon), dtype=torch.int8,
-                                                                    device=lib.device)
+                flags = torch.empty((3, nt, self.nlat, self.nlon), dtype=torch.int8, device=lib.device)
         # the rasteriser reads the intensity's member cells in their stored dtype and orientation
         inten, iflip = intensity, (0, 0)
         if isinstance(intensity, tuple):
@@ -340,9 +325,7 @@ class Detector:
                 # zonal means summed in the stored memory order (what numpy does on the user's array); longitude is
                 # the contiguous axis of a batch
                 u, v = intensity
-                if slot.mflux is None or slot.mflux.dtype != u.dtype:
-                    slot.mflux = torch.empty((slot.T, self.nlat, self.nlon), dtype=u.dtype, device=lib.device)
-                inten = slot.mflux[:nt]
+                inten = slot.buffer("mflux", u.dtype)[:nt]
                 lib.call("wbk_mflux", _lib.ptr(u), _lib.ptr(v), _lib.ptr(inten), _lib.dtype_code(u.dtype), nt,
                          self.nlat, self.nlon, 0, st)
         lib.call("wbk_events_raster", h, _lib.ptr(slot.job_off), _lib.ptr(slot.pt_off), _lib.ptr(slot.pts),
@@ -352,42 +335,30 @@ class Detector:
         lib.call("wbk_batch_fetch", h, _lib.ptr(slot.pt_off), _lib.ptr(slot.pts), _lib.ptr(slot.ev_int),
                  _lib.ptr(slot.ev_f64), _lib.ptr(slot.ev_job), _lib.ptr(slot.ring_off), _lib.ptr(slot.ring_pts),
                  slot.cap_e, slot.cap_r, _lib.ptr(slot.summary), st)
-        if flags is not None and self.want_pieces:
+        pieces = flags is not None and self.want_pieces
+        if pieces:
             lib.call("wbk_split_fetch", h, _lib.ptr(slot.sp_ev), _lib.ptr(slot.sp_off), _lib.ptr(slot.sp_xy), slot.cap_sr,
                      slot.cap_sv, _lib.ptr(slot.sp_cnt), st)
-            slot.h_sp_cnt.copy_(slot.sp_cnt, non_blocking=True)
-            slot.h_sp_ev.copy_(slot.sp_ev, non_blocking=True)
-            slot.h_sp_off.copy_(slot.sp_off, non_blocking=True)
-            slot.h_sp_xy.copy_(slot.sp_xy, non_blocking=True)
         if nvtx:
             nvtx.range_pop()
             nvtx.range_push("wbk.download")
         # asynchronous read-back of everything the host needs (tables are small; flags only on request)
-        slot.h_summary.copy_(slot.summary, non_blocking=True)
-        slot.h_near_cnt.copy_(slot.near_cnt, non_blocking=True)
-        slot.h_near.copy_(slot.near, non_blocking=True)
-        slot.h_ev_int.copy_(slot.ev_int, non_blocking=True)
-        slot.h_ev_f64.copy_(slot.ev_f64, non_blocking=True)
-        slot.h_ev_job.copy_(slot.ev_job, non_blocking=True)
-        slot.h_ring_off.copy_(slot.ring_off, non_blocking=True)
-        slot.h_ring_pts.copy_(slot.ring_pts, non_blocking=True)
+        for dev_buf, host_buf in slot.readback + (slot.readback_pieces if pieces else []):
+            host_buf.copy_(dev_buf, non_blocking=True)
         if flags_host is not None and flags is not None:
             flags_host[:, :nt].copy_(flags[:, :nt] if flags.shape[1] != nt else flags, non_blocking=True)
         if packed_host is not None and flags is not None:
             # one bit per cell on the wire (wbk_pack_flags); unpack_flags() restores the int8 grids on the host
             ncells = 3 * nt * self.nlat * self.nlon
-            if slot.packed is None:
-                slot.packed = torch.empty(packed_nbytes(3 * slot.T * self.nlat * self.nlon), dtype=torch.uint8,
-                                          device=lib.device)
+            packed = slot.buffer("packed", torch.uint8, packed_nbytes(3 * slot.T * self.nlat * self.nlon))
             fl = flags if flags.shape[1] == nt and flags.is_contiguous() else flags[:, :nt].contiguous()
-            lib.call("wbk_pack_flags", _lib.ptr(fl), _lib.ptr(slot.packed), ncells, st)
+            lib.call("wbk_pack_flags", _lib.ptr(fl), _lib.ptr(packed), ncells, st)
             nb = packed_nbytes(ncells)
-            packed_host[:nb].copy_(slot.packed[:nb], non_blocking=True)
+            packed_host[:nb].copy_(packed[:nb], non_blocking=True)
         if nvtx:
             nvtx.range_pop()
-        # (inten keeps the buffer a captured graph writes the momentum flux to alive)
-        return dict(raw=raw_in, nt=nt, flags=flags, flags_host=flags_host, gmax=gmax_nx, smoothed=smoothed, sm=sm,
-                    intensity=intensity, inten=inten, packed_host=packed_host)
+        return _Pending(raw=raw_in, nt=nt, flags=flags, flags_host=flags_host, packed_host=packed_host, gmax=gmax_nx,
+                        smoothed=smoothed, intensity=intensity, graph_bufs=(sm, inten))
 
     def submit(self, slot, raw, flags_out=None, flags_host=None, gmax_nx=None, smoothed=None, stream=None,
                intensity=None, packed_host=None):
@@ -410,7 +381,7 @@ class Detector:
         use_stream = stream if stream is not None else slot.stream
         args = (slot, raw, flags_out, flags_host, gmax_nx, smoothed, intensity, packed_host)
         if use_stream is None:  # emulator
-            slot.pending = dict(self._enqueue(*args), stream=None)
+            slot.pending = self._enqueue(*args)
             return slot
         graphable = self.graphs and smoothed is None and not isinstance(intensity, torch.Tensor)
         key = None
@@ -444,7 +415,7 @@ class Detector:
                 slot.pending = self._enqueue(*args)
                 if key is not None:
                     slot.graph_seen.add(key)
-            slot.pending = dict(slot.pending, stream=use_stream)  # (a replayed graph's record is shared: copy it)
+            slot.pending = replace(slot.pending, stream=use_stream)  # (a replayed graph's record is shared: copy it)
             slot.done.record()
         return slot
 
@@ -457,20 +428,34 @@ class Detector:
         pend = slot.pending
         if pend is None:
             raise RuntimeError("nothing was submitted on this slot")
-        if slot.done is not None:
-            slot.done.synchronize()
-        s = slot.h_summary.numpy()
+        while True:
+            if slot.done is not None:
+                slot.done.synchronize()
+            s = slot.h_summary.numpy()
+            status = int(s[5])
+            if status & _lib.ST_SPLIT_CHAINS:
+                raise _lib.WbkError(_lib.ERR_INVALID, "an event crosses the last meridian too often for the device "
+                                                      "clipper; its cells would be missing from the flag grids")
+            grow = self._outgrown(slot, pend, s)
+            if not grow:
+                break
+            self._grow = {**self._grow, **grow}
+            self._grow_version += 1
+            if max(self._grow.values()) > (1 << 28):
+                raise _lib.WbkError(_lib.ERR_CAPACITY, "arenas still overflow after repeated regrowth (status {})"
+                                    .format(status))
+            key = next(k for k, v in self._slots.items() if v is slot)
+            if self.lib.is_cuda:
+                torch.cuda.synchronize()
+            slot.close()
+            slot = self._slots[key] = _Slot(self, slot.T, self._grow)
+            slot.grow_seen = self._grow_version
+            self.submit(slot, pend.raw, flags_out=pend.flags, flags_host=pend.flags_host, gmax_nx=pend.gmax,
+                        smoothed=pend.smoothed, intensity=pend.intensity, packed_host=pend.packed_host)
+        pend, slot.pending = slot.pending, None  # (after a re-run: the new slot's record, with its stream)
         C, P, ns, no, nc, status, max_nx, n_split = (int(v) for v in s[:8])
         work = dict(segments=int(s[8]), pairs=int(s[9]), tiles=int(s[11]))
-        bad = status & (_lib.ST_SEG_OVERFLOW | _lib.ST_CONTOUR_OVERFLOW | _lib.ST_PAIR_OVERFLOW | _lib.ST_EVENT_OVERFLOW
-                        | _lib.ST_SEL_OVERFLOW | _lib.ST_PACK_OVERFLOW | _lib.ST_FETCH_OVERFLOW)
-        if status & _lib.ST_SPLIT_CHAINS:
-            raise _lib.WbkError(_lib.ERR_INVALID, "an event crosses the last meridian too often for the device clipper; "
-                                                  "its cells would be missing from the flag grids")
-        if bad:
-            return self._regrow_and_rerun(slot, status, climatology, trackers)
-        slot.pending = None
-        nt = pend["nt"]
+        nt = pend.nt
         L = len(self.levels)
         counts = (ns, no, nc)
         tables, o = {}, 0
@@ -494,18 +479,11 @@ class Detector:
             njobs=nt * L, nlevels=L, nlat=self.nlat, nlon=self.nlon, add=self.add, levels=self.levels,
             job_off=slot.job_off[:nt * L + 1], pt_off=slot.pt_off[:C + 1], meta=slot.meta[:C], pts=slot.pts[:P],
             status=np.full(nt * L, status, dtype=np.int32), max_nx=max_nx, h_ncontours=None, h_npoints=None)
-        flags = pend["flags_host"] if pend["flags_host"] is not None else pend["flags"]
-        packed = pend.get("packed_host")
+        flags = pend.flags_host if pend.flags_host is not None else pend.flags
         n_sp = int(sum(int((t.split == 1).sum()) for t in tables.values()))
         pieces = None
-        if self.want_pieces and pend["flags"] is not None:
+        if self.want_pieces and pend.flags is not None:
             npc, nvx, clip_over = (int(v) for v in slot.h_sp_cnt.numpy()[:3])
-            if npc > slot.cap_sr or nvx > slot.cap_sv:
-                grow = dict(self._grow)
-                grow["cap_sr"], grow["cap_sv"] = max(2 * slot.cap_sr, 2 * npc), max(2 * slot.cap_sv, 2 * nvx)
-                self._grow = grow
-                slot.pending = pend  # the re-run submits the batch again from its pending record
-                return self._regrow_and_rerun(slot, 0, climatology, trackers)
             off = slot.h_sp_off.numpy()[:npc + 1].astype(np.int64)
             pieces = dict(ev=slot.h_sp_ev.numpy()[:npc].copy(), off=off, xy=slot.h_sp_xy.numpy()[:nvx].copy(),
                           overflow=bool(clip_over))
@@ -517,46 +495,27 @@ class Detector:
         for tr in trackers or ():
             tr._add(slot, pend, tables, counts)
         return BatchResult(ntime=nt, contours=cs, tables=tables, flags=flags,
-                           gmax_nx=max_nx if pend["gmax"] is None else int(pend["gmax"]), n_split=n_sp,
-                           near=near.astype(np.int32), near_total=n_near, flags_packed=packed, work=work, pieces=pieces,
-                           counts=(ns, no, nc))
+                           gmax_nx=max_nx if pend.gmax is None else int(pend.gmax), n_split=n_sp,
+                           near=near.astype(np.int32), near_total=n_near, flags_packed=pend.packed_host, work=work,
+                           pieces=pieces, counts=(ns, no, nc))
 
-    def _regrow_and_rerun(self, slot, status, climatology=None, trackers=()):
-        pend = slot.pending
-        caps = dict(slot.ctx.caps)
-        grow = dict(self._grow)
-        if status & _lib.ST_SEG_OVERFLOW:
-            grow["seg_cap"] = caps["seg_cap"] * 2
-        if status & _lib.ST_CONTOUR_OVERFLOW:
-            grow["contour_cap"] = caps["contour_cap"] * 2
-        if status & _lib.ST_PAIR_OVERFLOW:
-            grow["pair_cap"] = caps["pair_cap"] * 4
-        if status & _lib.ST_EVENT_OVERFLOW:
-            grow["event_cap"] = caps["event_cap"] * 4
-        if status & _lib.ST_SEL_OVERFLOW:
-            grow["sel_cap"] = caps["sel_cap"] * 4
-        # the summary record holds the true totals of the batch: size the buffers for them (with headroom) in one go
-        C, P, ns, no, nc = (int(v) for v in slot.h_summary.numpy()[:5])
+    def _outgrown(self, slot, pend, summary):
+        """The capacities the slot's batch outgrew, grown (empty when the batch fit).  ``summary``: the batch's summary
+        record, whose true totals size the slot's own arenas (with headroom) in one go.  The device clipper's piece
+        counts are read only when no arena overflowed: only then do they count the whole batch."""
+        C, P, ns, no, nc, status = (int(v) for v in summary[:6])
+        grow = detect.grow_caps(slot.ctx.caps, status)
         if status & _lib.ST_PACK_OVERFLOW:
             grow["cap_c"] = max(slot.cap_c * 2, int(1.3 * C))
             grow["cap_p"] = max(slot.cap_p * 2, int(1.3 * P))
         if status & _lib.ST_FETCH_OVERFLOW:
             grow["cap_e"] = max(slot.cap_e * 2, int(1.3 * (ns + no + nc)))
             grow["cap_r"] = slot.cap_r * 2
-        self._grow = grow
-        self._grow_version += 1
-        if len(grow) and max(grow.values()) > (1 << 28):
-            raise _lib.WbkError(_lib.ERR_CAPACITY, "arenas still overflow after repeated regrowth (status {})".format(status))
-        key = next(k for k, v in self._slots.items() if v is slot)
-        if self.lib.is_cuda:
-            torch.cuda.synchronize()
-        slot.close()
-        new = _Slot(self, slot.T, grow)
-        new.grow_seen = self._grow_version
-        self._slots[key] = new
-        self.submit(new, pend["raw"], flags_out=pend["flags"], flags_host=pend["flags_host"], gmax_nx=pend["gmax"],
-                    smoothed=pend["smoothed"], intensity=pend["intensity"], packed_host=pend.get("packed_host"))
-        return self.collect(new, climatology, trackers)
+        if not grow and self.want_pieces and pend.flags is not None:
+            npc, nvx = (int(v) for v in slot.h_sp_cnt.numpy()[:2])
+            if npc > slot.cap_sr or nvx > slot.cap_sv:
+                grow = dict(cap_sr=max(2 * slot.cap_sr, 2 * npc), cap_sv=max(2 * slot.cap_sv, 2 * nvx))
+        return grow
 
     # ------------------------------------------------------------------ convenience
     def run_batch(self, raw, gmax_nx=None, smoothed=None, intensity=None):
@@ -742,7 +701,7 @@ class FlagClimatology:
 
     def _add(self, slot, pend):
         """Add the flag grids of one collected batch, on the stream the batch ran on."""
-        nt, flags = int(pend["nt"]), pend["flags"]
+        nt, flags = pend.nt, pend.flags
         if self.cursor + nt > len(self.groups):
             raise ValueError("the batch covers time steps {}..{} of the record, the group array has {}".format(
                 self.cursor, self.cursor + nt - 1, len(self.groups)))
@@ -751,14 +710,12 @@ class FlagClimatology:
         if (self._steps + add > 0xFFFFFFFF).any():
             raise ValueError("a group would count more than 2**32 - 1 time steps")
         lib = self.lib
-        st = pend.get("stream")
+        st = pend.stream
         with torch.cuda.stream(st) if st is not None else _null():
-            if slot.clim_group is None:
-                slot.clim_group = torch.empty(slot.T, dtype=torch.int32, device=lib.device)
-            slot.clim_group[:nt].copy_(torch.from_numpy(g), non_blocking=True)
+            group = slot.buffer("clim_group", torch.int32, slot.T)[:nt].copy_(torch.from_numpy(g), non_blocking=True)
             # the grids as the rasteriser wrote them: kind stride nt * nlat * nlon (also for a partial last batch)
-            lib.call("wbk_flag_counts", _lib.ptr(flags), 3, nt, self.nlat * self.nlon, _lib.ptr(slot.clim_group),
-                     self.ngroups, _lib.ptr(self._counts), lib.stream())
+            lib.call("wbk_flag_counts", _lib.ptr(flags), 3, nt, self.nlat * self.nlon, _lib.ptr(group), self.ngroups,
+                     _lib.ptr(self._counts), lib.stream())
         self._steps += add
         self.cursor += nt
 
@@ -1004,9 +961,9 @@ class EventTracker:
         import time
 
         tick = time.perf_counter()
-        nt = int(pend["nt"])
+        nt = pend.nt
         self._check_steps(self.cursor, nt)
-        st = pend.get("stream")
+        st = pend.stream
         with self._on_stream():
             if st is not None:
                 self._stream.wait_event(slot.done)  # the batch's buffers (final: collect has waited for this event)
