@@ -361,7 +361,12 @@ int wbk_track_overlap_exact(const int* d_edges, const int* d_vsign, const int* d
 /* events.py:205-214 for overlap > 0: float64 areas of event pairs.
  * Polygons are given as rings of double (x, y) vertices: polygon p = rings [d_poly_off[p], d_poly_off[p+1]),
  * ring r = vertices [d_ring_off[r], d_ring_off[r+1]) of d_xy (open rings).  For pair k = (d_pairs[2k],
- * d_pairs[2k+1]) writes d_out[3k..3k+2] = area(A), area(B), area(A n B). */
+ * d_pairs[2k+1]) writes d_out[3k..3k+2] = area(A), area(B), area(A n B).
+ * Every ring is the region it encloses under non-zero winding, whatever its orientation: area(P) is the sum of
+ * |area(ring)| over the rings of P, and a ring of zero area adds nothing.  The parts of one polygon must not overlap
+ * each other (such a MultiPolygon is invalid; GEOS does not define its area either).  The arithmetic runs on
+ * coordinates relative to the first vertex of A, so lattice pairs give the same areas bit for bit under any integer
+ * translation.  d_vsign of wbk_track_overlap_exact follows the same orientation rule. */
 int wbk_track_overlap(const double* d_xy, const int* d_ring_off, const int* d_poly_off, const int* d_pairs, int npairs,
                       double* d_out, void* stream);
 

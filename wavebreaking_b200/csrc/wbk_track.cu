@@ -1,14 +1,18 @@
 // Event tracking: exact polygon-overlap areas for the by_overlap method.
 // Reference: wavebreaking/processing/events.py:205-214 (geopandas intersection(...).area of event pairs).
 //
-// area(A n B) is evaluated without clipping A against B: every polygon is the signed sum of the triangles
-// (O, v_i, v_i+1) spanned by its edges and a common origin O, so
-//     area(A n B) = sum_a sum_b sign_a sign_b area(T_a n T_b)
-// and each triangle-triangle intersection is a tiny convex clip.  One CTA per event pair, threads over the
-// (edge of A) x (edge of B) products, fp64, deterministic block reduction.
+// area(A n B) is evaluated without clipping A against B: every ring is the signed sum of the triangles
+// (O, v_i, v_i+1) spanned by its edges and a common origin O, so with s_r the orientation sign of ring r
+//     area(A n B) = sum_ra sum_rb s_ra s_rb sum_(T_a in ra, T_b in rb) sign_a sign_b area(T_a n T_b)
+// and each triangle-triangle intersection is a tiny convex clip.  Each ring counts as the region it encloses whatever
+// its orientation (s_r: sign of its own doubled area; a ring of zero area adds nothing), so the parts of a
+// MultiPolygon may wind either way.  O is the first vertex of A and is subtracted from every vertex as it is loaded:
+// all arithmetic runs on coordinates relative to O, so lattice pairs give the same areas bit for bit wherever they
+// lie.  One CTA per event pair, threads over the (edge of A) x (edge of B) products, fp64, deterministic reductions.
 #include "wbk_common.cuh"
 
 #define TRK_THREADS 256
+#define TRK_RINGS 64  // rings per chunk whose doubled areas are held in shared memory
 
 struct TrkPoly {
   const double* xy;      // all vertices (x, y pairs)
@@ -16,10 +20,10 @@ struct TrkPoly {
   const int* poly_off;   // polygon p = rings [poly_off[p], poly_off[p+1])
 };
 
-// signed doubled area and CCW-ordered copy of triangle (o, a, b)
-__device__ __forceinline__ double tri_ccw(double ox, double oy, double ax, double ay, double bx, double by, double* t) {
-  const double c = (ax - ox) * (by - oy) - (ay - oy) * (bx - ox);
-  t[0] = ox; t[1] = oy;
+// signed doubled area and CCW-ordered copy of triangle (0, a, b)
+__device__ __forceinline__ double tri_ccw(double ax, double ay, double bx, double by, double* t) {
+  const double c = ax * by - ay * bx;
+  t[0] = 0.0; t[1] = 0.0;
   if (c >= 0) { t[2] = ax; t[3] = ay; t[4] = bx; t[5] = by; }
   else        { t[2] = bx; t[3] = by; t[4] = ax; t[5] = ay; }
   return c;
@@ -61,71 +65,103 @@ __device__ inline double tri_tri_area(const double* p, const double* q) {
   return a2 > 0 ? 0.5 * a2 : 0.0;
 }
 
-// edge k (0-based over all rings of polygon p) -> its two end points
-__device__ __forceinline__ void trk_edge(const TrkPoly& P, int p, int k, double& ax, double& ay, double& bx, double& by) {
-  int r = P.poly_off[p];
-  while (k >= P.ring_off[r + 1] - P.ring_off[r]) {
-    k -= P.ring_off[r + 1] - P.ring_off[r];
-    ++r;
-  }
-  const int s = P.ring_off[r], n = P.ring_off[r + 1] - s;
-  const int k2 = k + 1 == n ? 0 : k + 1;
-  ax = P.xy[2 * (s + k)]; ay = P.xy[2 * (s + k) + 1];
-  bx = P.xy[2 * (s + k2)]; by = P.xy[2 * (s + k2) + 1];
+// the edge that starts at vertex v of the rings [r, ...) (v >= ring_off[r]): its end points relative to (ox, oy);
+// returns the index of its ring relative to r
+__device__ __forceinline__ int trk_edge(const TrkPoly& P, int r, int v, double ox, double oy, double& ax, double& ay,
+                                        double& bx, double& by) {
+  int k = 0;
+  while (v >= P.ring_off[r + k + 1]) ++k;
+  const int v2 = v + 1 == P.ring_off[r + k + 1] ? P.ring_off[r + k] : v + 1;
+  ax = P.xy[2 * v] - ox; ay = P.xy[2 * v + 1] - oy;
+  bx = P.xy[2 * v2] - ox; by = P.xy[2 * v2 + 1] - oy;
+  return k;
 }
 
-__device__ __forceinline__ int trk_nedges(const TrkPoly& P, int p) {
-  return P.ring_off[P.poly_off[p + 1]] - P.ring_off[P.poly_off[p]];
+// a2[r - r0] = doubled signed area of ring r (fan about (ox, oy)) for the rings [r0, r1), r1 - r0 <= TRK_RINGS; one
+// warp per ring, fixed summation order.  All threads of the block call; a2 is ready after the barrier.
+__device__ __forceinline__ void trk_ring_areas(const TrkPoly& P, int r0, int r1, double ox, double oy, double* a2) {
+  const int lane = wbk_lane();
+  for (int r = r0 + wbk_warp(); r < r1; r += TRK_THREADS / 32) {
+    const int s = P.ring_off[r], e = P.ring_off[r + 1];
+    double sum = 0.0;
+    for (int v = s + lane; v < e; v += 32) {
+      double ax, ay, bx, by;
+      trk_edge(P, r, v, ox, oy, ax, ay, bx, by);
+      sum += ax * by - ay * bx;
+    }
+    sum = wbk_warp_sum_f64(sum);
+    if (lane == 0) a2[r - r0] = sum;
+  }
+  __syncthreads();
+}
+
+__device__ __forceinline__ double trk_sign(double a2) { return a2 > 0 ? 1.0 : (a2 < 0 ? -1.0 : 0.0); }
+
+// area of polygon p = sum over its rings of |area(ring)|; the result is valid in thread 0
+__device__ inline double trk_area(const TrkPoly& P, int p, double ox, double oy, double* a2) {
+  double area = 0.0;
+  for (int r0 = P.poly_off[p]; r0 < P.poly_off[p + 1]; r0 += TRK_RINGS) {
+    const int r1 = min(r0 + TRK_RINGS, P.poly_off[p + 1]);
+    trk_ring_areas(P, r0, r1, ox, oy, a2);
+    if (threadIdx.x == 0)
+      for (int r = r0; r < r1; ++r) area += fabs(0.5 * a2[r - r0]);
+    __syncthreads();
+  }
+  return area;
 }
 
 // out[3 * pair + {0,1,2}] = area(A), area(B), area(A n B)
 __global__ void __launch_bounds__(TRK_THREADS) track_overlap_kernel(TrkPoly P, const int* __restrict__ pairs, int npairs,
                                                                     double* __restrict__ out) {
   __shared__ double red[40];
+  __shared__ double s_a2[2][TRK_RINGS];  // doubled ring areas of the current chunks of A and of B
   for (int w = blockIdx.x; w < npairs; w += gridDim.x) {
     const int pa = pairs[2 * w], pb = pairs[2 * w + 1];
-    const int na = trk_nedges(P, pa), nb = trk_nedges(P, pb);
+    const int ra0 = P.poly_off[pa], ra1 = P.poly_off[pa + 1], rb0 = P.poly_off[pb], rb1 = P.poly_off[pb + 1];
     // common origin: first vertex of A (keeps the triangle areas small)
-    const int sa = P.ring_off[P.poly_off[pa]];
-    const double ox = na > 0 ? P.xy[2 * sa] : 0.0, oy = na > 0 ? P.xy[2 * sa + 1] : 0.0;
-    double area_a = 0, area_b = 0, inter = 0;
-    for (int k = threadIdx.x; k < na; k += TRK_THREADS) {
-      double ax, ay, bx, by;
-      trk_edge(P, pa, k, ax, ay, bx, by);
-      area_a += (ax - ox) * (by - oy) - (ay - oy) * (bx - ox);
+    const int sa = P.ring_off[ra0];
+    const bool has_a = P.ring_off[ra1] > sa;
+    const double ox = has_a ? P.xy[2 * sa] : 0.0, oy = has_a ? P.xy[2 * sa + 1] : 0.0;
+    const double area_a = trk_area(P, pa, ox, oy, s_a2[0]);
+    const double area_b = trk_area(P, pb, ox, oy, s_a2[0]);
+    double inter = 0;
+    // chunks of rings of A x chunks of rings of B, threads over the (edge of A) x (edge of B) products of a chunk pair
+    for (int ca = ra0; ca < ra1; ca += TRK_RINGS) {
+      const int ca1 = min(ca + TRK_RINGS, ra1);
+      trk_ring_areas(P, ca, ca1, ox, oy, s_a2[0]);
+      for (int cb = rb0; cb < rb1; cb += TRK_RINGS) {
+        const int cb1 = min(cb + TRK_RINGS, rb1);
+        trk_ring_areas(P, cb, cb1, ox, oy, s_a2[1]);
+        const int va = P.ring_off[ca], vb = P.ring_off[cb];
+        const int na = P.ring_off[ca1] - va, nb = P.ring_off[cb1] - vb;
+        const long long nprod = (long long)na * nb;
+        for (long long q = threadIdx.x; q < nprod; q += TRK_THREADS) {
+          const int ka = (int)(q / nb), kb = (int)(q - (long long)ka * nb);
+          double a0x, a0y, a1x, a1y, b0x, b0y, b1x, b1y, ta[6], tb[6];
+          const int ia = trk_edge(P, ca, va + ka, ox, oy, a0x, a0y, a1x, a1y);
+          const int ib = trk_edge(P, cb, vb + kb, ox, oy, b0x, b0y, b1x, b1y);
+          const double sr = trk_sign(s_a2[0][ia]) * trk_sign(s_a2[1][ib]);
+          if (sr == 0.0) continue;
+          const double cta = tri_ccw(a0x, a0y, a1x, a1y, ta);
+          const double ctb = tri_ccw(b0x, b0y, b1x, b1y, tb);
+          if (cta == 0.0 || ctb == 0.0) continue;
+          // quick reject on bounding boxes
+          const double axmin = fmin(0.0, fmin(a0x, a1x)), axmax = fmax(0.0, fmax(a0x, a1x));
+          const double bxmin = fmin(0.0, fmin(b0x, b1x)), bxmax = fmax(0.0, fmax(b0x, b1x));
+          const double aymin = fmin(0.0, fmin(a0y, a1y)), aymax = fmax(0.0, fmax(a0y, a1y));
+          const double bymin = fmin(0.0, fmin(b0y, b1y)), bymax = fmax(0.0, fmax(b0y, b1y));
+          if (axmax <= bxmin || bxmax <= axmin || aymax <= bymin || bymax <= aymin) continue;
+          const double s = ((cta > 0) == (ctb > 0)) ? sr : -sr;
+          inter += s * tri_tri_area(ta, tb);
+        }
+        __syncthreads();  // s_a2 is rewritten by the next chunk
+      }
     }
-    for (int k = threadIdx.x; k < nb; k += TRK_THREADS) {
-      double ax, ay, bx, by;
-      trk_edge(P, pb, k, ax, ay, bx, by);
-      area_b += (ax - ox) * (by - oy) - (ay - oy) * (bx - ox);
-    }
-    const long long nprod = (long long)na * nb;
-    for (long long q = threadIdx.x; q < nprod; q += TRK_THREADS) {
-      const int ka = (int)(q / nb), kb = (int)(q - (long long)ka * nb);
-      double a0x, a0y, a1x, a1y, b0x, b0y, b1x, b1y, ta[6], tb[6];
-      trk_edge(P, pa, ka, a0x, a0y, a1x, a1y);
-      trk_edge(P, pb, kb, b0x, b0y, b1x, b1y);
-      const double ca = tri_ccw(ox, oy, a0x, a0y, a1x, a1y, ta);
-      const double cb = tri_ccw(ox, oy, b0x, b0y, b1x, b1y, tb);
-      if (ca == 0.0 || cb == 0.0) continue;
-      // quick reject on bounding boxes
-      const double axmin = fmin(ox, fmin(a0x, a1x)), axmax = fmax(ox, fmax(a0x, a1x));
-      const double bxmin = fmin(ox, fmin(b0x, b1x)), bxmax = fmax(ox, fmax(b0x, b1x));
-      const double aymin = fmin(oy, fmin(a0y, a1y)), aymax = fmax(oy, fmax(a0y, a1y));
-      const double bymin = fmin(oy, fmin(b0y, b1y)), bymax = fmax(oy, fmax(b0y, b1y));
-      if (axmax <= bxmin || bxmax <= axmin || aymax <= bymin || bymax <= aymin) continue;
-      const double s = ((ca > 0) == (cb > 0)) ? 1.0 : -1.0;
-      inter += s * tri_tri_area(ta, tb);
-    }
-    area_a = wbk_block_sum_f64(area_a, red);
-    area_b = wbk_block_sum_f64(area_b, red);
     inter = wbk_block_sum_f64(inter, red);
     if (threadIdx.x == 0) {
-      // orientation of the rings does not matter: |area|, and the product of winding signs for the overlap
-      const double sgn = ((area_a > 0) == (area_b > 0)) ? 1.0 : -1.0;
-      out[3 * w + 0] = fabs(0.5 * area_a);
-      out[3 * w + 1] = fabs(0.5 * area_b);
-      out[3 * w + 2] = sgn * inter;
+      out[3 * w + 0] = area_a;
+      out[3 * w + 1] = area_b;
+      out[3 * w + 2] = inter;
     }
     __syncthreads();
   }
@@ -215,6 +251,8 @@ extern "C" int wbk_track_candidates(const int* d_lo, const int* d_hi, const int*
 //      squared edge length): strictly inside => overlap; on the other boundary (collinear pieces) => overlap iff
 //      both interiors lie on the same side of the shared piece (ring orientation signs).  Rings without a touched
 //      edge are covered by rule 2.
+// A ring of zero area (vsign 0: the two-point sliver pieces of the meridian split) bounds no region under non-zero
+// winding: its edges take part in no rule, and its vertices are not tested by rule 2.
 // Polygon p = vertices [poly_voff[p], poly_voff[p+1]) of the edge table (x0, y0, x1, y1 per vertex: the edge from
 // that vertex to the next one of its ring); vsign = orientation of the vertex's ring (+1 counter-clockwise).
 // result: 0 / 1, | 2 when rule 3 decided.
@@ -253,7 +291,7 @@ __global__ void __launch_bounds__(TRX_THREADS) track_exact_kernel(const int4* __
     // ---- rule 1: all edge pairs (thread: one edge of A against every edge of B, uniform broadcast reads)
     for (int at = 0; at < nA; at += TRX_THREADS) {
       const int ia = at + tid;
-      if (ia < nA) {
+      if (ia < nA && vsign[a0 + ia] != 0) {
         const int4 e = edges[a0 + ia];
         const int exmin = min(e.x, e.z), exmax = max(e.x, e.z), eymin = min(e.y, e.w), eymax = max(e.y, e.w);
         bool proper = false, touched = false;
@@ -264,17 +302,17 @@ __global__ void __launch_bounds__(TRX_THREADS) track_exact_kernel(const int4* __
           const long long d2 = trx_cross(f.z - f.x, f.w - f.y, e.z - f.x, e.w - f.y);
           const long long d3 = trx_cross(e.z - e.x, e.w - e.y, f.x - e.x, f.y - e.y);
           const long long d4 = trx_cross(e.z - e.x, e.w - e.y, f.z - e.x, f.w - e.y);
+          const bool meet = !((d1 > 0 && d2 > 0) || (d1 < 0 && d2 < 0) || (d3 > 0 && d4 > 0) || (d3 < 0 && d4 < 0));
+          if (!meet || vsign[b0 + ib] == 0) continue;  // (the edge of a ring of zero area bounds nothing)
           if (((d1 > 0 && d2 < 0) || (d1 < 0 && d2 > 0)) && ((d3 > 0 && d4 < 0) || (d3 < 0 && d4 > 0))) {
             proper = true;
             break;
           }
-          const bool meet = !((d1 > 0 && d2 > 0) || (d1 < 0 && d2 < 0) || (d3 > 0 && d4 > 0) || (d3 < 0 && d4 < 0));
-          if (meet) {  // closed segments share a point (collinear ones: their boxes intersect, checked above)
-            touched = true;
-            const int k = atomicAdd(&s_ntouch[1], 1);
-            if (k < TRX_MAXTOUCH) s_touch[1][k] = b0 + ib;
-            else s_flag[2] = 1;
-          }
+          // the closed segments share a point (collinear ones: their boxes intersect, checked above)
+          touched = true;
+          const int k = atomicAdd(&s_ntouch[1], 1);
+          if (k < TRX_MAXTOUCH) s_touch[1][k] = b0 + ib;
+          else s_flag[2] = 1;
         }
         if (proper) s_flag[0] = 1;
         if (touched) {
@@ -296,7 +334,7 @@ __global__ void __launch_bounds__(TRX_THREADS) track_exact_kernel(const int4* __
         const int pr0 = side == 0 ? poly_off[pa] : poly_off[pb], pr1 = side == 0 ? poly_off[pa + 1] : poly_off[pb + 1];
         const int o0 = side == 0 ? b0 : a0, o1 = side == 0 ? b1 : a1;
         for (int r = pr0; r < pr1 && !res; ++r) {
-          if (ring_off[r + 1] == ring_off[r]) continue;
+          if (ring_off[r + 1] == ring_off[r] || vsign[ring_off[r]] == 0) continue;
           const int4 v = edges[ring_off[r]];
           if (tid == 0) { s_w = 0; s_on = 0; }
           __syncthreads();
@@ -304,7 +342,9 @@ __global__ void __launch_bounds__(TRX_THREADS) track_exact_kernel(const int4* __
           bool on = false;
           for (int i = o0 + tid; i < o1; i += TRX_THREADS) {
             const int4 f = edges[i];
-            wsum += trx_wind(f.x, f.y, f.z, f.w, v.x, v.y, &on);
+            bool on_i = false;
+            wsum += trx_wind(f.x, f.y, f.z, f.w, v.x, v.y, &on_i);  // (the windings of a zero-area ring cancel)
+            on |= on_i && vsign[i] != 0;
           }
           if (wsum) atomicAdd(&s_w, wsum);
           if (on) s_on = 1;
@@ -350,7 +390,7 @@ __global__ void __launch_bounds__(TRX_THREADS) track_exact_kernel(const int4* __
               const int4 f = edges[i];
               bool on = false;
               wsum += trx_wind((long long)f.x * S, (long long)f.y * S, (long long)f.z * S, (long long)f.w * S, mx, my, &on);
-              if (on) atomicMax(&s_on, i);
+              if (on && vsign[i] != 0) atomicMax(&s_on, i);
             }
             if (wsum) atomicAdd(&s_w, wsum);
             __syncthreads();
