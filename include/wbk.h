@@ -35,7 +35,8 @@ extern "C" {
 
 #define WBK_F32 0
 #define WBK_F64 1
-#define WBK_I16 2 /* packed NetCDF shorts (input of wbk_smooth / wbk_smooth_contours / wbk_orient only) */
+#define WBK_I16 2 /* packed NetCDF shorts (input of wbk_smooth / wbk_smooth_contours / wbk_orient / wbk_mflux, and the
+                     intensity of wbk_events_raster) */
 
 /* rounding of the smoothing passes (scipy keeps the input dtype, the division by
  * np.sum(weights) promotes float32 to float64 under NumPy >= 2; SURVEY.md A.7) */
@@ -113,9 +114,13 @@ int wbk_nan_border(void* d_field, int dtype, int ntime, int nlat, int nlon, int 
 /* spatial.py:27-57 calculate_momentum_flux: (u - nanmean_lon(u)) * (v - nanmean_lon(v)).  The zonal means follow
  * numpy.nanmean bit for bit: pairwise summation in the data dtype when longitude is the contiguous axis of the
  * user's array (sequential = 0), plain left-to-right summation when it is not (sequential = 1), float64 quotient
- * rounded to the data dtype. */
+ * rounded to the data dtype.  The flux is computed and written in the stored order of u and v.
+ * dtype WBK_I16: u and v are packed NetCDF shorts, packing points at two wbk_smooth_opts (u, then v: scale, offset,
+ * fill as for wbk_smooth; flip_lat / flip_lon must be 0), every value is decoded as it is loaded and everything
+ * (NaN counts, sums, products) runs on the decoded float64 values; d_out is float64.  packing is NULL for WBK_F32 /
+ * WBK_F64 (d_out of the data dtype). */
 int wbk_mflux(const void* d_u, const void* d_v, void* d_out, int dtype, int ntime, int nlat, int nlon, int sequential,
-              void* stream);
+              const wbk_smooth_opts* packing, void* stream);
 
 /* utils/data_utils.py:196-213 correct_dimension_orientation: out[t, y, x] = in[t, flip_lat ? nlat-1-y : y,
  * flip_lon ? nlon-1-x : x] */
@@ -220,10 +225,11 @@ int wbk_index_run(wbk_ctx* ctx, int njobs, int nlevels, const int* d_job_off, co
 
 /* utils/index_utils.py:35-126 calculate_properties sums and processing/events.py:66-106 to_xarray flags for
  * the events of the last wbk_index_run.  d_data: [ntime, nlat, nlon], latitude and longitude ascending.
- * d_intensity: NULL (its sums are 0) or [ntime, nlat, nlon] of intensity_dtype (WBK_F32 / WBK_F64, independent of
- * dtype), stored with descending latitudes / longitudes where intensity_flip_lat / intensity_flip_lon are set (the
- * meaning of wbk_smooth_opts / wbk_flip): member cell (t, y, x) of the ascending grid is read from the stored array
- * and widened to double, so the sums equal those of a converted, re-oriented copy bit for bit.  Only member cells
+ * d_intensity: NULL (its sums are 0) or [ntime, nlat, nlon] of intensity_dtype (WBK_F32 / WBK_F64 / WBK_I16,
+ * independent of dtype), stored as intensity_opts describes it (NULL: ascending and not packed; flip_lat / flip_lon:
+ * descending latitudes / longitudes; scale, offset, fill: the CF packing of a WBK_I16 intensity, decoded as wbk_smooth
+ * does): member cell (t, y, x) of the ascending grid is read from the stored array and widened to double (decoded
+ * for WBK_I16), so the sums equal those of a converted (decoded), re-oriented copy bit for bit.  Only member cells
  * are read.
  * d_flags: NULL or int8 [3][ntime][nlat][nlon] (kind-major), zeroed here and set to 1 where an event of that
  * kind is present; events that straddle the last meridian (split = 1 in their record) are clipped on the
@@ -236,7 +242,7 @@ int wbk_index_run(wbk_ctx* ctx, int njobs, int nlevels, const int* d_job_off, co
  * (index_utils.py:47-50). */
 int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* d_pt_off, const uint32_t* d_pts,
                       const double* d_coords, const void* d_data, int dtype, const void* d_intensity,
-                      int intensity_dtype, int intensity_flip_lat, int intensity_flip_lon, int ntime, int8_t* d_flags,
+                      int intensity_dtype, const wbk_smooth_opts* intensity_opts, int ntime, int8_t* d_flags,
                       const wbk_index_params* params, void* stream);
 
 /* Near-threshold decisions of the streamer pair scan of the last wbk_index_run (streamer_index.py:130-139): every

@@ -75,7 +75,7 @@ _SIGNATURES = {
     "wbk_index_run": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p,
                               c_void_p, POINTER(IndexParams), c_void_p]),
     "wbk_events_raster": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p, c_int,
-                                  c_int, c_int, c_int, c_void_p, POINTER(IndexParams), c_void_p]),
+                                  POINTER(SmoothOpts), c_int, c_void_p, POINTER(IndexParams), c_void_p]),
     "wbk_split_clip": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p]),
     "wbk_split_fetch": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "wbk_pack_flags": (c_int, [c_void_p, c_void_p, ctypes.c_longlong, c_void_p]),
@@ -121,7 +121,8 @@ _SIGNATURES = {
     "wbk_convolve2d": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_int, POINTER(c_double), c_int,
                                c_int, c_int, c_int, c_double, c_void_p]),
     "wbk_nan_border": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
-    "wbk_mflux": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
+    "wbk_mflux": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, POINTER(SmoothOpts),
+                          c_void_p]),
     "wbk_flip": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "wbk_synth_pv": (c_int, [c_void_p, c_int, c_int, c_int, c_int, c_double, c_double, POINTER(c_double), c_int,
                              c_void_p]),

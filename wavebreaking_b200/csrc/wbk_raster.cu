@@ -259,16 +259,23 @@ __global__ void __launch_bounds__(1024) event_list_kernel(WbkIdx x, int J, int n
 #define RS_PRE 4             // 32-column groups of a row whose field values are prefetched before the scan
 #define RS_NO_INTENSITY (-1)  // events_raster_kernel without an intensity field
 
+// how the intensity is stored: flip bit 0 / bit 1 = latitudes / longitudes descending; for packed int16 the CF packing
+// value = float64(s) * scale + offset (two roundings), s == fill -> NaN (fill outside the int16 range: no fill value)
+struct RsInten {
+  int flip, fill;
+  double scale, offset;
+};
+
 // r2_flag: the squared flag radius in cells (dlon == dlat), or with ANISO the squared extent r / min(dlon, dlat) of
 // fm's band, which is below one cell: R and the margins below are those of r2_prop wherever that is >= 1 cell.
-// IT: the intensity's dtype (WBK_F32 / WBK_F64), or RS_NO_INTENSITY (its sum stays 0 and `intensity` is not read).
-// The intensity is read in its stored orientation (iflip: bit 0 latitudes, bit 1 longitudes descending) and widened
-// to double, so the sums equal those of a converted, re-oriented copy bit for bit.
+// IT: the intensity's dtype (WBK_F32 / WBK_F64 / WBK_I16), or RS_NO_INTENSITY (its sum stays 0 and `intensity` is not
+// read).  The intensity is read in its stored orientation (ist.flip) and widened to double, or decoded for WBK_I16, so
+// the sums equal those of a converted (decoded), re-oriented copy bit for bit.
 template <typename T, bool ANISO, int IT>
 __global__ void __launch_bounds__(RS_THREADS, 3)
 events_raster_kernel(WbkDev d, WbkIdx x, const int* __restrict__ job_off, const int* __restrict__ pt_off,
                      const u32* __restrict__ pts, const double* __restrict__ area, const T* __restrict__ data,
-                     const void* __restrict__ intensity, int iflip, int8_t* __restrict__ flags, int ntime, int nlevels,
+                     const void* __restrict__ intensity, RsInten ist, int8_t* __restrict__ flags, int ntime, int nlevels,
                      int J, int njobs, double r2_prop, double r2_flag, FlagMetric fm, int rowcap) {
   WBK_DYN_SMEM(int, sm);
   __shared__ int s_box[5];
@@ -401,10 +408,17 @@ events_raster_kernel(WbkDev d, WbkIdx x, const int* __restrict__ job_off, const 
           // sum(a) and sum(y * a) have one value per row: counted here, added once per row below
           dd_add(s_v, __dmul_rn(a, dv));
           if (IT != RS_NO_INTENSITY) {
-            const int ys = (iflip & 1) ? nlat - 1 - y : y, xs = (iflip & 2) ? nlon - 1 - xf : xf;
+            const int ys = (ist.flip & 1) ? nlat - 1 - y : y, xs = (ist.flip & 2) ? nlon - 1 - xf : xf;
             const size_t k = ((size_t)t * nlat + ys) * nlon + xs;
-            const double iv = IT == WBK_F32 ? (double)static_cast<const float*>(intensity)[k]
-                                            : static_cast<const double*>(intensity)[k];
+            double iv;
+            if (IT == WBK_I16) {
+              const short s = static_cast<const short*>(intensity)[k];
+              iv = (int)s == ist.fill ? __longlong_as_double(0x7ff8000000000000LL)
+                                      : __dadd_rn(__dmul_rn((double)s, ist.scale), ist.offset);
+            } else {
+              iv = IT == WBK_F32 ? (double)static_cast<const float*>(intensity)[k]
+                                 : static_cast<const double*>(intensity)[k];
+            }
             dd_add(s_i, __dmul_rn(a, iv));
           }
           dd_add(s_x, __dmul_rn((double)px, a));
@@ -838,7 +852,8 @@ static int grid_ratio(const char* who, double dlon, double dlat, FlagMetric* fm)
 template <typename T>
 static int launch_events_raster(bool aniso, int it, size_t smem, cudaStream_t st, int grid, const WbkDev& d,
                                 const WbkIdx& x, const int* d_job_off, const int* d_pt_off, const uint32_t* d_pts,
-                                const double* area, const T* data, const void* intensity, int iflip, int8_t* d_flags,
+                                const double* area, const T* data, const void* intensity, const RsInten& ist,
+                                int8_t* d_flags,
                                 int ntime, int nlevels, int J, int njobs, double r2_prop, double r2_flag,
                                 const FlagMetric& fm, int rowcap) {
   decltype(&events_raster_kernel<T, false, RS_NO_INTENSITY>) kern;
@@ -846,11 +861,13 @@ static int launch_events_raster(bool aniso, int it, size_t smem, cudaStream_t st
     kern = aniso ? events_raster_kernel<T, true, WBK_F32> : events_raster_kernel<T, false, WBK_F32>;
   else if (it == WBK_F64)
     kern = aniso ? events_raster_kernel<T, true, WBK_F64> : events_raster_kernel<T, false, WBK_F64>;
+  else if (it == WBK_I16)
+    kern = aniso ? events_raster_kernel<T, true, WBK_I16> : events_raster_kernel<T, false, WBK_I16>;
   else
     kern = aniso ? events_raster_kernel<T, true, RS_NO_INTENSITY> : events_raster_kernel<T, false, RS_NO_INTENSITY>;
   WBK_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   WBK_LAUNCH(KID_EVENTS_RASTER, kern, dim3(grid), dim3(RS_THREADS), smem, st, d, x, d_job_off, d_pt_off,
-             (const u32*)d_pts, area, data, intensity, iflip, d_flags, ntime, nlevels, J, njobs, r2_prop, r2_flag, fm,
+             (const u32*)d_pts, area, data, intensity, ist, d_flags, ntime, nlevels, J, njobs, r2_prop, r2_flag, fm,
              rowcap);
   WBK_LAUNCH_CHECK();
   return WBK_OK;
@@ -858,7 +875,7 @@ static int launch_events_raster(bool aniso, int it, size_t smem, cudaStream_t st
 
 extern "C" int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* d_pt_off, const uint32_t* d_pts,
                                  const double* d_coords, const void* d_data, int dtype, const void* d_intensity,
-                                 int intensity_dtype, int intensity_flip_lat, int intensity_flip_lon, int ntime,
+                                 int intensity_dtype, const wbk_smooth_opts* intensity_opts, int ntime,
                                  int8_t* d_flags, const wbk_index_params* prm, void* stream) {
   if (!ctx || !d_job_off || !d_pt_off || !d_coords || !d_data || !prm || ntime < 0) {
     wbk_set_error("wbk_events_raster: invalid argument");
@@ -868,8 +885,12 @@ extern "C" int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* 
     wbk_set_error("wbk_events_raster: unsupported dtype");
     return WBK_ERR_INVALID;
   }
-  if (d_intensity && intensity_dtype != WBK_F32 && intensity_dtype != WBK_F64) {
+  if (d_intensity && intensity_dtype != WBK_F32 && intensity_dtype != WBK_F64 && intensity_dtype != WBK_I16) {
     wbk_set_error("wbk_events_raster: unsupported intensity dtype %d", intensity_dtype);
+    return WBK_ERR_INVALID;
+  }
+  if (d_intensity && intensity_dtype == WBK_I16 && !intensity_opts) {
+    wbk_set_error("wbk_events_raster: a packed int16 intensity needs its packing (intensity_opts)");
     return WBK_ERR_INVALID;
   }
   FlagMetric fm;
@@ -899,15 +920,23 @@ extern "C" int wbk_events_raster(wbk_ctx* ctx, const int* d_job_off, const int* 
   const double* area = d_coords + 3 * (size_t)d.nlat;
   const int grid = 148 * 9;
   const int it = d_intensity ? intensity_dtype : RS_NO_INTENSITY;
-  const int iflip = (intensity_flip_lat ? 1 : 0) | (intensity_flip_lon ? 2 : 0);
+  RsInten ist{0, 0x7fffffff, 1.0, 0.0};
+  if (intensity_opts) {
+    ist.flip = (intensity_opts->flip_lat ? 1 : 0) | (intensity_opts->flip_lon ? 2 : 0);
+    if (intensity_dtype == WBK_I16) {
+      ist.fill = intensity_opts->has_fill ? intensity_opts->fill : 0x7fffffff;
+      ist.scale = intensity_opts->scale;
+      ist.offset = intensity_opts->offset;
+    }
+  }
   int rc;
   if (dtype == WBK_F32)
     rc = launch_events_raster<float>(aniso, it, smem, st, grid, d, ctx->x, d_job_off, d_pt_off, d_pts, area,
-                                     (const float*)d_data, d_intensity, iflip, d_flags, ntime, ctx->nlevels, J, njobs,
+                                     (const float*)d_data, d_intensity, ist, d_flags, ntime, ctx->nlevels, J, njobs,
                                      r_prop * r_prop, r_flag * r_flag, fm, rowcap);
   else
     rc = launch_events_raster<double>(aniso, it, smem, st, grid, d, ctx->x, d_job_off, d_pt_off, d_pts, area,
-                                      (const double*)d_data, d_intensity, iflip, d_flags, ntime, ctx->nlevels, J, njobs,
+                                      (const double*)d_data, d_intensity, ist, d_flags, ntime, ctx->nlevels, J, njobs,
                                       r_prop * r_prop, r_flag * r_flag, fm, rowcap);
   if (rc != WBK_OK) return rc;
   ctx->split_clipped = d_flags != nullptr;

@@ -1,6 +1,8 @@
 // Spatial pre-processing kernels: generic convolution, momentum flux, orientation flip / int16 decode,
 // synthetic PV generator.  (The fused multi-pass smoothing stencil lives in wbk_smooth.cu.)
 // Reference: wavebreaking/processing/spatial.py:27-128, utils/data_utils.py:196-213.
+#include <type_traits>
+
 #include "wbk_common.cuh"
 
 __device__ __forceinline__ int wrap_idx(int i, int n) {
@@ -193,11 +195,30 @@ __device__ inline int mf_leaves(int n, int* off, int* len) {
   return nl;
 }
 
+// CF packing of an int16 field (wbk_smooth_opts): value = float64(s) * scale + offset (two roundings), s == fill -> NaN
+struct MfPack {
+  double scale, offset;
+  int fill;  // outside the int16 range: no fill value
+};
+
+// value i of a stored field: as stored for float data, decoded for packed int16 (T = double)
+template <typename TL, typename T>
+__device__ __forceinline__ T mf_load(const TL* __restrict__ a, size_t i, const MfPack& pk) {
+  if constexpr (std::is_same<TL, short>::value) {
+    const short s = a[i];
+    return (int)s == pk.fill ? (T)__longlong_as_double(0x7ff8000000000000LL)
+                             : (T)__dadd_rn(__dmul_rn((double)s, pk.scale), pk.offset);
+  } else {
+    (void)pk;
+    return a[i];
+  }
+}
+
 // numpy's block sum of one leaf (n <= 128) over values with NaN -> 0
-template <typename T>
-__device__ inline T mf_leaf_sum(const T* __restrict__ a, int n) {
+template <typename TL, typename T>
+__device__ inline T mf_leaf_sum(const TL* __restrict__ a, int n, const MfPack& pk) {
   auto val = [&](int i) {
-    const T v = a[i];
+    const T v = mf_load<TL, T>(a, i, pk);
     return v != v ? (T)0 : v;
   };
   if (n < 8) {
@@ -251,9 +272,10 @@ __device__ inline T mf_combine(const T* leaf, int n) {
   return ret;
 }
 
-template <typename T>
-__global__ void mflux_kernel(const T* __restrict__ u, const T* __restrict__ v, T* __restrict__ out, int nlon,
-                             long long nrows, int sequential) {
+// TL: the stored type (T, or short for packed int16 fields, which are decoded as they are loaded and give T = double)
+template <typename TL, typename T>
+__global__ void mflux_kernel(const TL* __restrict__ u, const TL* __restrict__ v, T* __restrict__ out, int nlon,
+                             long long nrows, int sequential, MfPack pu, MfPack pv) {
   __shared__ int s_off[MF_MAXLEAF], s_len[MF_MAXLEAF];
   __shared__ T s_leaf[2][MF_MAXLEAF];
   __shared__ int s_nl, s_cnt[2];
@@ -267,7 +289,7 @@ __global__ void mflux_kernel(const T* __restrict__ u, const T* __restrict__ v, T
     __syncthreads();
     int cu = 0, cv = 0;
     for (int x = threadIdx.x; x < nlon; x += blockDim.x) {
-      const T a = u[row + x], b = v[row + x];
+      const T a = mf_load<TL, T>(u, row + x, pu), b = mf_load<TL, T>(v, row + x, pv);
       cu += a == a;
       cv += b == b;
     }
@@ -276,17 +298,18 @@ __global__ void mflux_kernel(const T* __restrict__ u, const T* __restrict__ v, T
     if (!sequential) {
       for (int k = threadIdx.x; k < 2 * nl; k += blockDim.x) {
         const int w = k >= nl, l = w ? k - nl : k;
-        s_leaf[w][l] = mf_leaf_sum<T>((w ? v : u) + row + s_off[l], s_len[l]);
+        s_leaf[w][l] = mf_leaf_sum<TL, T>((w ? v : u) + row + s_off[l], s_len[l], w ? pv : pu);
       }
     }
     __syncthreads();
     if (threadIdx.x < 2) {
-      const T* src = (threadIdx.x ? v : u) + row;
+      const TL* src = (threadIdx.x ? v : u) + row;
+      const MfPack& pk = threadIdx.x ? pv : pu;
       T tot;
       if (sequential) {
         tot = (T)0;  // strided reduce: out = a[0], then out += a[i] one row of the other axis at a time
         for (int x = 0; x < nlon; ++x) {
-          const T val = src[x];
+          const T val = mf_load<TL, T>(src, x, pk);
           tot = x == 0 ? (val != val ? (T)0 : val) : tot + (val != val ? (T)0 : val);
         }
       } else {
@@ -298,25 +321,44 @@ __global__ void mflux_kernel(const T* __restrict__ u, const T* __restrict__ v, T
     __syncthreads();
     const T mu = (T)means[0], mv = (T)means[1];
     for (int x = threadIdx.x; x < nlon; x += blockDim.x) {
-      T up = u[row + x] - mu;
-      T vp = v[row + x] - mv;
+      T up = mf_load<TL, T>(u, row + x, pu) - mu;
+      T vp = mf_load<TL, T>(v, row + x, pv) - mv;
       out[row + x] = up * vp;
     }
     __syncthreads();
   }
 }
 
+static MfPack mf_pack(const wbk_smooth_opts& o) {
+  return MfPack{o.scale, o.offset, o.has_fill ? o.fill : 0x7fffffff};
+}
+
 extern "C" int wbk_mflux(const void* d_u, const void* d_v, void* d_out, int dtype, int ntime, int nlat, int nlon,
-                         int sequential, void* stream) {
+                         int sequential, const wbk_smooth_opts* packing, void* stream) {
   if (!d_u || !d_v || !d_out || nlat < 1 || nlon < 1 || (!sequential && nlon > 64 * MF_MAXLEAF)) {
     wbk_set_error("wbk_mflux: invalid argument");
+    return WBK_ERR_INVALID;
+  }
+  if (dtype != WBK_F32 && dtype != WBK_F64 && dtype != WBK_I16) {
+    wbk_set_error("wbk_mflux: unsupported dtype %d", dtype);
+    return WBK_ERR_INVALID;
+  }
+  if ((dtype == WBK_I16) != (packing != nullptr)) {
+    wbk_set_error("wbk_mflux: packed int16 u / v need their two packings (u, v); float u / v take none");
+    return WBK_ERR_INVALID;
+  }
+  if (packing && (packing[0].flip_lat || packing[0].flip_lon || packing[1].flip_lat || packing[1].flip_lon)) {
+    wbk_set_error("wbk_mflux: the flux is computed and written in stored order (packing with flip set)");
     return WBK_ERR_INVALID;
   }
   if (ntime == 0) return WBK_OK;
   const long long nrows = (long long)nlat * ntime;
   dim3 grid((unsigned)(nrows < (1 << 20) ? nrows : (1 << 20)));
-  if (dtype == WBK_F32) WBK_LAUNCH(KID_MFLUX, mflux_kernel<float>, grid, dim3(256), 0, (cudaStream_t)stream, (const float*)d_u, (const float*)d_v, (float*)d_out, nlon, nrows, sequential);
-  else WBK_LAUNCH(KID_MFLUX, mflux_kernel<double>, grid, dim3(256), 0, (cudaStream_t)stream, (const double*)d_u, (const double*)d_v, (double*)d_out, nlon, nrows, sequential);
+  cudaStream_t st = (cudaStream_t)stream;
+  const MfPack none{1.0, 0.0, 0x7fffffff};
+  if (dtype == WBK_F32) WBK_LAUNCH(KID_MFLUX, (mflux_kernel<float, float>), grid, dim3(256), 0, st, (const float*)d_u, (const float*)d_v, (float*)d_out, nlon, nrows, sequential, none, none);
+  else if (dtype == WBK_F64) WBK_LAUNCH(KID_MFLUX, (mflux_kernel<double, double>), grid, dim3(256), 0, st, (const double*)d_u, (const double*)d_v, (double*)d_out, nlon, nrows, sequential, none, none);
+  else WBK_LAUNCH(KID_MFLUX, (mflux_kernel<short, double>), grid, dim3(256), 0, st, (const short*)d_u, (const short*)d_v, (double*)d_out, nlon, nrows, sequential, mf_pack(packing[0]), mf_pack(packing[1]));
   WBK_LAUNCH_CHECK();
   return WBK_OK;
 }

@@ -301,7 +301,7 @@ def run_indices(cs, data, coords, dlon, dlat, intensity=None, which=KINDS, gmax_
                  ctypes.byref(prm), lib.stream())
         lib.call("wbk_events_raster", ctx.handle, _lib.ptr(cs.job_off), _lib.ptr(cs.pt_off), _lib.ptr(cs.pts),
                  _lib.ptr(coords), _lib.ptr(data), _lib.dtype_code(data.dtype), _lib.ptr(intensity),
-                 _lib.dtype_code(data.dtype), 0, 0, ntime, _lib.ptr(flags), ctypes.byref(prm), lib.stream())
+                 _lib.dtype_code(data.dtype), None, ntime, _lib.ptr(flags), ctypes.byref(prm), lib.stream())
         try:
             lib.call("wbk_events_counts", ctx.handle, _iptr(counts), _iptr(status), lib.stream())
             break

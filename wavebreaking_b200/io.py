@@ -17,8 +17,13 @@ import torch
 from . import _lib
 
 
+_TORCH_DTYPES = {np.dtype(np.float32): torch.float32, np.dtype(np.float64): torch.float64,
+                 np.dtype(np.int16): torch.int16}
+
+
 def open_field(path, shape=None, dtype=np.float32):
-    """Memory-map a (time, lat, lon) field: ``.npy`` (shape / dtype from the header) or raw binary (given)."""
+    """Memory-map a (time, lat, lon) field: ``.npy`` (shape / dtype from the header) or raw binary (given).  float32,
+    float64, or int16 for CF-packed fields (decoded on the device: ``Detector(packing=..., intensity_packing=...)``)."""
     if str(path).endswith(".npy"):
         arr = np.load(path, mmap_mode="r")
     else:
@@ -27,8 +32,8 @@ def open_field(path, shape=None, dtype=np.float32):
         arr = np.memmap(path, dtype=dtype, mode="r", shape=tuple(shape))
     if arr.ndim != 3:
         raise ValueError("expected a (time, lat, lon) array, got shape {}".format(arr.shape))
-    if arr.dtype not in (np.float32, np.float64):
-        raise TypeError("field dtype has to be float32 or float64, got {}".format(arr.dtype))
+    if arr.dtype not in _TORCH_DTYPES:
+        raise TypeError("field dtype has to be float32 or float64 (or packed int16), got {}".format(arr.dtype))
     return arr
 
 
@@ -49,8 +54,8 @@ def iter_batches(field, batch, depth=3, start=0, stop=None, intensity=None):
     if intensity is not None:
         arrays += list(intensity) if isinstance(intensity, (tuple, list)) else [intensity]
     nbuf = depth + 2
-    bufs = [[torch.empty((batch,) + tuple(a.shape[1:]), dtype=torch.float32 if a.dtype == np.float32 else torch.float64,
-                         pin_memory=pin) for a in arrays] for _ in range(nbuf)]
+    bufs = [[torch.empty((batch,) + tuple(a.shape[1:]), dtype=_TORCH_DTYPES[np.dtype(a.dtype)], pin_memory=pin)
+             for a in arrays] for _ in range(nbuf)]
     free = queue.Queue()
     for b in range(nbuf):
         free.put(b)
@@ -97,8 +102,13 @@ def detect_file(path, lat, lon, batch=296, depth=3, shape=None, dtype=np.float32
     ``pipeline.FlagClimatology`` for the same grid; the flag grids of every batch are added to it on the device.
     ``trackers``: a list of ``pipeline.EventTracker`` for the same grid, which track the events of every batch.
     ``intensity``: the path of an intensity field, or a pair of paths ``(u_path, v_path)`` whose momentum flux is the
-    intensity (see ``Detector.stream``); opened like ``path`` (same ``shape`` / ``dtype`` for raw binary files) and
-    stored like the field."""
+    intensity (see ``Detector.stream``); opened like ``path`` (same ``shape`` / ``dtype`` for raw binary files; a
+    ``.npy`` file carries its own dtype) and stored like the field.
+
+    Packed int16 files (ERA5's ``scale_factor`` / ``add_offset`` / ``_FillValue``) go from disk to the device as they
+    are stored and are decoded in the kernels that read them: give ``packing=(scale, offset, fill)`` for an int16
+    field and ``intensity_packing=`` for int16 intensity files (one packing for a field, ``((su, ou, fu), (sv, ov,
+    fv))`` for u and v); both are passed to the ``Detector`` with the other keyword arguments."""
     from . import pipeline
 
     field = open_field(path, shape=shape, dtype=dtype)

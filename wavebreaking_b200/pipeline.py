@@ -14,6 +14,7 @@ host<->device copies overlap with kernels (``Detector.stream``).
 """
 
 import ctypes
+import gc
 import logging
 from dataclasses import dataclass, replace
 
@@ -60,9 +61,33 @@ def _pinned(shape, dtype, lib):
     return torch.empty(shape, dtype=dtype, pin_memory=lib.is_cuda)
 
 
-def _intensity_item(item, shape):
+def _cf_packing(p, what):
+    """``(scale, offset, fill)`` of a CF-packed int16 field with a finite scale and offset; a fill value that no int16
+    can take (or None) means no fill."""
+    if not isinstance(p, (tuple, list)) or len(p) != 3:
+        raise ValueError("{} has to be (scale_factor, add_offset, _FillValue or None), got {!r}".format(what, p))
+    scale, offset, fill = float(p[0]), float(p[1]), p[2]
+    if not (np.isfinite(scale) and np.isfinite(offset)):
+        raise ValueError("{}: scale_factor and add_offset have to be finite, got {} and {}".format(what, scale, offset))
+    if fill is not None and not (float(fill) == int(fill) and -32768 <= int(fill) <= 32767):
+        fill = None
+    return scale, offset, None if fill is None else int(fill)
+
+
+def _intensity_packing(p):
+    """``Detector(intensity_packing=...)`` normalised: None, one packing ``(scale, offset, fill)`` for single-field
+    items, or a pair of them ``((su, ou, fu), (sv, ov, fv))`` for ``(u, v)`` items."""
+    if p is None:
+        return None
+    if isinstance(p, (tuple, list)) and len(p) == 2 and all(isinstance(q, (tuple, list)) for q in p):
+        return _cf_packing(p[0], "the packing of u"), _cf_packing(p[1], "the packing of v")
+    return (_cf_packing(p, "intensity_packing"),)
+
+
+def _intensity_item(item, shape, packing=None):
     """One intensity item of ``Detector.stream`` as the tuple ``(field,)`` or ``(u, v)``; raises ValueError unless its
-    tensors are float32 / float64 and shaped like the batch (``shape``), and u and v agree in shape and dtype."""
+    tensors are float32 / float64, or int16 with a matching ``packing`` (``_intensity_packing``: one packing for a
+    field, two for u and v), shaped like the batch (``shape``), and u and v agree in shape and dtype."""
     fields = tuple(item) if isinstance(item, (tuple, list)) else (item,)
     if len(fields) not in (1, 2) or not all(isinstance(f, torch.Tensor) for f in fields):
         raise ValueError("an intensity item is a tensor or a pair (u, v) of tensors")
@@ -70,12 +95,22 @@ def _intensity_item(item, shape):
         raise ValueError("u and v differ: shapes {} and {}, dtypes {} and {}".format(
             tuple(fields[0].shape), tuple(fields[1].shape), fields[0].dtype, fields[1].dtype))
     for f in fields:
-        if f.dtype not in (torch.float32, torch.float64):
-            raise ValueError("intensity has to be float32 or float64, got {} (packed int16 u / v are not "
-                             "supported)".format(f.dtype))
+        if f.dtype not in (torch.float32, torch.float64, torch.int16):
+            raise ValueError("intensity has to be float32 or float64 (or CF-packed int16 with intensity_packing), "
+                             "got {}".format(f.dtype))
         if tuple(f.shape) != tuple(shape):
             raise ValueError("an intensity item of shape {} for a batch of shape {}".format(tuple(f.shape),
                                                                                           tuple(shape)))
+    packed = fields[0].dtype == torch.int16
+    if packed and packing is None:
+        raise ValueError("a packed int16 intensity needs its CF packing: Detector(intensity_packing=(scale, offset, "
+                         "fill)) for a field, ((su, ou, fu), (sv, ov, fv)) for (u, v)")
+    if not packed and packing is not None:
+        raise ValueError("the Detector has an intensity_packing, but the intensity is {} (the packing is for int16 "
+                         "items)".format(fields[0].dtype))
+    if packed and len(packing) != len(fields):
+        raise ValueError("intensity_packing has {} packing(s), the item {} field(s): one packing goes with a field, "
+                         "a pair of packings with (u, v)".format(len(packing), len(fields)))
     return fields
 
 
@@ -165,7 +200,7 @@ class Detector:
 
     def __init__(self, lat, lon, levels=(2.0,), periodic_add=120, passes=5, which=detect.KINDS, geo_dis=800.0,
                  cont_dis=1500.0, range_group=5.0, ot_min_exp=5.0, co_min_exp=5.0, want_flags=True, fuse=True,
-                 packing=None, graphs=False, nvtx=True, want_pieces=False):
+                 packing=None, graphs=False, nvtx=True, want_pieces=False, intensity_packing=None):
         self.lib = _lib.get()
         self.lat = np.asarray(lat, dtype=np.float64)
         self.lon = np.asarray(lon, dtype=np.float64)
@@ -194,6 +229,9 @@ class Detector:
         self.fuse = bool(fuse)
         # CF packing of int16 input (scale_factor, add_offset, _FillValue or None), decoded in the smoothing loads
         self.packing = tuple(packing) if packing is not None else (1.0, 0.0, None)
+        # CF packing of int16 intensity items (see stream): None, (scale, offset, fill) for a field, or one such triple
+        # for u and one for v; decoded inside the kernels that read the items
+        self.intensity_packing = _intensity_packing(intensity_packing)
         # also download the device clipper's pieces of the events that straddle the last meridian (events_soup then
         # needs no host-side polygon clipping; used by the tracking leg)
         self.want_pieces = bool(want_pieces)
@@ -317,21 +355,28 @@ class Detector:
                 flags = slot.buffer("flags", torch.int8, (3, slot.T, self.nlat, self.nlon))
             else:
                 flags = torch.empty((3, nt, self.nlat, self.nlon), dtype=torch.int8, device=lib.device)
-        # the rasteriser reads the intensity's member cells in their stored dtype and orientation
-        inten, iflip = intensity, (0, 0)
+        # the rasteriser reads the intensity's member cells in their stored dtype and orientation (and decodes packed
+        # int16 ones as it reads them)
+        inten, iopts = intensity, None
         if isinstance(intensity, tuple):
-            inten, iflip = intensity[0], (int(self.flip_lat), int(self.flip_lon))
+            inten = intensity[0]
+            packed = inten.dtype == torch.int16
             if len(intensity) == 2:
                 # zonal means summed in the stored memory order (what numpy does on the user's array); longitude is
-                # the contiguous axis of a batch
+                # the contiguous axis of a batch.  Packed u and v are decoded in the loads into a float64 flux.
                 u, v = intensity
-                inten = slot.buffer("mflux", u.dtype)[:nt]
+                inten = slot.buffer("mflux", torch.float64 if packed else u.dtype)[:nt]
+                mpk = (_lib.SmoothOpts * 2)(*(_lib.smooth_opts(False, False, *p) for p in self.intensity_packing)) \
+                    if packed else None
                 lib.call("wbk_mflux", _lib.ptr(u), _lib.ptr(v), _lib.ptr(inten), _lib.dtype_code(u.dtype), nt,
-                         self.nlat, self.nlon, 0, st)
+                         self.nlat, self.nlon, 0, mpk, st)
+                iopts = _lib.smooth_opts(self.flip_lat, self.flip_lon)
+            else:
+                iopts = _lib.smooth_opts(self.flip_lat, self.flip_lon, *(self.intensity_packing[0] if packed else ()))
         lib.call("wbk_events_raster", h, _lib.ptr(slot.job_off), _lib.ptr(slot.pt_off), _lib.ptr(slot.pts),
                  _lib.ptr(self.coords), _lib.ptr(sm), _lib.dtype_code(sm.dtype), _lib.ptr(inten),
-                 _lib.dtype_code(sm.dtype if inten is None else inten.dtype), iflip[0], iflip[1], nt, _lib.ptr(flags),
-                 ctypes.byref(prm), st)
+                 _lib.dtype_code(sm.dtype if inten is None else inten.dtype),
+                 None if iopts is None else ctypes.byref(iopts), nt, _lib.ptr(flags), ctypes.byref(prm), st)
         lib.call("wbk_batch_fetch", h, _lib.ptr(slot.pt_off), _lib.ptr(slot.pts), _lib.ptr(slot.ev_int),
                  _lib.ptr(slot.ev_f64), _lib.ptr(slot.ev_job), _lib.ptr(slot.ring_off), _lib.ptr(slot.ring_pts),
                  slot.cap_e, slot.cap_r, _lib.ptr(slot.summary), st)
@@ -377,7 +422,7 @@ class Detector:
         if nt > slot.T:
             raise ValueError("batch of {} time steps exceeds the slot size {}".format(nt, slot.T))
         if isinstance(intensity, tuple):
-            intensity = _intensity_item(intensity, raw.shape)
+            intensity = _intensity_item(intensity, raw.shape, self.intensity_packing)
         use_stream = stream if stream is not None else slot.stream
         args = (slot, raw, flags_out, flags_host, gmax_nx, smoothed, intensity, packed_host)
         if use_stream is None:  # emulator
@@ -403,8 +448,18 @@ class Detector:
                 use_stream.synchronize()
                 g = torch.cuda.CUDAGraph()
                 n0 = lib.cdll.wbk_launch_count()
-                with torch.cuda.graph(g, stream=use_stream, capture_error_mode="relaxed"):
-                    pend = self._enqueue(*args)
+                # no garbage collection during the capture: a dead slot's pinned buffers, freed then, would record
+                # their release events on a pool stream that may be the one being captured, and those events could
+                # never be queried again
+                gc_on = gc.isenabled()
+                gc.collect()
+                gc.disable()
+                try:
+                    with torch.cuda.graph(g, stream=use_stream, capture_error_mode="relaxed"):
+                        pend = self._enqueue(*args)
+                finally:
+                    if gc_on:
+                        gc.enable()
                 nk = int(lib.cdll.wbk_launch_count() - n0)
                 slot.graphs[key] = (g, pend, nk)
                 g.replay()
@@ -571,7 +626,13 @@ class Detector:
         field for every contour level; without it that column is 0.  Host items are uploaded into the slot's own
         buffers, so the batch, the upload and the momentum flux included, is captured in its CUDA graph.  A batch is
         (time, lat, lon) with longitude contiguous, so the zonal means of the momentum flux are summed pairwise, as
-        ``spatial.momentum_flux(u, v, lon_contiguous=True)`` does.
+        ``spatial.momentum_flux(u, v, lon_contiguous=True)`` does.  Items may also be CF-packed int16, as ERA5 stores
+        intensity and wind: build the Detector with ``intensity_packing=(scale, offset, fill)`` for field items or
+        ``((su, ou, fu), (sv, ov, fv))`` for ``(u, v)`` items (u and v each with their own packing; ``fill`` None for
+        no fill value).  Packed u and v are decoded in ``wbk_mflux``'s loads into a float64 flux, a packed field at the
+        member cells the rasteriser reads, with xarray's rule ``float64(s) * scale + offset`` (fill -> NaN); the
+        results equal those of float64 items holding the decoded values.  A packed item without the packing, or a
+        packing with float items, raises ValueError before any device work on the batch.
         """
         inten_it = iter(intensity) if intensity is not None else None
         if climatology is not None:
@@ -603,7 +664,7 @@ class Detector:
                 item = next(inten_it, None)
                 if item is None:
                     raise ValueError("the intensity iterable ended before the batches (batch {})".format(i))
-                item = _intensity_item(item, raw.shape)
+                item = _intensity_item(item, raw.shape, self.intensity_packing)
             for tr, start in zip(trackers, starts):  # before any device work on a batch the dates do not cover
                 tr._check_steps(start + submitted, int(raw.shape[0]))
             submitted += int(raw.shape[0])

@@ -163,7 +163,7 @@ def momentum_flux(u, v, lon_contiguous=True):
     out = torch.empty_like(a)
     ntime, nlat, nlon = a.shape
     lib.call("wbk_mflux", _lib.ptr(a), _lib.ptr(b), _lib.ptr(out), _lib.dtype_code(a.dtype), ntime, nlat, nlon,
-             0 if lon_contiguous else 1, lib.stream())
+             0 if lon_contiguous else 1, None, lib.stream())
     return out
 
 
